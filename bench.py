@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ManyTor step loop on B200 (contract: see the task README / DESIGN.md).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input: ONE
 fused-kernel launch advancing every env of the shard by one env-step, actions
@@ -263,6 +263,26 @@ def run_reference_arm(args) -> None:
 # ----------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------
+DUMP_ENVS = 1 << 18       # 2^18 envs x (30 obs + reward + done) x 4 B = 32 MiB
+
+
+def dump_sample(n: int):
+    """The envs `--dump-outputs` writes: the same seeded sample of DUMP_ENVS of the n envs in every run, ascending."""
+    import numpy as np
+    return np.sort(np.random.RandomState(0).choice(n, size=min(n, DUMP_ENVS), replace=False))
+
+
+def dump_outputs(out_dir: str, outputs: dict) -> None:
+    """`--dump-outputs`: write each output of the last timed step as out_dir/<name>.npy (float32), rows dump_sample(n),
+    so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    sel = torch.from_numpy(dump_sample(outputs["reward"].shape[0])).to(outputs["reward"].device)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, sel).float().cpu().numpy())
+
+
 def run_gpu(args) -> None:
     import numpy as np
     import torch
@@ -304,18 +324,24 @@ def run_gpu(args) -> None:
     def fence():
         torch.cuda.synchronize(); barrier(); torch.cuda.synchronize()
 
-    # ---- steady state: clock warm-up + burn-in with in-kernel random actions (never cycled) -----------
-    env.clear_stats()
-    env.rollout_random(args.burn_in, write_obs=False)
+    # ---- steady state: clock warm-up, then burn-in with in-kernel random actions (never cycled) ---------
     t_warm = time.perf_counter()
     while time.perf_counter() - t_warm < args.clock_warm_s:          # same kernel family, obs written: clocks/power settle
         env.rollout_random(200, write_obs=True)
         torch.cuda.synchronize()
+    # The warm-up ran for a wall-clock time, so it left the envs after a varying number of steps: start over
+    # from the seed, so that the timed steps see the same state and actions in every run with the same arguments.
+    env.set_seed(SEED)
+    env.reset()
+    env.clear_stats()
+    env.rollout_random(args.burn_in, write_obs=False)
     refill()
     torch.cuda.synchronize()
 
+    last = []                                         # outputs of the latest step (buffers every step rewrites)
+
     def step_fn(i):
-        env.step(actions[i % n_buf])
+        last[:] = env.step(actions[i % n_buf])
 
     def capture(body):
         try:
@@ -368,6 +394,8 @@ def run_gpu(args) -> None:
             refill()                                  # fresh random actions for every repeat (untimed)
         ms_all, ms_k, st = timed_region(graph, lambda: [step_fn(W + i) for i in range(K)])
         reps.append((mtd.max_over_ranks(ms_all, dev), mtd.max_over_ranks(ms_k, dev)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("obs", "reward", "done"), last)))   # before other modes overwrite them
     stats = mtd.stats_dict(st)                        # burn-in + warm-ups + every timed repeat, all ranks
     launches_timed = (K + 1) if graph is not None else (env.launch_count - l0) // R - W
     order = sorted(range(R), key=lambda i: reps[i][0])
@@ -503,7 +531,7 @@ def run_gpu(args) -> None:
                        "actions": f"uniform integer degrees in [-180,180), read from HBM [N][4] fp32; {n_buf} distinct buffers "
                                   "(one per warm-up and timed step), refilled before every repeat: no action is ever replayed",
                        "submission": "one K-node CUDA graph" if graph is not None else "K stream launches",
-                       "burn_in": f"{args.burn_in} + {args.clock_warm_s:.1f} s of in-kernel random-action steps before the first repeat (steady state of the episode process)",
+                       "burn_in": f"{args.clock_warm_s:.1f} s of in-kernel random-action steps (clocks), then re-seed + reset and {args.burn_in} in-kernel random-action steps before the first repeat (steady state of the episode process)",
                        "repeats": f"{R} timed regions of exactly K steps each (W warm-up steps before each); value = the median region, best reported beside it",
                        "l2": f"working set {(n * (B + 8 * 4)) / 2**20:.0f} MiB per step > 126 MiB L2 (inputs larger than L2, no flush needed)",
                        "parallelism": f"env-sharded x{world}, no per-step collective, 1 stats all-reduce inside the timed region "
@@ -560,9 +588,17 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--repeats", type=int, default=10, help="timed regions of K steps each; value = median, best beside it")
     ap.add_argument("--reference-port", action="store_true", help="--impl reference: time the numpy port even when oracle/_ref exists")
-    ap.add_argument("--burn-in", type=int, default=HORIZON,
-                    help="untimed random-action steps before warm-up so episodes reach their steady state")
+    # 20 horizons: episodes end at random steps (all objectives caught), so the wave of truncations that the common
+    # start at step 0 sends every horizon has died out before the timed steps
+    ap.add_argument("--burn-in", type=int, default=20 * HORIZON,
+                    help="untimed random-action steps after the clock warm-up and the re-seeded reset, before the "
+                         "warm-up steps of the first repeat, so that episodes reach their steady state")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's obs, reward and done (rank 0, a fixed sample "
+                         f"of {DUMP_ENVS} envs) as DIR/<name>.npy in float32")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     # stdout carries exactly ONE line, the JSON result: anything a library writes to file descriptor 1 on the
     # way (NCCL prints its version there when the box sets NCCL_DEBUG) is sent to stderr instead
     sys.stdout.flush()

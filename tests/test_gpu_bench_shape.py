@@ -164,3 +164,66 @@ def test_one_large_handle_equals_many_small_ones(mt, rand):
     for key in tw:
         assert tw[key] == sum(q[key] for q in ts), key
     assert tw["env_steps"] == n * k and tw["episodes"] >= n * (k // 5)
+
+
+def test_bench_dump_outputs_are_reproducible(mt, tmp_path):
+    """bench.py --dump-outputs: the outputs of the last timed step at the rows of bench.dump_sample -- equal to a replay
+    of bench.py's seeded sequence through BatchedEnvs, identical in two runs whatever the wall-clock warm-up ran, and a
+    different last step when --steps differs."""
+    import subprocess
+    import sys
+    import torch
+    import bench
+
+    K, W, R, burn_in = 4, 3, 2, 300
+
+    def run(name, steps, clock_warm_s):
+        out = tmp_path / name
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", str(W),
+               "--repeats", str(R), "--burn-in", str(burn_in), "--clock-warm-s", str(clock_warm_s), "--clock-probe-s", "0",
+               "--clock-period-ms", "0", "--no-cpu", "--dump-outputs", str(out)]
+        res = subprocess.run(cmd, capture_output=True, text=True, cwd=tmp_path)
+        assert res.returncode == 0, res.stderr[-2000:]
+        line = json.loads(res.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps
+        files = sorted(p.name for p in out.iterdir())
+        assert files == ["done.npy", "obs.npy", "reward.npy"], files
+        assert sum((out / f).stat().st_size for f in files) <= 64 << 20
+        return {f[:-4]: np.load(out / f) for f in files}, line
+
+    (a, line), (b, _), (c, _) = run("a", K, 0.0), run("b", K, 0.5), run("c", K + 1, 0.0)
+    for k in a:
+        np.testing.assert_array_equal(a[k], b[k], err_msg=k)
+    assert not np.array_equal(a["obs"], c["obs"])
+
+    # replay: re-seeded reset, burn-in, then the action buffers in bench.py's order -- with a CUDA graph, 3 steps while
+    # capturing and one untimed replay of the K steps -- and per repeat a refill, W warm-up steps and the K timed steps
+    n = bench.ENVS_PER_GPU
+    env = mt.BatchedEnvs(n, bench.OBJ, device=0, horizon=bench.HORIZON, auto_reset=True, seed=bench.SEED)
+    env.reset()
+    env.set_seed(bench.SEED)
+    env.reset()
+    env.rollout_random(burn_in, write_obs=False)
+    gen = torch.Generator(device="cuda")
+    gen.manual_seed(bench.SEED)
+    actions = [torch.empty((n, 4), device="cuda", dtype=torch.float32) for _ in range(K + W)]
+
+    def refill():
+        for t in actions:
+            t.copy_(torch.randint(-180, 180, (n, 4), device="cuda", generator=gen))
+
+    refill()
+    order = list(range(W, W + 3)) + list(range(W, W + K)) if line["config"]["submission"] == "one K-node CUDA graph" else []
+    for r in range(R):
+        if r:
+            for i in order:
+                out = env.step(actions[i])
+            order = []
+            refill()
+        order += list(range(W + K))
+    for i in order:
+        out = env.step(actions[i])
+    sel = torch.from_numpy(bench.dump_sample(n)).cuda()
+    for name, t in zip(("obs", "reward", "done"), out):
+        np.testing.assert_array_equal(a[name], t.index_select(0, sel).float().cpu().numpy(), err_msg=name)
+    assert a["obs"].shape == (min(n, bench.DUMP_ENVS), 3 * bench.OBJ) and a["done"].any()
