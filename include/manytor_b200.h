@@ -58,7 +58,7 @@ typedef struct mt_config {
     int32_t device;                /* CUDA device ordinal                                 */
     int64_t n_envs;                /* N: environments in this shard                       */
     int64_t env_id_base;           /* global id of env 0 (keys the RNG: shard-invariant)  */
-    int32_t n_joints;              /* J, 1..MT_MAX_JOINTS (reference: 4)                  */
+    int32_t n_joints;              /* J, 2..MT_MAX_JOINTS (reference: 4)                  */
     int32_t n_obj;                 /* X, 1..MT_MAX_OBJ (Environment(obj_number), :130)    */
     float dh[MT_MAX_JOINTS][4];    /* rows (a, alpha, d, theta_offset), radians (:42-48)  */
     int32_t obs_frame;             /* frame anchoring observations (reference: 3, :143)   */

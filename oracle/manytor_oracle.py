@@ -248,6 +248,7 @@ class StepResult(NamedTuple):
     neg: np.ndarray            # (N,)   bool ground flag (sticky over the 25 poses)
     ground_margin: np.ndarray  # (N,)   min |z| over sub-poses and ground frames
     catch_margin: np.ndarray   # (N, X) distance of the catch decision from flipping
+    frames: np.ndarray         # (N, J+1, 3) origins of frames 0..J at the final pose, indexed by frame number
 
 
 class OracleEnvs:
@@ -275,7 +276,12 @@ class OracleEnvs:
 
     # -- frame helpers ------------------------------------------------------
     def _row(self, frame: int) -> int:
-        """Row of ``joints_coordinates`` holding ``frame`` (row 0 = base, row r = frame r+1)."""
+        """Row of ``joints_coordinates`` holding ``frame`` (row 0 = base, row r = frame r+1).
+
+        Frame 1 has no row there (manytor.py:188-189): select it from ``StepResult.frames`` /
+        ``fk_frames``, which are indexed by frame number and hold every frame."""
+        if frame == 1:
+            raise ValueError("joints_coordinates has no row for frame 1; index fk_frames / StepResult.frames instead")
         return 0 if frame == 0 else frame - 1
 
     # -- reset --------------------------------------------------------------
@@ -309,7 +315,8 @@ class OracleEnvs:
     def get_observations(self) -> np.ndarray:
         """manytor.py:141-153, including the side effect of zeroing dead points."""
         self.points[~self.alive] = 0.0                              # :148
-        return observations(self.joints[:, self._row(self.spec.obs_frame)], self.points, self.alive)
+        anchor = fk_frames(self.goals, self.spec)[:, self.spec.obs_frame]
+        return observations(anchor, self.points, self.alive)
 
     # -- step ---------------------------------------------------------------
     def step(self, action) -> StepResult:
@@ -332,9 +339,10 @@ class OracleEnvs:
         self.goals = route[-1].copy()                               # :184 (last pose == action)
         self.joints = np.concatenate([fr[:, 0:1], fr[:, 2:]], axis=1)   # :189
 
-        obs2 = observations(self.joints[:, self._row(spec.obs_frame)], self.points, self.alive)  # :204
+        # anchor and catcher by frame number: joints_coordinates has no row for frame 1
+        obs2 = observations(fr[:, spec.obs_frame], self.points, self.alive)  # :204
 
-        ee = self.joints[:, self._row(spec.catch_frame)]            # :162
+        ee = fr[:, spec.catch_frame]                                # :162
         dist = np.abs(ee[:, None, :] - self.points)                 # (N, X, 3)
         close = dist <= spec.catch_tol                              # math.isclose(abs_tol), rel term < 6e-8
         caught = close.all(axis=-1)                                 # :167
@@ -351,7 +359,7 @@ class OracleEnvs:
         if self.terminate_on_ground:
             done = done | neg
         return StepResult(obs2, reward, done, self.joints.copy(), self.alive.copy(), neg,
-                          margin, catch_margin)
+                          margin, catch_margin, fr)
 
     # -- state exchange with the device path ---------------------------------
     def alive_mask_u32(self) -> np.ndarray:

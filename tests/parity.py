@@ -27,6 +27,8 @@ class Report:
     max_angle_excess: float = 0.0      # worst (error / allowed)
     near_threshold: int = 0            # reported, allowed
     hard_mismatch: int = 0             # must stay 0
+    rewarded: int = 0                  # env-steps with reward +1 (oracle): catches were compared
+    ground: int = 0                    # env-steps with ground contact (oracle): the ground test was compared
     notes: list = field(default_factory=list)
 
     def ok(self) -> bool:
@@ -35,7 +37,7 @@ class Report:
     def summary(self) -> str:
         return (f"{self.env_steps} env-steps: joint err {self.max_joint_err:.2e}, dist err {self.max_dist_err:.2e}, "
                 f"angle err/allowed {self.max_angle_excess:.2f}, near-threshold flips {self.near_threshold}, "
-                f"hard mismatches {self.hard_mismatch}")
+                f"hard mismatches {self.hard_mismatch}; events: reward +1 {self.rewarded}, ground {self.ground}")
 
 
 def reach_of(spec) -> float:
@@ -52,6 +54,8 @@ def compare_step(rep: Report, spec, ora, r, points_before, alive_before, dev_obs
     pos_tol = REL_POS_TOL * reach
     thr = THRESH_TOL * (reach / 55.6)
     rep.env_steps += n
+    rep.rewarded += int((r.reward == 1).sum())
+    rep.ground += int(r.neg.sum())
 
     if dev_joints is not None:
         je = np.abs(dev_joints.astype(np.float64) - r.joints).max()
@@ -76,12 +80,22 @@ def compare_step(rep: Report, spec, ora, r, points_before, alive_before, dev_obs
                          f"ground margin {r.ground_margin[i]:.3e}, catch margin {cm[i]:.3e}")
 
     # observations (computed from alive_before, which is kept in sync)
-    anchor = r.joints[:, ora._row(spec.obs_frame)]
-    d = np.abs(anchor[:, None, :] - points_before)
+    compare_obs(rep, spec, r.frames[:, spec.obs_frame], points_before, alive_before, dev_obs, r.obs)
+    return bad
+
+
+def compare_obs(rep: Report, spec, anchor, points, alive, dev_obs, ref_obs):
+    """Compare observations (N, 3X) of objectives `points` (N, X, 3) seen from `anchor` (N, 3): distances within
+    DIST_ATOL_REL of reach, bearings within the error a position error of REL_POS_TOL moves them by (plus a floor),
+    dead objectives exactly zero.  Misses count as hard mismatches."""
+    n, x = alive.shape
+    reach = reach_of(spec)
+    pos_tol = REL_POS_TOL * reach
+    d = np.abs(anchor[:, None, :] - points)
     hxy = np.hypot(d[..., 0], d[..., 1])
     dist = np.sqrt(hxy ** 2 + d[..., 2] ** 2)
     o_dev = dev_obs.astype(np.float64).reshape(n, x, 3)
-    o_ref = r.obs.reshape(n, x, 3)
+    o_ref = ref_obs.reshape(n, x, 3)
     de = np.abs(o_dev[..., 0] - o_ref[..., 0])
     rep.max_dist_err = max(rep.max_dist_err, float(de.max()))
     dist_tol = DIST_ATOL_REL * reach + pos_tol
@@ -95,11 +109,10 @@ def compare_step(rep: Report, spec, ora, r, points_before, alive_before, dev_obs
     if de.max() > dist_tol or ex > 1.0:
         rep.hard_mismatch += 1
         rep.notes.append(f"obs mismatch: dist err {de.max():.3e} (tol {dist_tol:.3e}), angle err/allowed {ex:.2f}")
-    dead = ~alive_before
+    dead = ~alive
     if dead.any() and np.abs(o_dev[dead]).max() != 0.0:
         rep.hard_mismatch += 1
         rep.notes.append("dead objective did not read as zeros")
-    return bad
 
 
 def alive_bits_to_matrix(words: np.ndarray, x: int) -> np.ndarray:
@@ -139,7 +152,7 @@ class ChunkedOracle:
     """One OracleEnvs interface over several smaller ones (bounded temporaries at 2^18..2^20 envs).
 
     Exposes what `compare_step` / the lock-step loops use: n, x, spec, goals, alive, points,
-    total_reward, ep_len, step(), reset(), _row()."""
+    total_reward, ep_len, step(), reset()."""
 
     def __init__(self, n_envs: int, obj_number: int, spec, chunk: int = 1 << 16, **kw):
         from oracle import OracleEnvs
@@ -155,9 +168,6 @@ class ChunkedOracle:
     points = property(lambda self: self._cat("points"))
     total_reward = property(lambda self: self._cat("total_reward"))
     ep_len = property(lambda self: self._cat("ep_len"))
-
-    def _row(self, frame):
-        return self.parts[0]._row(frame)
 
     def reset(self, mask=None, points=None):
         for (a, b), p in zip(self.bounds, self.parts):

@@ -63,6 +63,16 @@ def test_bad_config_is_rejected(lib):
     cfg.n_obj = 33
     assert lib.mt_create(C.byref(cfg), C.byref(h)) == -1
     assert not h
+    for J in (1, 9):                                   # the generic chain is built for J = 2 .. MT_MAX_JOINTS
+        cfg = _lib.default_config()
+        cfg.n_joints = J
+        assert lib.mt_create(C.byref(cfg), C.byref(h)) == -1
+        assert b"n_joints must be in [2, 8]" in lib.mt_last_error() and not h
+    for field in ("obs_frame", "ground_frame_a", "ground_frame_b", "catch_frame"):
+        cfg = _lib.default_config()                    # frames 0 .. J exist; J + 1 does not
+        setattr(cfg, field, cfg.n_joints + 1)
+        assert lib.mt_create(C.byref(cfg), C.byref(h)) == -1
+        assert b"frame selector 5 outside [0, 4]" in lib.mt_last_error() and not h
 
 
 def test_no_gpu_means_loud_failure(lib):

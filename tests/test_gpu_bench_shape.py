@@ -34,12 +34,12 @@ def mt():
     return manytor_b200
 
 
-def _seed_late_episode(env, ora, rs, n, x, horizon):
+def _seed_late_episode(env, ora, rs, n, x, horizon, alive_p=0.35):
     """Put every env somewhere inside an episode: random poses, a random subset of objectives already
     collected (many envs one catch away from termination), random episode lengths up to the horizon --
     so that the few steps of the test see terminations, truncations and fresh objectives."""
     goals = rs.randint(-180, 180, size=(n, ora.spec.n_joints)).astype(np.float64)
-    alive = rs.rand(n, x) < 0.35
+    alive = rs.rand(n, x) < alive_p
     alive[np.arange(n), rs.randint(0, x, size=n)] = True               # at least one objective alive
     total = -rs.randint(0, 40, size=n).astype(np.float64)
     ep = rs.randint(0, horizon, size=n)
@@ -54,7 +54,7 @@ def _seed_late_episode(env, ora, rs, n, x, horizon):
         p.joints = joints_coordinates(p.goals, p.spec)
 
 
-def _bench_shape_run(mt, n, x, steps, horizon, spec, arm, fk_mode, seed, scale=1.0, sets=3):
+def _bench_shape_run(mt, n, x, steps, horizon, spec, arm, fk_mode, seed, scale=1.0, sets=3, alive_p=0.35):
     rs = np.random.RandomState(seed)
     stream = np.float32(half_ball_points(rs, (sets, n, x), radius=spec.radius)).astype(np.float64)
     env = mt.BatchedEnvs(n, x, arm=arm, device=0, auto_reset=True, horizon=horizon, fk_mode=fk_mode, seed=seed)
@@ -62,7 +62,7 @@ def _bench_shape_run(mt, n, x, steps, horizon, spec, arm, fk_mode, seed, scale=1
     env.reset()
     ora = ChunkedOracle(n, x, spec)
     ora.reset(points=stream[0])
-    _seed_late_episode(env, ora, rs, n, x, horizon)
+    _seed_late_episode(env, ora, rs, n, x, horizon, alive_p)
     # objectives near the arm make catches (and therefore terminations) frequent enough to be seen in a few steps
     J = spec.n_joints
     rep, stats, slack, forked = lockstep_auto_reset(env, ora, spec, stream,
@@ -127,6 +127,20 @@ def test_nvrtc_arm_at_benchmark_shape(mt):
     rep, stats, slack, forked, s, ora = _bench_shape_run(mt, n, x, steps, horizon, oarm, arm, 3, seed=9)
     _check(rep, stats, slack, forked, s, ora, n, steps)
     _record("nvrtc_5joint_2p18", rep, n, steps)
+
+
+@pytest.mark.parametrize("fk_mode", [3, 1])
+def test_eight_joint_arm_at_benchmark_shape(mt, fk_mode):
+    """The 8-joint table of tests/arms.py at X = 32 -- the largest tiles (12 KB per warp) of the 16-warp generic kernel,
+    1.7 tiles per warp at 2^17 envs -- specialised at run time (fk_mode 3) and with the run-time table (fk_mode 1)."""
+    from arms import arm_pair
+    n, x, steps, horizon = 1 << 17, 32, 2, 50
+    oarm, arm = arm_pair(8)
+    # at X = 32 few envs are one catch from the end of their episode unless most objectives are already collected
+    rep, stats, slack, forked, s, ora = _bench_shape_run(mt, n, x, steps, horizon, oarm, arm, fk_mode, seed=17,
+                                                         alive_p=0.02)
+    _check(rep, stats, slack, forked, s, ora, n, steps)
+    _record(f"8joint_x32_fk{fk_mode}_2p17", rep, n, steps)
 
 
 @pytest.mark.parametrize("rand", [True, False])

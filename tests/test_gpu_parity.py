@@ -207,8 +207,10 @@ def test_auto_reset_with_objective_stream(mt):
 # on-device RNG streams
 # --------------------------------------------------------------------------
 def test_sample_actions_match_philox_oracle(mt):
+    """Joints 0 .. 3 come from one Philox block, joints 4 .. 7 from a second one (draw_actions, mt_step.cuh)."""
+    from arms import arm_pair
     n = 1000
-    for J, arm in ((4, mt.REFERENCE_ARM), (6, mt.UR5_ARM)):
+    for J, arm in ((4, mt.REFERENCE_ARM), (6, mt.UR5_ARM), *((J, arm_pair(J)[1]) for J in (2, 3, 5, 7, 8))):
         env = mt.BatchedEnvs(n, 3, arm=arm, device=0, seed=0x1234567890ABCDEF, env_id_base=(1 << 33) + 5)
         env.reset()
         a0 = env.sample_actions().cpu().numpy()
@@ -555,9 +557,21 @@ def test_custom_arm_runtime_specialisation(mt, x, fk_mode):
 def test_runtime_specialisation_matches_runtime_table_path(mt):
     """Same arm, same seed: the NVRTC-specialised kernels and the run-time-table kernels walk the same
     trajectory (rewards / done / alive identical, observations to fp32 rounding), also through auto-reset."""
+    arm = mt.ArmSpec(dh=_CUSTOM_DH, obs_frame=4, ground_frames=(4, 5), catch_frame=5, radius=0.9, catch_tol=0.15)
+    _specialised_equals_runtime_table(mt, arm)
+
+
+@pytest.mark.parametrize("J", [2, 3, 4, 5, 6, 7, 8])
+def test_runtime_specialisation_matches_runtime_table_path_at_every_joint_count(mt, J):
+    """The same comparison for the table of every joint count in tests/arms.py (Preset<1000 + J> against
+    step_kernel<J, 0, ...>), whose inner rows hold every alpha and offset the specialisation folds."""
+    from arms import arm_pair
+    _specialised_equals_runtime_table(mt, arm_pair(J)[1])
+
+
+def _specialised_equals_runtime_table(mt, arm):
     import torch
     n, x = 4096 + 5, 12
-    arm = mt.ArmSpec(dh=_CUSTOM_DH, obs_frame=4, ground_frames=(4, 5), catch_frame=5, radius=0.9, catch_tol=0.15)
     a = mt.BatchedEnvs(n, x, arm=arm, device=0, fk_mode=3, seed=5, auto_reset=True, horizon=9)
     b = mt.BatchedEnvs(n, x, arm=arm, device=0, fk_mode=1, seed=5, auto_reset=True, horizon=9)
     a.reset(); b.reset()

@@ -404,7 +404,8 @@ def test_multi_gpu_c_host_runs(mt, tmp_path):
 @pytest.mark.parametrize("arm_name,n,x,obs,oar", [("ref", 150_003, 10, True, False), ("ref", 40_000, 10, False, False),
                                                   ("ref", 5_000, 7, True, True), ("ref", 33, 32, True, False),
                                                   ("ur5", 90_001, 20, True, True), ("ur5", 3_000, 5, False, False),
-                                                  ("ref-jit", 9_000, 7, True, False), ("custom-jit", 70_000, 12, True, True)])
+                                                  ("ref-jit", 9_000, 7, True, False), ("custom-jit", 70_000, 12, True, True),
+                                                  ("j2-jit", 9_001, 1, True, False), ("j8-jit", 70_003, 32, True, True)])
 def test_multi_step_rollout_equals_per_step_launches(mt, arm_name, n, x, obs, oar):
     """mt_rollout_random(k) keeps a tile's pose / alive word / total reward in registers and its objectives in shared
     memory for all k steps (one launch); MT_ROLLOUT_PERSISTENT=0 forces k launches of the step kernel.  Outputs of
@@ -417,6 +418,9 @@ def test_multi_step_rollout_equals_per_step_launches(mt, arm_name, n, x, obs, oa
                             (0.0, -np.pi / 2, 0.20, -np.pi / 2), (0.10, 0.0, 0.05, 0.0)),
                         obs_frame=4, ground_frames=(4, 5), catch_frame=5, radius=0.9, catch_tol=0.15)
     arm = mt.UR5_ARM if arm_name == "ur5" else (custom if arm_name == "custom-jit" else mt.REFERENCE_ARM)
+    if arm_name in ("j2-jit", "j8-jit"):            # the 2- and 8-joint tables of tests/arms.py
+        from arms import arm_pair
+        arm = arm_pair(int(arm_name[1]))[1]
     kw = dict(arm=arm, device=0, seed=13, auto_reset=True, horizon=4, obs_after_reset=oar)
     res = []
     for persistent in ("1", "0"):
@@ -463,16 +467,22 @@ def test_policy_loop_example_feeds_fresh_observations(mt):
 
 
 @pytest.mark.parametrize("arm_name,x,lo,hi", [("ref", 10, -180, 180), ("ref", 10, -90, 45), ("ref", 7, -1000, 1000),
-                                              ("ur5", 20, -180, 180), ("ur5", 6, -30, 400)])
+                                              ("ur5", 20, -180, 180), ("ur5", 6, -30, 400), ("j7", 13, -180, 180),
+                                              ("j8", 32, -180, 180)])
 def test_action_sincos_table_is_a_pure_memoisation(mt, arm_name, x, lo, hi):
     """In-kernel actions are integer degrees, so the kernels look the sin / cos of the joint targets up in a per-block
     table filled by the very evaluation they would otherwise run per env and step (ActionTrig, mt_step.cuh).  With the
     table (default), without it (MT_ACTION_TABLE=0), and through mt_step on the sampled actions (which always
-    evaluates), every output must be bit-identical -- also for other action ranges and for a range too wide to tabulate."""
+    evaluates), every output must be bit-identical -- also for other action ranges and for a range too wide to tabulate.
+    The 7-joint table runs the per-step run-time-table kernels (fk_mode 1), the 8-joint one NVRTC's (fk_mode 3)."""
     import torch
+    from arms import arm_pair
     arm = mt.UR5_ARM if arm_name == "ur5" else mt.REFERENCE_ARM
+    if arm_name in ("j7", "j8"):
+        arm = arm_pair(int(arm_name[1]))[1]
+    fk_mode = {"j7": 1, "j8": 3}.get(arm_name, 0)         # run-time table for the 7-joint arm, NVRTC for the 8-joint one
     n = 20_000
-    kw = dict(arm=arm, device=0, seed=21, auto_reset=True, horizon=6, action_low=lo, action_high=hi)
+    kw = dict(arm=arm, device=0, seed=21, auto_reset=True, horizon=6, action_low=lo, action_high=hi, fk_mode=fk_mode)
     runs = []
     for table in ("1", "0", "step"):
         os.environ["MT_ACTION_TABLE"] = "0" if table == "0" else "1"

@@ -1,6 +1,7 @@
 """Property tests of the CPU oracle (hypothesis): invariants the reference's geometry implies, used to
 cross-check the restatement beyond the recorded traces."""
 import numpy as np
+import pytest
 from hypothesis import given, settings, strategies as st
 
 from oracle import OracleEnvs, REFERENCE_ARM, fk_frames, observations
@@ -63,3 +64,33 @@ def test_ground_flag_is_sticky_over_the_route(g, a):
     under = min(start[3, 2], start[4, 2], end[3, 2], end[4, 2]) < 0
     assert (not under) or bool(r.neg[0])
     assert r.reward[0] == -1 if r.neg[0] else r.reward[0] in (0, 1)
+
+
+@pytest.mark.parametrize("J", [2, 3, 8])
+def test_frame_selectors_pick_the_frame_of_that_number(J):
+    """Frame k is the origin after the first k DH rows (frame 0 the base): every selector in 0 .. J must observe from,
+    and catch with, exactly fk_frames(goals)[:, k] -- including frame 1, which joints_coordinates has no row for."""
+    import dataclasses
+    from arms import arm_pair
+    spec0, _ = arm_pair(J)
+    rng = np.random.RandomState(J)
+    n, x = 64, 5
+    for f in range(J + 1):
+        spec = dataclasses.replace(spec0, obs_frame=f, catch_frame=f)
+        env = OracleEnvs(n, x, spec=spec)
+        pts = rng.uniform(-1, 1, size=(n, x, 3)) * spec.radius
+        env.reset(points=pts)
+        np.testing.assert_array_equal(env.get_observations(),
+                                      observations(fk_frames(np.zeros((n, J)), spec)[:, f], pts, np.ones((n, x), bool)))
+        act = rng.randint(-180, 180, size=(n, J)).astype(np.float64)
+        frames = fk_frames(act, spec)
+        # objective 0 of every other env sits just inside the catch cube of frame f at the new pose
+        env.points[::2, 0] = frames[::2, f] + 0.5 * spec.catch_tol
+        points_before, alive_before = env.points.copy(), env.alive.copy()
+        r = env.step(act)
+        np.testing.assert_array_equal(r.obs, observations(frames[:, f], points_before, alive_before))
+        caught = (np.abs(frames[:, f][:, None, :] - points_before) <= spec.catch_tol).all(axis=-1)
+        np.testing.assert_array_equal(r.alive, alive_before & ~caught)
+        assert caught[::2, 0].all()
+        np.testing.assert_array_equal(env.get_observations(), observations(frames[:, f], env.points, env.alive))
+    np.testing.assert_array_equal(r.frames, frames)                   # what the GPU comparisons read the anchor from
