@@ -5,7 +5,9 @@ The reference draws actions from the global MT19937 stream
 (``np.random.randint(-180, 180)``, manytor.py:215-217), which a GPU cannot
 reproduce in lock step; the CUDA path uses a counter-based Philox stream keyed
 by (seed, global env id, step index) instead.  This restates that stream in
-integer arithmetic so tests can check the device's actions bit for bit.
+integer arithmetic so tests can check the device's actions bit for bit, and
+restates the objective map of the device's auto-reset (``device_points``) in
+fp64 so tests can check the refreshed objectives value by value.
 Pinned by the Random123 known-answer vectors in tests/test_philox.py.
 """
 from __future__ import annotations
@@ -57,3 +59,34 @@ def device_actions(seed: int, env_ids: np.ndarray, step_index: int, n_joints: in
             if j < n_joints:
                 out[:, j] = low + ((w[i].astype(np.uint64) * span) >> np.uint64(32)).astype(np.int64)
     return out
+
+
+def _u01(w: np.ndarray) -> np.ndarray:
+    """mt_math.cuh ``uniform01``: the top 24 bits times 2^-24, exact in fp32 and fp64."""
+    return (w >> np.uint32(8)).astype(np.float64) * 2.0 ** -24
+
+
+def device_points(seed: int, env_ids: np.ndarray, episodes, x: int, radius: float = 51.3) -> np.ndarray:
+    """The (N, X, 3) objectives the device draws for the reset that starts episode ``episodes[i]`` of env
+    ``env_ids[i]`` (manytor_b200/csrc/mt_step.cuh: sample_point, called by reset_kernel and settle_step),
+    in fp64.  ``episodes`` is per env (or one value for all): the number of resets the env had before.
+
+    Counter (gid lo, gid hi, episode * 32 + objective mod 2^32, STREAM_POINTS), key (seed lo, seed hi);
+    words x, y, z of the block give r = min(R cbrt(1 - u01(x)), R), cos(theta) = u01(y) and
+    phi = 2 pi u01(z), where R is the fp32 radius the config holds.  The device evaluates the same map in
+    fp32 (cbrtf, sincospif, 1 - ct^2 as one FFMA), a few fp32 roundings of R from these values."""
+    env_ids = np.asarray(env_ids, dtype=np.uint64).reshape(-1)
+    n = env_ids.size
+    ep = np.broadcast_to(np.asarray(episodes, dtype=np.uint64).reshape(-1), (n,))
+    lo = np.repeat((env_ids & _MASK).astype(np.uint32)[:, None], x, axis=1)
+    hi = np.repeat((env_ids >> np.uint64(32)).astype(np.uint32)[:, None], x, axis=1)
+    ctr = ((ep[:, None] * np.uint64(32) + np.arange(x, dtype=np.uint64)[None, :]) & _MASK).astype(np.uint32)
+    k0 = np.full_like(lo, seed & 0xFFFFFFFF)
+    k1 = np.full_like(lo, (seed >> 32) & 0xFFFFFFFF)
+    wx, wy, wz, _ = philox4x32_10(lo, hi, ctr, np.full_like(lo, STREAM_POINTS), k0, k1)
+    big_r = float(np.float32(radius))
+    r = np.minimum(big_r * np.cbrt(1.0 - _u01(wx)), big_r)
+    ct = _u01(wy)
+    st = np.sqrt(np.maximum(1.0 - ct * ct, 0.0))          # ct has 24 bits: ct^2 and 1 - ct^2 are exact here
+    phi = 2.0 * np.pi * _u01(wz)
+    return np.stack([r * st * np.cos(phi), r * st * np.sin(phi), r * ct], axis=-1)

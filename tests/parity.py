@@ -29,6 +29,7 @@ class Report:
     hard_mismatch: int = 0             # must stay 0
     rewarded: int = 0                  # env-steps with reward +1 (oracle): catches were compared
     ground: int = 0                    # env-steps with ground contact (oracle): the ground test was compared
+    max_point_err: float = 0.0         # refreshed objectives against their fp64 restatement (Philox objectives)
     notes: list = field(default_factory=list)
 
     def ok(self) -> bool:
@@ -46,9 +47,10 @@ def reach_of(spec) -> float:
 
 
 def compare_step(rep: Report, spec, ora, r, points_before, alive_before, dev_obs, dev_reward, dev_done,
-                 dev_alive, dev_joints=None, scale=None):
+                 dev_alive, dev_joints=None, scale=None, obs_rows=None):
     """Compare one step.  `r` is the oracle StepResult; returns the bool mask of
-    envs whose flags differ (all of them near-threshold, or hard_mismatch grows)."""
+    envs whose flags differ (all of them near-threshold, or hard_mismatch grows).
+    The observations are compared on the rows `obs_rows` (default all; none when `dev_obs` is None)."""
     n, x = alive_before.shape
     reach = reach_of(spec)
     pos_tol = REL_POS_TOL * reach
@@ -80,7 +82,9 @@ def compare_step(rep: Report, spec, ora, r, points_before, alive_before, dev_obs
                          f"ground margin {r.ground_margin[i]:.3e}, catch margin {cm[i]:.3e}")
 
     # observations (computed from alive_before, which is kept in sync)
-    compare_obs(rep, spec, r.frames[:, spec.obs_frame], points_before, alive_before, dev_obs, r.obs)
+    if dev_obs is not None and (obs_rows is None or obs_rows.any()):
+        o = slice(None) if obs_rows is None else obs_rows
+        compare_obs(rep, spec, r.frames[o, spec.obs_frame], points_before[o], alive_before[o], dev_obs[o], r.obs[o])
     return bad
 
 
@@ -183,23 +187,111 @@ class ChunkedOracle:
         return StepResult(*[np.concatenate([getattr(r, f) for r in rs], axis=0) for f in StepResult._fields])
 
 
+def _seed_late_episode(env, ora, rs, n, x, horizon, alive_p=0.35):
+    """Put every env somewhere inside an episode: random poses, a random subset of objectives already
+    collected (many envs one catch away from termination), random episode lengths up to the horizon --
+    so that the few steps of a test see terminations, truncations and fresh objectives.  `ora` is a
+    ChunkedOracle."""
+    goals = rs.randint(-180, 180, size=(n, ora.spec.n_joints)).astype(np.float64)
+    alive = rs.rand(n, x) < alive_p
+    alive[np.arange(n), rs.randint(0, x, size=n)] = True               # at least one objective alive
+    total = -rs.randint(0, 40, size=n).astype(np.float64)
+    ep = rs.randint(0, horizon, size=n)
+    env.set_state(goals=goals.astype(np.float32), alive=alive, total_reward=total.astype(np.float32),
+                  ep_len=ep.astype(np.int32))
+    from oracle.manytor_oracle import joints_coordinates
+    for (a, b), p in zip(ora.bounds, ora.parts):
+        p.goals = goals[a:b].copy()
+        p.alive = alive[a:b].copy()
+        p.total_reward = total[a:b].copy()
+        p.ep_len = ep[a:b].astype(np.int64)
+        p.joints = joints_coordinates(p.goals, p.spec)
+
+
+def point_tol_of(spec) -> float:
+    """Tolerance of a device-drawn objective against its fp64 restatement (oracle.philox.device_points), per
+    component: 4 fp32 ulps of the radius.  cbrtf and sincospif are within 1 ulp, the rest adds a few roundings,
+    and 1 - ct^2 is one FFMA (no cancellation near the pole)."""
+    return 4.0 * float(np.spacing(np.float32(spec.radius)))
+
+
+def philox_fresh(seed: int, env_ids, x: int, radius: float):
+    """`fresh(episode, ended)` for the loops below: the fp64 objectives (N, X, 3) the device draws for the reset that
+    starts episode `episode[i]` of each ended env (rows outside `ended` are zeros)."""
+    from oracle.philox import device_points
+    env_ids = np.asarray(env_ids, dtype=np.uint64)
+
+    def fresh(episode, ended):
+        out = np.zeros((env_ids.size, x, 3))
+        out[ended] = device_points(seed, env_ids[ended], episode[ended], x, radius)
+        return out
+    return fresh
+
+
+def _zero_pose_obs(spec, points):
+    """The first observation of an episode (obs_after_reset): objectives `points` (M, X, 3), all alive, seen from
+    the obs frame at the zero pose.  Returns (anchor (M, 3), observations (M, 3X))."""
+    from oracle.manytor_oracle import fk_frames, observations
+    m, x = points.shape[:2]
+    anchor = np.repeat(fk_frames(np.zeros((1, spec.n_joints)), spec)[:, spec.obs_frame], m, axis=0)
+    return anchor, observations(anchor, points, np.ones((m, x), dtype=bool))
+
+
+def _check_fresh_points(rep, dev, want, exact, tol):
+    """Refreshed objectives: bit-exact against an uploaded stream, within `tol` of the fp64 restatement otherwise."""
+    if exact:
+        np.testing.assert_array_equal(dev, np.float32(want))
+        return
+    err = float(np.abs(dev.astype(np.float64) - want).max()) if dev.size else 0.0
+    rep.max_point_err = max(rep.max_point_err, err)
+    if err > tol:
+        rep.hard_mismatch += 1
+        rep.notes.append(f"refreshed objective off by {err:.3e} > {tol:.3e}")
+
+
+def _new_stats():
+    return dict(env_steps=0, episodes=0, terminated=0, reward_sum=0, length_sum=0, catches=0, ground_steps=0,
+                live_reward_sum=0)
+
+
+def _fold_ended(stats, x, r, ended, total, ep_len):
+    stats["episodes"] += int(ended.sum())
+    stats["terminated"] += int(r.done.sum())
+    stats["reward_sum"] += int(total[ended].sum())
+    stats["length_sum"] += int(ep_len[ended].sum())
+    stats["catches"] += int((x - r.alive[ended].sum(axis=1)).sum())
+
+
 def lockstep_auto_reset(env, ora, spec, stream, actions_fn, steps: int, horizon: int, rep: Report | None = None,
-                        check_points: bool = True):
-    """Device auto-reset (in-kernel, objectives from the uploaded `stream` (E, N, X, 3)) against the oracle
-    reset on the host with the same sets.  The device must already hold set 0 (env.reset() after
-    set_objective_stream) and the oracle too.  Returns (report, expected statistics, reward slack, forked):
-    a near-threshold catch/done flip changes WHICH envs reset, after which the two sides are no longer
-    comparable -- the loop stops there and says so (`forked`)."""
+                        check_points: bool = True, fresh=None, device_step=None, episode=None):
+    """Device auto-reset (in-kernel) against the oracle reset on the host with the same objectives.
+
+    The fresh objectives of the e-th reset of an env come either from the uploaded `stream` (E, N, X, 3), set e mod E,
+    which the device must copy bit for bit; or, with `stream` None, from `fresh(episode, ended)` -> (N, X, 3) fp64,
+    the restated on-device draw (`philox_fresh`): the oracle resets with its fp32 rounding and the device's objectives
+    must lie within `point_tol_of(spec)` of it.  `episode` (N,) counts each env's resets so far and is advanced in
+    place; by default both sides have had exactly one (episode 0).  `device_step(act)` -> (obs, reward, done) advances the device (default `env.step`).  With
+    obs_after_reset an ended env's observation is the first one of its next episode: it is compared with the
+    oracle's observation of the fresh objectives from the zero pose.
+
+    Returns (report, expected statistics (all eight words), reward slack, forked): a near-threshold catch/done flip
+    changes WHICH envs reset, after which the two sides are no longer comparable -- the loop stops there and says
+    so (`forked`)."""
     rep = rep or Report()
     n, x = ora.n, ora.x
-    sets = stream.shape[0]
-    episode = np.ones(n, dtype=np.int64)                   # resets so far
-    stats = dict(env_steps=0, episodes=0, terminated=0, reward_sum=0, length_sum=0, catches=0)
+    if stream is not None:
+        sets = stream.shape[0]
+        fresh = lambda ep, ended: stream[ep % sets, np.arange(n)]
+    device_step = device_step or (lambda a: env.step(a.astype(np.float32)))
+    oar = bool(env.cfg.obs_after_reset)
+    tol = point_tol_of(spec)
+    episode = np.ones(n, dtype=np.int64) if episode is None else episode      # resets so far
+    stats = _new_stats()
     slack, forked = 0, False
     for t in range(steps):
         act = np.float32(np.asarray(actions_fn(t))).astype(np.float64)
         alive_before, points_before = ora.alive.copy(), ora.points.copy()
-        obs, rew, done = (o.cpu().numpy() for o in env.step(act.astype(np.float32)))
+        obs, rew, done = (o.cpu().numpy() for o in device_step(act))
         r = ora.step(act)
         ep_len, total = ora.ep_len, ora.total_reward
         trunc = (ep_len >= horizon) & ~r.done if horizon > 0 else np.zeros(n, dtype=bool)
@@ -207,8 +299,11 @@ def lockstep_auto_reset(env, ora, spec, stream, actions_fn, steps: int, horizon:
         st = env.get_state()
         dev_alive_after = alive_bits_to_matrix(st["alive"].cpu().numpy(), x)
         dev_alive = np.where(ended[:, None], r.alive, dev_alive_after)       # ended envs were reset on the device
-        bad = compare_step(rep, spec, ora, r, points_before, alive_before, obs, rew, done, dev_alive, None)
+        keep_obs = ~ended if oar else None
+        bad = compare_step(rep, spec, ora, r, points_before, alive_before, obs, rew, done, dev_alive, None,
+                           obs_rows=keep_obs)
         stats["env_steps"] += n
+        stats["ground_steps"] += int(np.where(bad, rew == -1, r.neg).sum())   # the device's own flag where it flipped
         if not rep.ok():
             break
         if bad.any():
@@ -221,20 +316,104 @@ def lockstep_auto_reset(env, ora, spec, stream, actions_fn, steps: int, horizon:
                 env.set_state(total_reward=total, mask=bad & ~ended)
         assert np.array_equal((done & 2).astype(bool), trunc), "truncation flags differ"
         if ended.any():
-            stats["episodes"] += int(ended.sum())
-            stats["terminated"] += int(r.done.sum())
-            stats["reward_sum"] += int(total[ended].sum())
-            stats["length_sum"] += int(ep_len[ended].sum())
-            stats["catches"] += int((x - r.alive[ended].sum(axis=1)).sum())
-            fresh = stream[episode % sets, np.arange(n)]
-            ora.reset(mask=ended, points=fresh)
+            _fold_ended(stats, x, r, ended, total, ep_len)
+            pts = fresh(episode, ended)
+            ora.reset(mask=ended, points=np.float32(pts).astype(np.float64))
             episode[ended] += 1
             assert np.all(dev_alive_after[ended]) and np.all(st["goals"].cpu().numpy()[ended] == 0)
             assert np.all(st["ep_len"].cpu().numpy()[ended] == 0) and np.all(st["total_reward"].cpu().numpy()[ended] == 0)
             if check_points:
-                np.testing.assert_array_equal(env.get_points(zero_dead=False).cpu().numpy()[ended],
-                                              np.float32(fresh[ended]))
+                _check_fresh_points(rep, env.get_points(zero_dead=False).cpu().numpy()[ended], pts[ended],
+                                    stream is not None, tol)
+            if oar:
+                anchor, want = _zero_pose_obs(spec, ora.points[ended])
+                compare_obs(rep, spec, anchor, ora.points[ended], np.ones((int(ended.sum()), x), dtype=bool),
+                            obs[ended], want)
+    stats["live_reward_sum"] = int(ora.total_reward.sum())
     return rep, stats, slack, forked
+
+
+def _rows(r, keep):
+    return type(r)(*[f[keep] for f in r])
+
+
+def lockstep_chunked(env, ora, spec, fresh, seed: int, k: int, chunks: int, horizon: int, rep: Report | None = None,
+                     write_obs: bool = True, episode=None):
+    """`chunks` calls of env.rollout_random(k) (in-kernel actions, auto-reset, Philox objectives) against the oracle
+    advanced k steps per call with the restated actions (oracle.philox.device_actions at env.step_index + s) and
+    objectives (`fresh`, as in lockstep_auto_reset).  Only the last step of a call can be read back: its outputs
+    are compared (compare_step), and so are the full state -- goals, alive words, total_reward and ep_len exactly
+    -- and the objectives refreshed during the call.  `episode` is as in lockstep_auto_reset.
+
+    A near-threshold flip inside a call cannot be re-synchronised.  Every env depends on its own id alone, so an
+    env whose state differs after a call in which one of its margins came within THRESH_TOL is dropped from all
+    later comparisons and counted as a near-threshold flip; a difference without such a margin is a hard mismatch.
+    Returns (report, expected statistics, dropped mask): the statistics are comparable when nothing was dropped."""
+    from oracle.philox import device_actions
+    rep = rep or Report()
+    n, x, J = ora.n, ora.x, spec.n_joints
+    ids = np.uint64(env.cfg.env_id_base) + np.arange(n, dtype=np.uint64)
+    oar = bool(env.cfg.obs_after_reset) and write_obs
+    thr = THRESH_TOL * (reach_of(spec) / 55.6)
+    tol = point_tol_of(spec)
+    episode = np.ones(n, dtype=np.int64) if episode is None else episode
+    keep = np.ones(n, dtype=bool)
+    stats = _new_stats()
+    s0 = env.step_index
+    for c in range(chunks):
+        out = env.rollout_random(k, write_obs=write_obs)
+        obs = out[0].cpu().numpy() if write_obs else None
+        rew, done = out[1].cpu().numpy(), out[2].cpu().numpy()
+        near = np.zeros(n, dtype=bool)
+        refreshed = np.zeros(n, dtype=bool)
+        last_pts = np.zeros((n, x, 3))
+        for s in range(k):
+            act = device_actions(seed, ids, s0 + c * k + s, J).astype(np.float64)
+            alive_before, points_before = ora.alive.copy(), ora.points.copy()
+            r = ora.step(act)
+            ep_len, total = ora.ep_len, ora.total_reward
+            trunc = (ep_len >= horizon) & ~r.done if horizon > 0 else np.zeros(n, dtype=bool)
+            ended = r.done | trunc
+            cm = np.where(alive_before, np.abs(r.catch_margin), np.inf).min(axis=1)
+            near |= (r.ground_margin < thr) | (cm < thr)
+            stats["env_steps"] += n
+            stats["ground_steps"] += int(r.neg.sum())
+            if ended.any():
+                _fold_ended(stats, x, r, ended, total, ep_len)
+                pts = fresh(episode, ended)
+                ora.reset(mask=ended, points=np.float32(pts).astype(np.float64))
+                episode[ended] += 1
+                refreshed |= ended
+                last_pts[ended] = pts[ended]
+        st = {key: v.cpu().numpy() for key, v in env.get_state().items()}
+        dev_alive_after = alive_bits_to_matrix(st["alive"], x)
+        differs = ((st["goals"] != np.float32(ora.goals)).any(axis=1) | (dev_alive_after != ora.alive).any(axis=1) |
+                   (st["total_reward"] != np.float32(ora.total_reward)) | (st["ep_len"] != ora.ep_len)) & keep
+        hard = differs & ~near
+        if hard.any():
+            rep.hard_mismatch += int(hard.sum())
+            i = int(np.nonzero(hard)[0][0])
+            rep.notes.append(f"call {c}: env {i} state differs with no margin near a threshold")
+        rep.near_threshold += int((differs & near).sum())
+        keep &= ~differs
+        # the last step of the call, on the envs both sides still agree on
+        dev_alive = np.where(ended[:, None], r.alive, dev_alive_after)
+        rk = _rows(r, keep)
+        compare_step(rep, spec, None, rk, points_before[keep], alive_before[keep], None if obs is None else obs[keep],
+                     rew[keep], done[keep], dev_alive[keep], None, obs_rows=(~ended[keep] if oar else None))
+        rep.env_steps += (k - 1) * int(keep.sum())
+        if not np.array_equal((done[keep] & 2).astype(bool), trunc[keep]):
+            rep.hard_mismatch += 1
+            rep.notes.append(f"call {c}: truncation flags differ")
+        if oar and (ended & keep).any():
+            e = ended & keep
+            anchor, want = _zero_pose_obs(spec, ora.points[e])
+            compare_obs(rep, spec, anchor, ora.points[e], np.ones((int(e.sum()), x), dtype=bool), obs[e], want)
+        sel = refreshed & keep
+        if sel.any():
+            _check_fresh_points(rep, env.get_points(zero_dead=False).cpu().numpy()[sel], last_pts[sel], False, tol)
+    stats["live_reward_sum"] = int(ora.total_reward.sum())
+    return rep, stats, ~keep
 
 
 def half_ball_points(rs, shape, radius=51.3):

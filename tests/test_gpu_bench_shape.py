@@ -18,7 +18,7 @@ import pytest
 
 from oracle import ArmSpec as OArm, REFERENCE_ARM, UR5_ARM
 
-from parity import ChunkedOracle, Report, half_ball_points, lockstep_auto_reset
+from parity import ChunkedOracle, Report, _seed_late_episode, half_ball_points, lockstep_auto_reset
 
 pytestmark = pytest.mark.gpu
 
@@ -32,26 +32,6 @@ def mt():
     import manytor_b200
     manytor_b200.load_library()
     return manytor_b200
-
-
-def _seed_late_episode(env, ora, rs, n, x, horizon, alive_p=0.35):
-    """Put every env somewhere inside an episode: random poses, a random subset of objectives already
-    collected (many envs one catch away from termination), random episode lengths up to the horizon --
-    so that the few steps of the test see terminations, truncations and fresh objectives."""
-    goals = rs.randint(-180, 180, size=(n, ora.spec.n_joints)).astype(np.float64)
-    alive = rs.rand(n, x) < alive_p
-    alive[np.arange(n), rs.randint(0, x, size=n)] = True               # at least one objective alive
-    total = -rs.randint(0, 40, size=n).astype(np.float64)
-    ep = rs.randint(0, horizon, size=n)
-    env.set_state(goals=goals.astype(np.float32), alive=alive, total_reward=total.astype(np.float32),
-                  ep_len=ep.astype(np.int32))
-    from oracle.manytor_oracle import joints_coordinates
-    for (a, b), p in zip(ora.bounds, ora.parts):
-        p.goals = goals[a:b].copy()
-        p.alive = alive[a:b].copy()
-        p.total_reward = total[a:b].copy()
-        p.ep_len = ep[a:b].astype(np.int64)
-        p.joints = joints_coordinates(p.goals, p.spec)
 
 
 def _bench_shape_run(mt, n, x, steps, horizon, spec, arm, fk_mode, seed, scale=1.0, sets=3, alive_p=0.35):
