@@ -22,7 +22,9 @@
  *
  * Array layouts (row-major, fp32 unless noted)
  *   actions [N][J]        obs [N][3*X]  (per objective: distance, r, theta;
- *   reward  [N]                          zeros for a dead objective, manytor.py:141-153)
+ *   reward  [N]                          zeros for a dead objective, manytor.py:141-153),
+ *                         elements of the handle's format: fp32, or binary16 when
+ *                         mt_config.obs_dtype = MT_OBS_F16 (6*X bytes per row)
  *   done    [N] uint8     bit0 = terminated (no objective alive, manytor.py:170-171,
  *                                  or ground contact when terminate_on_ground)
  *                         bit1 = truncated (episode reached cfg.horizon steps)
@@ -38,9 +40,13 @@
 extern "C" {
 #endif
 
-#define MT_ABI_VERSION 2
+#define MT_ABI_VERSION 3
 #define MT_MAX_JOINTS 8
 #define MT_MAX_OBJ 32
+
+/* mt_config.obs_dtype: the element type of every observation a handle writes */
+#define MT_OBS_F32 0   /* float                                                         */
+#define MT_OBS_F16 1   /* IEEE binary16, rounded to nearest even from the fp32 result   */
 
 typedef enum mt_status {
     MT_OK = 0,
@@ -84,6 +90,9 @@ typedef struct mt_config {
     int32_t action_low;            /* action_sample range [low, high) (-180, 180, :216)   */
     int32_t action_high;
     uint64_t seed;                 /* Philox key for on-device actions / objectives       */
+    int32_t obs_dtype;             /* MT_OBS_F32 (default) or MT_OBS_F16: the format of the
+                                      obs buffers of mt_step, mt_observe, mt_rollout_random
+                                      and mt_step_host (the values are the fp32 ones rounded) */
 } mt_config;
 
 /* Episode statistics; summed over the shard, reducible across shards by plain
@@ -136,12 +145,12 @@ int mt_set_step_index(mt_env *env, uint64_t value);
 int mt_reset(mt_env *env, const uint8_t *mask_dev, void *stream);
 
 /* Environment.get_observations -- manytor.py:141-153: current obs of every env. */
-int mt_observe(mt_env *env, float *obs_dev, void *stream);
+int mt_observe(mt_env *env, void *obs_dev, void *stream);
 
 /* Environment.step / Multienv.step -- manytor.py:255-260, 115-122: ONE fused kernel
  * (FK over the 25 sub-poses, ground flag, obs2, catch, reward, done, auto-reset).
  * joints_dev may be NULL. */
-int mt_step(mt_env *env, const float *actions_dev, float *obs_dev, float *reward_dev,
+int mt_step(mt_env *env, const float *actions_dev, void *obs_dev, float *reward_dev,
             uint8_t *done_dev, float *joints_dev, void *stream);
 
 /* Environment.action_sample / Multienv.action_sample -- manytor.py:215-217, 111-113:
@@ -160,7 +169,7 @@ int mt_sample_actions(mt_env *env, float *actions_dev, void *stream);
  * (observations, reward, done) leaves the SM each step.  Results are bit-identical to
  * n_steps launches of the step kernel, which run-time DH tables without NVRTC still
  * take (MT_ROLLOUT_PERSISTENT=0 forces them for everyone). */
-int mt_rollout_random(mt_env *env, int32_t n_steps, float *obs_dev, float *reward_dev,
+int mt_rollout_random(mt_env *env, int32_t n_steps, void *obs_dev, float *reward_dev,
                       uint8_t *done_dev, void *stream);
 
 /* Host-buffer step: actions_host/obs_host/reward_host/done_host must be pinned
@@ -168,7 +177,7 @@ int mt_rollout_random(mt_env *env, int32_t n_steps, float *obs_dev, float *rewar
  * internal streams so copies overlap the kernels; synchronous on return.  Ordered after
  * everything submitted earlier to the legacy default stream / blocking streams (work on
  * cudaStreamNonBlocking streams must be synchronised by the caller). */
-int mt_step_host(mt_env *env, const float *actions_host, float *obs_host, float *reward_host,
+int mt_step_host(mt_env *env, const float *actions_host, void *obs_host, float *reward_host,
                  uint8_t *done_host);
 /* mt_step_host has two implementations with identical results -- chunks staged through device buffers,
  * or one launch reading and writing the pinned host buffers across PCIe itself -- and by default times
@@ -238,7 +247,8 @@ int mt_joints(mt_env *env, const float *goals_dev, float *out_dev, int64_t m, vo
 int mt_r_theta(const float *v1_dev, const float *v2_dev, float *out_dev, int64_t m, void *stream);
 
 /* Introspection for bench.py: kernels launched by this handle since create, and
- * the algorithmic bytes per env-step of mt_step (SURVEY.md section 8d). */
+ * the algorithmic bytes per env-step of mt_step (SURVEY.md section 8d): 12J + 24X + 21
+ * for an fp32 handle, 12J + 18X + 21 for a binary16 one (observations 6X instead of 12X). */
 int64_t mt_launch_count(const mt_env *env);
 int64_t mt_bytes_per_env_step(const mt_env *env, int32_t actions_from_hbm, int32_t obs_written);
 /* Device time (ms) of the step kernels launched by the last mt_rollout_random /

@@ -13,7 +13,9 @@ from . import build as _build
 MT_MAX_JOINTS = 8
 MT_MAX_OBJ = 32
 MT_STATS_WORDS = 8
-MT_ABI_VERSION = 2
+MT_ABI_VERSION = 3
+MT_OBS_F32 = 0
+MT_OBS_F16 = 1
 
 STATS_FIELDS = ("env_steps", "episodes", "terminated", "reward_sum", "length_sum", "catches",
                 "ground_steps", "live_reward_sum")
@@ -43,6 +45,7 @@ class MtConfig(C.Structure):
         ("action_low", C.c_int32),
         ("action_high", C.c_int32),
         ("seed", C.c_uint64),
+        ("obs_dtype", C.c_int32),
     ]
 
 

@@ -51,10 +51,21 @@ UR5_ARM = ArmSpec(
     radius=0.81725, catch_tol=0.81725 * 8.0 / 51.3)
 
 
+# observation dtype -> mt_config.obs_dtype
+OBS_DTYPES = {torch.float32: _lib.MT_OBS_F32, torch.float16: _lib.MT_OBS_F16}
+
+
+def obs_format(dtype) -> int:
+    """mt_config.obs_dtype of a torch dtype; anything but float32 / float16 (bf16 included) is refused."""
+    if dtype not in OBS_DTYPES:
+        raise ValueError(f"obs_dtype must be torch.float32 or torch.float16, not {dtype}")
+    return OBS_DTYPES[dtype]
+
+
 def make_config(n_envs: int, obj_number: int, arm: ArmSpec, device: int, env_id_base: int = 0,
                 horizon: int = 0, auto_reset: bool = False, terminate_on_ground: bool = False,
                 obs_after_reset: bool = False, seed: int = 0, fk_mode: int = 0, substeps: int = 25,
-                action_low: int = -180, action_high: int = 180) -> MtConfig:
+                action_low: int = -180, action_high: int = 180, obs_dtype=torch.float32) -> MtConfig:
     cfg = _lib.default_config()
     cfg.device = int(device)
     cfg.n_envs = int(n_envs)
@@ -78,6 +89,7 @@ def make_config(n_envs: int, obj_number: int, arm: ArmSpec, device: int, env_id_
     cfg.action_low = int(action_low)
     cfg.action_high = int(action_high)
     cfg.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+    cfg.obs_dtype = obs_format(obs_dtype)
     return cfg
 
 
@@ -133,13 +145,20 @@ class PinnedArray:
 
 
 class BatchedEnvs:
-    """N environments in HBM advanced by one fused kernel per step."""
+    """N environments in HBM advanced by one fused kernel per step.
+
+    obs_dtype: torch.float32 (default) or torch.float16.  Every observation this object returns
+    (step, observe, reset(returnable=True), rollout_random, step_host) is of that dtype; float16
+    observations are the float32 ones rounded to nearest even, written by the kernels themselves
+    (half the bytes to HBM and across PCIe)."""
 
     def __init__(self, n_envs: int, obj_number: int = 10, arm: ArmSpec = REFERENCE_ARM, device=None,
                  env_id_base: int = 0, horizon: int = 0, auto_reset: bool = False,
                  terminate_on_ground: bool = False, obs_after_reset: bool = False, seed: int = 0,
                  fk_mode: int = 0, substeps: int = 25, action_low: int = -180, action_high: int = 180,
-                 lib_path: Optional[str] = None):
+                 lib_path: Optional[str] = None, obs_dtype=torch.float32):
+        obs_format(obs_dtype)
+        self.obs_dtype = obs_dtype
         self._lib = _lib.load(lib_path)
         self._h = C.c_void_p()
         dev = _device_index(device)
@@ -148,7 +167,7 @@ class BatchedEnvs:
         self.n, self.x, self.j = int(n_envs), int(obj_number), arm.n_joints
         self.cfg = make_config(n_envs, obj_number, arm, dev, env_id_base, horizon, auto_reset,
                                terminate_on_ground, obs_after_reset, seed, fk_mode, substeps,
-                               action_low, action_high)
+                               action_low, action_high, obs_dtype)
         _lib.check(self._lib.mt_create(C.byref(self.cfg), C.byref(self._h)))
         self._obs = self._reward = self._done = self._joints = self._actions = None
         self._stream_keepalive = None
@@ -195,7 +214,7 @@ class BatchedEnvs:
             self._reward = self._empty((self.n,), torch.float32)
             self._done = self._empty((self.n,), torch.uint8)
         if want_obs and self._obs is None:
-            self._obs = self._empty((self.n, 3 * self.x), torch.float32)
+            self._obs = self._empty((self.n, 3 * self.x), self.obs_dtype)
         if want_joints and self._joints is None:
             self._joints = self._empty((self.n, self.j, 3), torch.float32)
 
@@ -212,15 +231,18 @@ class BatchedEnvs:
         return None
 
     def observe(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Environment.get_observations (manytor.py:141-153) for every env -> (N, 3X)."""
-        out = out if out is not None else self._empty((self.n, 3 * self.x), torch.float32)
+        """Environment.get_observations (manytor.py:141-153) for every env -> (N, 3X) of obs_dtype."""
+        if out is None:
+            out = self._empty((self.n, 3 * self.x), self.obs_dtype)
+        elif out.dtype != self.obs_dtype:
+            raise ValueError(f"observe(out=...) needs a {self.obs_dtype} buffer (this handle's obs_dtype), got {out.dtype}")
         _lib.check(self._lib.mt_observe(self._h, self._p(out), self._stream()))
         return out
 
     def step(self, actions, joints: bool = False, write_obs: bool = True):
         """Environment.step / Multienv.step (manytor.py:255-260, 115-122).
 
-        actions: (N, J) degrees.  Returns (obs (N,3X) f32, reward (N,) f32,
+        actions: (N, J) degrees.  Returns (obs (N,3X) obs_dtype, reward (N,) f32,
         done (N,) u8 [, joints (N,J,3)]) -- views of buffers this object reuses
         on the next step.
         """
@@ -268,7 +290,8 @@ class BatchedEnvs:
         io = self._host_io.get(write_obs)
         if io is None:                                     # buffers and addresses once: a batch of one is pure latency
             act = self.pinned("actions", (self.n, self.j), np.float32)
-            obs = self.pinned("obs", (self.n, 3 * self.x), np.float32) if write_obs else None
+            obs_np = np.float16 if self.obs_dtype == torch.float16 else np.float32
+            obs = self.pinned("obs", (self.n, 3 * self.x), obs_np) if write_obs else None
             rew = self.pinned("reward", (self.n,), np.float32)
             done = self.pinned("done", (self.n,), np.uint8)
             addr = lambda a: self._pinned_ptr[id(a)] if a is not None else None

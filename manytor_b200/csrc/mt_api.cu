@@ -64,12 +64,13 @@ struct mt_env {
     mt_config cfg;
     long long n, n_pad, n_tiles;
     int arm;  // 0 = closed form reference arm, 2..8 = J (run-time DH table), >= 100 = preset arm
+    bool f16 = false;  // observations written as binary16 (mt_config.obs_dtype)
     // NVRTC-specialised step kernels for this handle's own DH table (mt_jit.cuh); the helper kernels
     // keep using the run-time table (`arm`)
     bool jit = false;
     int jit_id = 0, jit_x = 0;
     std::string jit_preset;
-    cudaKernel_t jit_kernel[2][2] = {};      // [in-kernel actions][observations written]
+    cudaKernel_t jit_kernel[2][2] = {};      // [in-kernel actions][observations written] (in the handle's format)
     cudaKernel_t jit_rollout[2] = {};        // multi-step rollout kernel, [observations written]
     bool jit_rollout_failed = false;
     float *goals = nullptr, *total_reward = nullptr, *points = nullptr;
@@ -99,7 +100,8 @@ struct mt_env {
     // mt_step_host variant: 0 staged, 1 zero-copy, 2 auto (decided from the first calls' own timings)
     int host_mode = 2, host_calls = 0;
     double host_best[2] = {1e30, 1e30};
-    float *h_actions = nullptr, *h_obs = nullptr, *h_reward = nullptr;
+    float *h_actions = nullptr, *h_reward = nullptr;
+    void *h_obs = nullptr;
     uint8_t *h_done = nullptr;
     // timing
     bool timing = false;
@@ -168,6 +170,7 @@ extern "C" int mt_config_init(mt_config *cfg) {
     cfg->action_low = -180;
     cfg->action_high = 180;
     cfg->seed = 0;
+    cfg->obs_dtype = MT_OBS_F32;
     return MT_OK;
 }
 
@@ -207,6 +210,8 @@ static int validate(const mt_config &c) {
     if (!(c.radius > 0.f) || !(c.catch_tol >= 0.f)) return fail(MT_ERR_INVALID, "radius must be > 0 and catch_tol >= 0");
     if (c.fk_mode < 0 || c.fk_mode > 3) return fail(MT_ERR_INVALID, "fk_mode must be 0, 1, 2 or 3");
     if (c.fk_mode == 2 && !is_reference_arm(c)) return fail(MT_ERR_INVALID, "fk_mode=2 (closed form) needs the reference DH table and frames");
+    if (c.obs_dtype != MT_OBS_F32 && c.obs_dtype != MT_OBS_F16)
+        return fail(MT_ERR_INVALID, "obs_dtype must be MT_OBS_F32 (0) or MT_OBS_F16 (1), not %d", c.obs_dtype);
     return MT_OK;
 }
 
@@ -284,6 +289,7 @@ extern "C" int mt_create(const mt_config *cfg, mt_env **out) {
     e->n = cfg->n_envs;
     e->n_tiles = (e->n + kTile - 1) / kTile;
     e->n_pad = e->n_tiles * kTile;
+    e->f16 = cfg->obs_dtype == MT_OBS_F16;
     e->arm = cfg->n_joints;                                   // run-time DH table
     if (cfg->fk_mode != 1) {
         if (is_reference_arm(*cfg)) e->arm = 0;               // closed form
@@ -385,7 +391,7 @@ extern "C" int mt_create(const mt_config *cfg, mt_env **out) {
             e->jit_id = runtime_table ? 1000 + nj : e->arm;
             e->jit_x = cfg->n_obj;                                    // compile-time X: unrolled objective walk
             e->jit_preset = runtime_table ? preset_source(e->jit_id, nj, e->base.arm) : std::string();
-            JitKernel k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, false, true, err);
+            JitKernel k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, false, true, e->f16, err);
             if (k.kernel) {
                 e->jit = true;
                 e->jit_kernel[0][1] = k.kernel;
@@ -499,7 +505,8 @@ __global__ void reset_kernel(const __grid_constant__ StepParams P, const uint8_t
     if (!P.ep_shift) P.counters[env] = 0u;
 }
 
-__global__ void observe_kernel(const __grid_constant__ StepParams P, int arm, float *obs) {
+template <bool F16>
+__global__ void observe_kernel(const __grid_constant__ StepParams P, int arm, void *obs) {
     const long long env = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (env >= P.n) return;
     const int x = P.n_obj, J = P.n_joints;
@@ -509,12 +516,12 @@ __global__ void observe_kernel(const __grid_constant__ StepParams P, int arm, fl
     pose_of(P, arm, g, f, nullptr);
     const uint32_t alive = alive_mask_of(P, P.alive[env]);
     const float *row = P.points + env * 3 * x;
-    float *dst = obs + env * 3 * x;
+    void *dst = obs_at<F16>(obs, (size_t)env * 3 * x);
     for (int pt = 0; pt < x; ++pt) {
         float px = row[point_index(P.pair_layout, pt, 0)], py = row[point_index(P.pair_layout, pt, 1)],
               pz = row[point_index(P.pair_layout, pt, 2)];
         one_objective<true>(px, py, pz, f, P.catch_tol, (alive >> pt) & 1u);
-        dst[pt * 3] = px; dst[pt * 3 + 1] = py; dst[pt * 3 + 2] = pz;
+        store_obs<F16>(dst, pt * 3, px); store_obs<F16>(dst, pt * 3 + 1, py); store_obs<F16>(dst, pt * 3 + 2, pz);
     }
 }
 
@@ -666,32 +673,37 @@ __global__ void r_theta_kernel(const float *v1, const float *v2, long long m, fl
 // ----------------------------------------------------------------------------
 typedef void (*StepFn)(const StepParams);
 
+template <int ARM, int X, bool RAND>
+static StepFn pick_obs(bool wobs, bool f16) {
+    if (!wobs) return step_kernel<ARM, X, RAND, false, false>;
+    return f16 ? step_kernel<ARM, X, RAND, true, true> : step_kernel<ARM, X, RAND, true, false>;
+}
+
 template <int ARM, int X>
-static StepFn pick_flags(bool rnd, bool wobs) {
-    if (rnd) return wobs ? step_kernel<ARM, X, true, true> : step_kernel<ARM, X, true, false>;
-    return wobs ? step_kernel<ARM, X, false, true> : step_kernel<ARM, X, false, false>;
+static StepFn pick_flags(bool rnd, bool wobs, bool f16) {
+    return rnd ? pick_obs<ARM, X, true>(wobs, f16) : pick_obs<ARM, X, false>(wobs, f16);
 }
 
 template <int ARM>
-static StepFn pick_x(int x, bool rnd, bool wobs) {
+static StepFn pick_x(int x, bool rnd, bool wobs, bool f16) {
     switch (x) {
-        case 10: return pick_flags<ARM, 10>(rnd, wobs);
-        case 20: return pick_flags<ARM, 20>(rnd, wobs);
-        default: return pick_flags<ARM, 0>(rnd, wobs);
+        case 10: return pick_flags<ARM, 10>(rnd, wobs, f16);
+        case 20: return pick_flags<ARM, 20>(rnd, wobs, f16);
+        default: return pick_flags<ARM, 0>(rnd, wobs, f16);
     }
 }
 
-static StepFn pick_kernel(int arm, int x, bool rnd, bool wobs) {
+static StepFn pick_kernel(int arm, int x, bool rnd, bool wobs, bool f16) {
     switch (arm) {
-        case 0: return pick_x<0>(x, rnd, wobs);
-        case 2: return pick_flags<2, 0>(rnd, wobs);
-        case 3: return pick_flags<3, 0>(rnd, wobs);
-        case 4: return pick_flags<4, 0>(rnd, wobs);
-        case 5: return pick_flags<5, 0>(rnd, wobs);
-        case 6: return pick_x<6>(x, rnd, wobs);
-        case 7: return pick_flags<7, 0>(rnd, wobs);
-        case 8: return pick_flags<8, 0>(rnd, wobs);
-#define MT_PICK(ID) case ID: return pick_x<ID>(x, rnd, wobs);
+        case 0: return pick_x<0>(x, rnd, wobs, f16);
+        case 2: return pick_flags<2, 0>(rnd, wobs, f16);
+        case 3: return pick_flags<3, 0>(rnd, wobs, f16);
+        case 4: return pick_flags<4, 0>(rnd, wobs, f16);
+        case 5: return pick_flags<5, 0>(rnd, wobs, f16);
+        case 6: return pick_x<6>(x, rnd, wobs, f16);
+        case 7: return pick_flags<7, 0>(rnd, wobs, f16);
+        case 8: return pick_flags<8, 0>(rnd, wobs, f16);
+#define MT_PICK(ID) case ID: return pick_x<ID>(x, rnd, wobs, f16);
         MT_FOR_EACH_PRESET_ARM(MT_PICK)
 #undef MT_PICK
     }
@@ -785,7 +797,7 @@ static int launch_pdl(const void *fn, const LaunchShape &shape, const StepParams
 }
 
 // launch the fused step kernel over tiles [t0, t1): a persistent grid sized to the SMs
-static int launch_step(mt_env *e, const float *actions, float *obs, float *reward, uint8_t *done, float *joints,
+static int launch_step(mt_env *e, const float *actions, void *obs, float *reward, uint8_t *done, float *joints,
                        bool rnd, long long t0, long long t1, cudaStream_t st, int ticket_slot = 0, bool advance = true) {
     StepParams P = e->base;
     P.actions = actions;
@@ -808,12 +820,12 @@ static int launch_step(mt_env *e, const float *actions, float *obs, float *rewar
         cudaKernel_t &k = e->jit_kernel[rnd ? 1 : 0][wobs ? 1 : 0];
         if (!k) {                                             // other variants compile on first use
             std::string err;
-            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, rnd, wobs, err).kernel;
+            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, rnd, wobs, e->f16, err).kernel;
             if (!k) return fail(MT_ERR_CUDA, "run-time specialisation failed: %s", err.c_str());
         }
         fn = (const void *)k;
     } else {
-        fn = (const void *)pick_kernel(e->arm, e->cfg.n_obj, rnd, wobs);
+        fn = (const void *)pick_kernel(e->arm, e->cfg.n_obj, rnd, wobs, e->f16);
     }
     if (!fn) return fail(MT_ERR_INVALID, "no kernel for arm=%d", e->arm);
     const size_t nb = e->arm == 0 ? StepBuffers<0>::value : StepBuffers<1>::value;   // tile buffers per warp
@@ -827,26 +839,32 @@ static int launch_step(mt_env *e, const float *actions, float *obs, float *rewar
 
 // Multi-step random rollout in ONE launch (rollout_kernel, mt_step.cuh): built-in arms and handles whose kernels
 // come from NVRTC; run-time DH tables take the per-step launches instead (`launched` stays false).
+template <int ARM, int X>
+static StepFn pick_rollout_obs(bool wobs, bool f16) {
+    if (!wobs) return rollout_kernel<ARM, X, false, false>;
+    return f16 ? rollout_kernel<ARM, X, true, true> : rollout_kernel<ARM, X, true, false>;
+}
+
 template <int ARM>
-static StepFn pick_rollout_x(int x, bool wobs) {
+static StepFn pick_rollout_x(int x, bool wobs, bool f16) {
     switch (x) {
-        case 10: return wobs ? rollout_kernel<ARM, 10, true> : rollout_kernel<ARM, 10, false>;
-        case 20: return wobs ? rollout_kernel<ARM, 20, true> : rollout_kernel<ARM, 20, false>;
-        default: return wobs ? rollout_kernel<ARM, 0, true> : rollout_kernel<ARM, 0, false>;
+        case 10: return pick_rollout_obs<ARM, 10>(wobs, f16);
+        case 20: return pick_rollout_obs<ARM, 20>(wobs, f16);
+        default: return pick_rollout_obs<ARM, 0>(wobs, f16);
     }
 }
 
-static StepFn pick_rollout(int arm, int x, bool wobs) {
+static StepFn pick_rollout(int arm, int x, bool wobs, bool f16) {
     switch (arm) {
-        case 0: return pick_rollout_x<0>(x, wobs);
-#define MT_PICK(ID) case ID: return pick_rollout_x<ID>(x, wobs);
+        case 0: return pick_rollout_x<0>(x, wobs, f16);
+#define MT_PICK(ID) case ID: return pick_rollout_x<ID>(x, wobs, f16);
         MT_FOR_EACH_PRESET_ARM(MT_PICK)
 #undef MT_PICK
     }
     return nullptr;
 }
 
-static int launch_rollout(mt_env *e, int n_steps, float *obs, float *reward, uint8_t *done, cudaStream_t st, bool &launched) {
+static int launch_rollout(mt_env *e, int n_steps, void *obs, float *reward, uint8_t *done, cudaStream_t st, bool &launched) {
     launched = false;
     if (n_steps < 2) return MT_OK;
     if (const char *v = std::getenv("MT_ROLLOUT_PERSISTENT"))
@@ -857,7 +875,7 @@ static int launch_rollout(mt_env *e, int n_steps, float *obs, float *reward, uin
         cudaKernel_t &k = e->jit_rollout[obs ? 1 : 0];
         if (!k) {
             std::string err;
-            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, true, obs != nullptr, err, true).kernel;
+            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, true, obs != nullptr, e->f16, err, true).kernel;
             if (!k) {
                 e->jit_rollout_failed = true;                 // keep working through the per-step launches
                 return MT_OK;
@@ -865,7 +883,7 @@ static int launch_rollout(mt_env *e, int n_steps, float *obs, float *reward, uin
         }
         fn = (const void *)k;
     } else {
-        fn = (const void *)pick_rollout(e->arm, e->cfg.n_obj, obs != nullptr);
+        fn = (const void *)pick_rollout(e->arm, e->cfg.n_obj, obs != nullptr, e->f16);
     }
     if (!fn) return MT_OK;
     StepParams P = e->base;
@@ -922,12 +940,13 @@ extern "C" int mt_reset(mt_env *e, const uint8_t *mask_dev, void *stream) {
     return MT_OK;
 }
 
-extern "C" int mt_observe(mt_env *e, float *obs_dev, void *stream) {
+extern "C" int mt_observe(mt_env *e, void *obs_dev, void *stream) {
     if (!e) return fail(MT_ERR_INVALID, "env is NULL");
     if (int rc = check_ptr(obs_dev, "obs_dev", true)) return rc;
     if (!e->was_reset) return fail(MT_ERR_STATE, "mt_observe before mt_reset (the reference raises IndexError here, manytor.py:143)");
     DeviceGuard guard(e->cfg.device);
-    observe_kernel<<<blocks_for(e->n, 128), 128, 0, (cudaStream_t)stream>>>(e->base, e->arm, obs_dev);
+    (e->f16 ? observe_kernel<true> : observe_kernel<false>)<<<blocks_for(e->n, 128), 128, 0, (cudaStream_t)stream>>>(
+        e->base, e->arm, obs_dev);
     CU(cudaGetLastError());
     e->launches++;
     return MT_OK;
@@ -946,7 +965,7 @@ static int timing_end(mt_env *e, cudaStream_t st) {
     return MT_OK;
 }
 
-extern "C" int mt_step(mt_env *e, const float *actions_dev, float *obs_dev, float *reward_dev, uint8_t *done_dev,
+extern "C" int mt_step(mt_env *e, const float *actions_dev, void *obs_dev, float *reward_dev, uint8_t *done_dev,
                        float *joints_dev, void *stream) {
     if (!e) return fail(MT_ERR_INVALID, "env is NULL");
     if (!e->was_reset) return fail(MT_ERR_STATE, "mt_step before mt_reset (the reference raises IndexError here, manytor.py:143)");
@@ -971,7 +990,7 @@ extern "C" int mt_sample_actions(mt_env *e, float *actions_dev, void *stream) {
     return MT_OK;
 }
 
-extern "C" int mt_rollout_random(mt_env *e, int32_t n_steps, float *obs_dev, float *reward_dev, uint8_t *done_dev,
+extern "C" int mt_rollout_random(mt_env *e, int32_t n_steps, void *obs_dev, float *reward_dev, uint8_t *done_dev,
                                  void *stream) {
     if (!e) return fail(MT_ERR_INVALID, "env is NULL");
     if (!e->was_reset) return fail(MT_ERR_STATE, "mt_rollout_random before mt_reset");
@@ -1036,13 +1055,13 @@ static bool device_visible_host(const void *p) {
     return a.type == cudaMemoryTypeHost && a.devicePointer == p && ((uintptr_t)p & 15u) == 0;
 }
 
-extern "C" int mt_step_host(mt_env *e, const float *actions_host, float *obs_host, float *reward_host,
+extern "C" int mt_step_host(mt_env *e, const float *actions_host, void *obs_host, float *reward_host,
                             uint8_t *done_host) {
     if (!e) return fail(MT_ERR_INVALID, "env is NULL");
     if (!e->was_reset) return fail(MT_ERR_STATE, "mt_step_host before mt_reset");
     if (!actions_host || !reward_host || !done_host) return fail(MT_ERR_INVALID, "NULL host buffer");
     DeviceGuard guard(e->cfg.device);
-    const size_t J = e->cfg.n_joints, R = 3 * (size_t)e->cfg.n_obj;
+    const size_t J = e->cfg.n_joints, R = 3 * (size_t)e->cfg.n_obj * (e->f16 ? 2 : 4);   // R: bytes per observation row
     if (!e->hs[0]) {
         for (auto &s : e->hs) CU(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
         for (auto &v : e->hev) CU(cudaEventCreateWithFlags(&v, cudaEventDisableTiming));
@@ -1078,7 +1097,7 @@ extern "C" int mt_step_host(mt_env *e, const float *actions_host, float *obs_hos
     CU(cudaEventRecord(e->hev[mt_env::kStreams], nullptr));       // everything submitted so far (blocking streams)
     if (!e->h_actions) {
         CU(cudaMalloc((void **)&e->h_actions, (size_t)e->n_pad * J * 4));
-        CU(cudaMalloc((void **)&e->h_obs, (size_t)e->n_pad * R * 4));
+        CU(cudaMalloc(&e->h_obs, (size_t)e->n_pad * R));
         CU(cudaMalloc((void **)&e->h_reward, (size_t)e->n_pad * 4));
         CU(cudaMalloc((void **)&e->h_done, (size_t)e->n_pad));
     }
@@ -1095,7 +1114,8 @@ extern "C" int mt_step_host(mt_env *e, const float *actions_host, float *obs_hos
         if (int rc = launch_step(e, e->h_actions, obs_host ? e->h_obs : nullptr, e->h_reward, e->h_done, nullptr, false,
                                  t0, t1, st, 1 + k, t1 == e->n_tiles))
             return rc;
-        if (obs_host) CU(cudaMemcpyAsync(obs_host + e0 * R, e->h_obs + e0 * R, cnt * R * 4, cudaMemcpyDeviceToHost, st));
+        if (obs_host)
+            CU(cudaMemcpyAsync((char *)obs_host + e0 * R, (char *)e->h_obs + e0 * R, cnt * R, cudaMemcpyDeviceToHost, st));
     }
     // reward / done of the whole shard: two copies once every chunk's kernel has run
     for (int i = 1; i < mt_env::kStreams; ++i) {
@@ -1463,14 +1483,15 @@ extern "C" int mt_r_theta(const float *v1_dev, const float *v2_dev, float *out_d
 
 extern "C" int64_t mt_launch_count(const mt_env *e) { return e ? e->launches : 0; }
 
-// SURVEY.md section 8(d): B = 12J + 24X + 21 with actions read from HBM and obs
-// written; minus 4J when actions are drawn in-kernel, minus 12X without obs.
+// SURVEY.md section 8(d): B = 12J + 24X + 21 with actions read from HBM and fp32 obs
+// written (12J + 18X + 21 with binary16 obs); minus 4J when actions are drawn in-kernel,
+// minus the observations (12X or 6X) without them.
 extern "C" int64_t mt_bytes_per_env_step(const mt_env *e, int32_t actions_from_hbm, int32_t obs_written) {
     if (!e) return 0;
     const int64_t J = e->cfg.n_joints, X = e->cfg.n_obj;
     int64_t b = 8 * J + 12 * X + 21;  // goals r+w, points r, alive r+w, reward w, done w, total_reward r+w
     if (actions_from_hbm) b += 4 * J;
-    if (obs_written) b += 12 * X;
+    if (obs_written) b += (e->f16 ? 6 : 12) * X;
     return b;
 }
 

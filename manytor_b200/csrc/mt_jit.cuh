@@ -2,7 +2,7 @@
 //
 // A preset arm (mt_step.cuh) gets its DH table folded at compile time; this file gives ANY table the
 // same treatment without rebuilding the library: at mt_create the table is printed into a
-// `Preset<ID>` specialisation, NVRTC compiles `step_kernel<ID, X, RAND, WOBS>` for sm_100a from the
+// `Preset<ID>` specialisation, NVRTC compiles `step_kernel<ID, X, RAND, WOBS, F16>` for sm_100a from the
 // very same headers the library was built from (embedded as strings by manytor_b200/build.py), and
 // the cubin is loaded through the runtime's library API.  ~0.8 s per variant, cached per process.
 // NVRTC is dlopen'ed: when it is absent the handle simply keeps the run-time-table kernels.
@@ -91,16 +91,19 @@ static std::string preset_source(int id, int J, const JointConst *rows) {
     return s;
 }
 
-// Compile (or fetch from the per-process cache) step_kernel<id, x_template, rnd, wobs> for the table
+// Compile (or fetch from the per-process cache) step_kernel<id, x_template, rnd, wobs, f16> for the table
 // described by `preset`.  Returns an empty JitKernel and fills `err` on failure.
-// `rollout` selects the multi-step rollout_kernel<id, x_template, wobs> (in-kernel actions; `rnd` is ignored).
-static JitKernel jit_step_kernel(const std::string &preset, int id, int x_template, bool rnd, bool wobs, std::string &err,
-                                 bool rollout = false) {
+// `rollout` selects the multi-step rollout_kernel<id, x_template, wobs, f16> (in-kernel actions; `rnd` is ignored).
+// The cache key holds the template arguments, so handles with the same table and different observation
+// formats get different kernels.
+static JitKernel jit_step_kernel(const std::string &preset, int id, int x_template, bool rnd, bool wobs, bool f16,
+                                 std::string &err, bool rollout = false) {
     static std::mutex mu;
     static std::map<std::string, JitKernel> cache;
-    const std::string targs = rollout ? std::to_string(id) + ", " + std::to_string(x_template) + ", " + (wobs ? "true" : "false")
+    const char *obs = wobs ? (f16 ? "true, true" : "true, false") : "false, false";
+    const std::string targs = rollout ? std::to_string(id) + ", " + std::to_string(x_template) + ", " + obs
                                       : std::to_string(id) + ", " + std::to_string(x_template) + ", " + (rnd ? "true" : "false") +
-                                            ", " + (wobs ? "true" : "false");
+                                            ", " + obs;
     const std::string kname = rollout ? "rollout_kernel" : "step_kernel";
     const std::string inst = "mt::" + kname + "<" + targs + ">";
     const std::string key = preset + inst;

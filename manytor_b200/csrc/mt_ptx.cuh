@@ -60,6 +60,27 @@ __device__ __forceinline__ void sts_f2(uint32_t a, float2 v) {
 __device__ __forceinline__ void sts_f(uint32_t a, float v) {
     asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory");
 }
+__device__ __forceinline__ float4 lds_f4(uint32_t a) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a) : "memory");
+    return v;
+}
+__device__ __forceinline__ void sts_u2(uint32_t a, uint32_t x, uint32_t y) {
+    asm volatile("st.shared.v2.b32 [%0], {%1,%2};" ::"r"(a), "r"(x), "r"(y) : "memory");
+}
+
+// IEEE binary16, round to nearest even (written as PTX: NVRTC compiles these headers without cuda_fp16.h)
+__device__ __forceinline__ uint16_t f32_to_f16(float v) {
+    uint16_t h;
+    asm("cvt.rn.f16.f32 %0, %1;" : "=h"(h) : "f"(v));
+    return h;
+}
+// two halves in one word, `lo` at the lower address
+__device__ __forceinline__ uint32_t f32x2_to_f16x2(float lo, float hi) {
+    uint32_t h;
+    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(h) : "f"(hi), "f"(lo));
+    return h;
+}
 // one thread's atomic on a shared counter (written as PTX so that ptxas does not wrap it into its
 // warp-aggregation sequence: the caller already elected one lane)
 __device__ __forceinline__ int atom_add_s(uint32_t a, int v) {

@@ -69,7 +69,7 @@ struct StepParams {
     float *points;           // [Npad][X][3]
     // per-step I/O
     const float *actions;    // [N][J] or nullptr when drawn in-kernel
-    float *obs;              // [N][3X]
+    void *obs;               // [N][3X] fp32, or binary16 in the kernels built for F16 (mt_config.obs_dtype)
     float *reward;           // [N]
     uint8_t *done;           // [N]
     float *joints;           // [N][J][3] or nullptr
@@ -618,6 +618,40 @@ __device__ __forceinline__ uint32_t walk_row(uint32_t row, uint32_t orow, int x,
 }
 
 // ---------------------------------------------------------------------------
+// binary16 observations (mt_config.obs_dtype = MT_OBS_F16).  Every kernel computes a tile's observations in fp32
+// in shared memory, exactly as for an fp32 handle; only the way out differs.
+// ---------------------------------------------------------------------------
+// Pack a full tile of observations, [32][rowlen] fp32 at `buf`, to binary16 in place: element i moves from byte 4i
+// to byte 2i, so the packed tile ([32][rowlen] halves, 64 rowlen = 192 X bytes) is contiguous at the start of the
+// buffer and leaves by one bulk store.  Lane l converts the 4-element quads l, l + 32, ...: round r reads bytes
+// [512r, 512r + 512) and writes [256r, 256r + 256), which round r / 2 <= r has read.  The writes of a round land on
+// words other lanes of the SAME round read (r = 0), so each round reads into registers, syncs the warp, then writes;
+// later rounds read only above what earlier rounds wrote.  The caller has synced the warp after writing the tile.
+template <int X>
+__device__ __forceinline__ void pack_tile_f16(uint32_t buf, int rowlen, int lane) {
+    const int quads = (X ? 3 * X : rowlen) * (kTile / 4);
+#pragma unroll
+    for (int q0 = 0; q0 < quads; q0 += kTile) {
+        const int q = q0 + lane;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (q < quads) v = lds_f4(buf + 16u * (uint32_t)q);
+        __syncwarp();
+        if (q < quads) sts_u2(buf + 8u * (uint32_t)q, f32x2_to_f16x2(v.x, v.y), f32x2_to_f16x2(v.z, v.w));
+    }
+}
+
+// element i of the caller's observation buffer, in the kernel's format
+template <bool F16>
+__device__ __forceinline__ void *obs_at(void *obs, size_t i) {
+    return F16 ? (void *)((uint16_t *)obs + i) : (void *)((float *)obs + i);
+}
+template <bool F16>
+__device__ __forceinline__ void store_obs(void *obs, size_t i, float v) {
+    if (F16) ((uint16_t *)obs)[i] = f32_to_f16(v);
+    else ((float *)obs)[i] = v;
+}
+
+// ---------------------------------------------------------------------------
 // objective refresh (manytor.py:228-241): uniform in the upper half ball.
 // The reference rejects from the cube; the direct map below has the same
 // distribution: r = R u^(1/3), z/r uniform on [0,1], azimuth uniform.
@@ -874,6 +908,7 @@ __device__ __forceinline__ void block_epilogue(const StepParams &P, int lane, in
 //   ARM  0 = reference arm closed form (J = 4); else J of the generic chain
 //   X    objectives per env, 0 = run-time P.n_obj
 //   RAND draw actions in-kernel (mt_rollout_random)   WOBS write observations
+//   F16  observations leave as binary16 (pack_tile_f16); only instantiated with WOBS
 //
 // Persistent blocks: one per SM (as many warps as the SM holds; several smaller
 // blocks for launches with few tiles), each owning every G-th tile and handing
@@ -895,9 +930,10 @@ __device__ __forceinline__ unsigned long long trace_now() {
 }
 #endif
 
-template <int ARM, int X, bool RAND, bool WOBS>
+template <int ARM, int X, bool RAND, bool WOBS, bool F16>
 __global__ void __launch_bounds__(((ARM == 0) ? kMaxWarpsRefArm : kMaxWarpsGeneric) * kTile, 1)
 step_kernel(const __grid_constant__ StepParams P) {
+    static_assert(WOBS || !F16, "F16 is an observation format");
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ int queue_next;
     __shared__ unsigned int warps_done, warps_seen;
@@ -1072,15 +1108,16 @@ step_kernel(const __grid_constant__ StepParams P) {
             }
             if (WOBS) {
                 if (full) {
+                    if (F16) pack_tile_f16<X>(buf_cur, rowlen, lane);
                     fence_async_smem();
                     __syncwarp();
                     if (lane == 0) {
-                        bulk_store_hint_s(P.obs + (size_t)env0 * rowlen, buf_cur, tile_bytes, pol_store);
+                        bulk_store_hint_s(obs_at<F16>(P.obs, (size_t)env0 * rowlen), buf_cur, F16 ? tile_bytes / 2 : tile_bytes, pol_store);
                         bulk_commit();
                     }
                 } else if (valid) {
-                    float *dst = P.obs + env * rowlen;
-                    for (int i = 0; i < rowlen; ++i) dst[i] = lds_f(row + 4u * i);
+                    void *dst = obs_at<F16>(P.obs, env * rowlen);
+                    for (int i = 0; i < rowlen; ++i) store_obs<F16>(dst, i, lds_f(row + 4u * i));
                 }
             }
 
@@ -1129,9 +1166,10 @@ step_kernel(const __grid_constant__ StepParams P) {
 // staggered start and drain; results are bit-identical (same arithmetic, same action stream: step index of
 // the launch + s).  Algorithmic bytes per env-step: 12 X + 5 written, plus (48 + 12 X) / n_steps.
 // ---------------------------------------------------------------------------
-template <int ARM, int X, bool WOBS>
+template <int ARM, int X, bool WOBS, bool F16>
 __global__ void __launch_bounds__(((ARM == 0) ? kMaxWarpsRefArm : kMaxWarpsGeneric) * kTile, 1)
 rollout_kernel(const __grid_constant__ StepParams P) {
+    static_assert(WOBS || !F16, "F16 is an observation format");
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ int queue_next;
     __shared__ unsigned int warps_done, warps_seen;
@@ -1216,15 +1254,16 @@ rollout_kernel(const __grid_constant__ StepParams P) {
                 }
                 if (WOBS) {
                     if (full) {
+                        if (F16) pack_tile_f16<X>(obuf, rowlen, lane);
                         fence_async_smem();
                         __syncwarp();
                         if (lane == 0) {
-                            bulk_store_hint_s(P.obs + (size_t)env0 * rowlen, obuf, tile_bytes, pol_store);
+                            bulk_store_hint_s(obs_at<F16>(P.obs, (size_t)env0 * rowlen), obuf, F16 ? tile_bytes / 2 : tile_bytes, pol_store);
                             bulk_commit();
                         }
                     } else if (valid) {
-                        float *dst = P.obs + env * rowlen;
-                        for (int i = 0; i < rowlen; ++i) dst[i] = lds_f(orow + 4u * i);
+                        void *dst = obs_at<F16>(P.obs, env * rowlen);
+                        for (int i = 0; i < rowlen; ++i) store_obs<F16>(dst, i, lds_f(orow + 4u * i));
                     }
                 }
             }
