@@ -132,7 +132,12 @@ int mt_set_seed(mt_env *env, uint64_t seed);
  * mt_step_host and of each step of mt_rollout_random), as are mt_stats.env_steps and the other
  * statistics.  Consequence for CUDA graphs: a captured mt_step / mt_rollout_random can be replayed
  * any number of times -- every replay counts its env-steps and draws fresh actions, exactly like the
- * same calls issued eagerly.  Get/set are synchronous 8-byte copies (checkpoint / resume). */
+ * same calls issued eagerly.  Get/set are synchronous 8-byte copies (checkpoint / resume).
+ * The index lies in [0, MT_STEP_INDEX_MAX]; mt_set_step_index returns MT_ERR_INVALID above it and leaves
+ * the index as it was.  The bound exists because the kernels' launch bookkeeping needs bit 63 of the index
+ * to be clear: each warp orders its launch ticket after its read of the index through that bit.  At most
+ * 4096 steps pass per launch, so climbing from 2^62 to 2^63 would take more than 10^15 launches. */
+#define MT_STEP_INDEX_MAX 0x4000000000000000ull /* 2^62 */
 int mt_get_step_index(mt_env *env, uint64_t *out);
 int mt_set_step_index(mt_env *env, uint64_t value);
 

@@ -16,6 +16,7 @@ MT_STATS_WORDS = 8
 MT_ABI_VERSION = 3
 MT_OBS_F32 = 0
 MT_OBS_F16 = 1
+MT_STEP_INDEX_MAX = 1 << 62
 
 STATS_FIELDS = ("env_steps", "episodes", "terminated", "reward_sum", "length_sum", "catches",
                 "ground_steps", "live_reward_sum")

@@ -402,7 +402,11 @@ class BatchedEnvs:
 
     @step_index.setter
     def step_index(self, value: int):
-        _lib.check(self._lib.mt_set_step_index(self._h, int(value) & 0xFFFFFFFFFFFFFFFF))
+        """Resume from a checkpoint.  Accepts [0, 2^62] (MT_STEP_INDEX_MAX); anything else raises ValueError."""
+        value = int(value)
+        if not 0 <= value <= _lib.MT_STEP_INDEX_MAX:
+            raise ValueError(f"step_index must be in [0, 2**62], not {value}")
+        _lib.check(self._lib.mt_set_step_index(self._h, value))
 
     # -- statistics ---------------------------------------------------------------
     def stats_tensor(self) -> torch.Tensor:

@@ -453,6 +453,9 @@ extern "C" int mt_get_step_index(mt_env *e, uint64_t *out) {
 }
 extern "C" int mt_set_step_index(mt_env *e, uint64_t value) {
     if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    // the kernels' launch ticket depends on bit 63 of the index being clear (launch_ticket, mt_step.cuh)
+    if (value > MT_STEP_INDEX_MAX)
+        return fail(MT_ERR_INVALID, "step index %llu is above MT_STEP_INDEX_MAX (2^62)", (unsigned long long)value);
     DeviceGuard guard(e->cfg.device);
     const unsigned long long v = value;
     CU(cudaMemcpy(e->ctrl + kCtrlStep, &v, 8, cudaMemcpyHostToDevice));
