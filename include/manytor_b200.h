@@ -91,8 +91,9 @@ typedef struct mt_config {
     int32_t action_high;
     uint64_t seed;                 /* Philox key for on-device actions / objectives       */
     int32_t obs_dtype;             /* MT_OBS_F32 (default) or MT_OBS_F16: the format of the
-                                      obs buffers of mt_step, mt_observe, mt_rollout_random
-                                      and mt_step_host (the values are the fp32 ones rounded) */
+                                      obs buffers of mt_step, mt_observe, mt_rollout_random,
+                                      mt_rollout and mt_step_host (the values are the fp32
+                                      ones rounded) */
 } mt_config;
 
 /* Episode statistics; summed over the shard, reducible across shards by plain
@@ -176,6 +177,26 @@ int mt_sample_actions(mt_env *env, float *actions_dev, void *stream);
  * take (MT_ROLLOUT_PERSISTENT=0 forces them for everyone). */
 int mt_rollout_random(mt_env *env, int32_t n_steps, void *obs_dev, float *reward_dev,
                       uint8_t *done_dev, void *stream);
+
+/* n_steps x step() in one call, keeping EVERY step (a trajectory).  Slice s of each array holds exactly
+ * what the s-th of n_steps consecutive mt_step calls would have written, bit for bit.
+ *   actions_dev [n_steps][N][J]  the caller's actions; step s reads actions_dev + s*N*J.
+ *                                NULL = drawn in-kernel: the stream of mt_rollout_random / mt_sample_actions
+ *                                (Philox keyed by seed, env id, step index + s)
+ *   drawn_dev   [n_steps][N][J]  receives the drawn actions when actions_dev is NULL; may be NULL;
+ *                                must be NULL when actions_dev is given
+ *   obs_dev     [n_steps][N][3X] in the handle's obs format, or NULL (no observations written)
+ *   reward_dev  [n_steps][N] fp32, done_dev [n_steps][N] u8: required
+ * Slices are packed (a stride of exactly N rows); every base pointer is 16-byte aligned.  n_steps < 0 is
+ * MT_ERR_INVALID, n_steps = 0 does nothing, a call before the first mt_reset is MT_ERR_STATE.
+ * The step index, env-step count and statistics advance exactly as for n_steps mt_step calls.
+ * Like mt_rollout_random this is one launch of the multi-step rollout kernel per 4096 steps (state in
+ * registers, objectives in shared memory), and n_steps launches of the step kernel for run-time DH
+ * tables without NVRTC or under MT_ROLLOUT_PERSISTENT=0.  The caller's actions are read once each, so
+ * an open-loop planner or a replay of logged actions moves 4J bytes of actions per env-step instead of
+ * the full state round trip of one mt_step per step. */
+int mt_rollout(mt_env *env, int32_t n_steps, const float *actions_dev, float *drawn_dev, void *obs_dev,
+               float *reward_dev, uint8_t *done_dev, void *stream);
 
 /* Host-buffer step: actions_host/obs_host/reward_host/done_host must be pinned
  * (mt_host_alloc).  Copies actions H2D, steps, copies results D2H, chunked over

@@ -11,6 +11,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import weakref
+from collections import namedtuple
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -49,6 +50,11 @@ UR5_ARM = ArmSpec(
         (0.0, math.pi / 2, 0.10915, 0.0), (0.0, -math.pi / 2, 0.09465, 0.0), (0.0, 0.0, 0.0823, 0.0)),
     obs_frame=5, ground_frames=(5, 6), catch_frame=6,
     radius=0.81725, catch_tol=0.81725 * 8.0 / 51.3)
+
+
+# What BatchedEnvs.rollout returns: obs (K, N, 3X) of the handle's obs_dtype or None, reward (K, N) float32,
+# done (K, N) uint8, actions (K, N, J) float32 (the caller's, or the recorded draws) or None.
+Trajectory = namedtuple("Trajectory", "obs reward done actions")
 
 
 # observation dtype -> mt_config.obs_dtype
@@ -271,6 +277,70 @@ class BatchedEnvs:
         _lib.check(self._lib.mt_rollout_random(self._h, int(n_steps), self._p(self._obs if write_obs else None),
                                                self._p(self._reward), self._p(self._done), self._stream()))
         return (self._obs if write_obs else None, self._reward, self._done)
+
+    def rollout(self, actions=None, n_steps: Optional[int] = None, write_obs: bool = True,
+                record_actions: bool = False, out: Optional[Trajectory] = None) -> Trajectory:
+        """K steps in one call, keeping every step: slice s of the returned Trajectory is what the s-th of K
+        consecutive `step` calls would have returned, bit for bit (mt_rollout).
+
+        actions: (K, N, J) degrees, converted like `step`'s input; K comes from it.  None = actions drawn
+        in-kernel (the stream of `rollout_random` / `sample_actions`); `n_steps` then gives K, and
+        `record_actions=True` returns the drawn actions as well.  `out`: a Trajectory of preallocated buffers
+        (obs of this handle's obs_dtype, or None when write_obs is False; actions only with record_actions),
+        e.g. fixed storage for a CUDA graph that captures this call.  Shape and dtype errors raise ValueError
+        before the library is called."""
+        if actions is not None:
+            if record_actions:
+                raise ValueError("record_actions records in-kernel draws: it cannot be combined with actions")
+            shape = tuple(actions.shape) if hasattr(actions, "shape") else tuple(np.shape(actions))
+            if len(shape) != 3 or shape[1:] != (self.n, self.j):
+                raise ValueError(f"actions must have shape (K, {self.n}, {self.j}), not {shape}")
+            if n_steps is not None and int(n_steps) != shape[0]:
+                raise ValueError(f"n_steps={n_steps} disagrees with the {shape[0]} steps of actions")
+            k = shape[0]
+        else:
+            if n_steps is None:
+                raise ValueError("rollout needs actions or n_steps")
+            k = int(n_steps)
+        if k < 0:
+            raise ValueError(f"n_steps must be >= 0, not {k}")
+        want = {"obs": ((k, self.n, 3 * self.x), self.obs_dtype) if write_obs else None,
+                "reward": ((k, self.n), torch.float32), "done": ((k, self.n), torch.uint8),
+                "actions": ((k, self.n, self.j), torch.float32) if record_actions else None}
+        if out is not None:
+            if not isinstance(out, Trajectory):
+                raise ValueError("out must be a Trajectory")
+            for name, spec in want.items():
+                t = getattr(out, name)
+                if spec is None:
+                    if t is not None:
+                        raise ValueError(f"out.{name} must be None here (write_obs={write_obs}, "
+                                         f"record_actions={record_actions})")
+                    continue
+                if not isinstance(t, torch.Tensor):
+                    raise ValueError(f"out.{name} must be a tensor of shape {spec[0]} and dtype {spec[1]}")
+                if tuple(t.shape) != spec[0] or t.dtype != spec[1]:
+                    raise ValueError(f"out.{name} must have shape {spec[0]} and dtype {spec[1]}, "
+                                     f"not {tuple(t.shape)} {t.dtype}")
+                if not t.is_contiguous() or t.device != self.device:
+                    raise ValueError(f"out.{name} must be a contiguous tensor on {self.device}")
+            bufs = out
+        else:
+            bufs = Trajectory(*(self._empty(*spec) if spec is not None else None for spec in want.values()))
+        if actions is not None:
+            if (isinstance(actions, torch.Tensor) and actions.is_cuda and actions.device == self.device
+                    and actions.dtype == torch.float32 and actions.is_contiguous()):
+                a = actions                                # fast path: already the device layout
+            else:
+                a = self._as_dev(actions, torch.float32, (k, self.n, self.j))
+            bufs = bufs._replace(actions=a)
+        if k == 0:                                         # nothing to do (and empty tensors have no address)
+            return bufs
+        _lib.check(self._lib.mt_rollout(self._h, k, self._p(a if actions is not None else None),
+                                        self._p(bufs.actions if actions is None else None), self._p(bufs.obs),
+                                        self._p(bufs.reward), self._p(bufs.done), self._stream()))
+        self._rollout_io = bufs                            # keep alive until the stream has consumed them
+        return bufs
 
     # -- host-buffer (end-to-end) step ------------------------------------------
     def pinned(self, name: str, shape, dtype) -> np.ndarray:

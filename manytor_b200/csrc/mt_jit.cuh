@@ -93,15 +93,18 @@ static std::string preset_source(int id, int J, const JointConst *rows) {
 
 // Compile (or fetch from the per-process cache) step_kernel<id, x_template, rnd, wobs, f16> for the table
 // described by `preset`.  Returns an empty JitKernel and fills `err` on failure.
-// `rollout` selects the multi-step rollout_kernel<id, x_template, wobs, f16> (in-kernel actions; `rnd` is ignored).
-// The cache key holds the template arguments, so handles with the same table and different observation
-// formats get different kernels.
+// `rollout_mode` >= 0 selects the multi-step rollout_kernel<id, x_template, wobs, f16, RolloutMode(rollout_mode)>
+// (`rnd` is ignored).  The cache key holds the template arguments, so handles with the same table and different
+// observation formats or rollout modes get different kernels.
 static JitKernel jit_step_kernel(const std::string &preset, int id, int x_template, bool rnd, bool wobs, bool f16,
-                                 std::string &err, bool rollout = false) {
+                                 std::string &err, int rollout_mode = -1) {
     static std::mutex mu;
     static std::map<std::string, JitKernel> cache;
+    static const char *const kModes[] = {"mt::RolloutMode::kDrawLast", "mt::RolloutMode::kDrawTrajectory",
+                                         "mt::RolloutMode::kActionsTrajectory"};
+    const bool rollout = rollout_mode >= 0;
     const char *obs = wobs ? (f16 ? "true, true" : "true, false") : "false, false";
-    const std::string targs = rollout ? std::to_string(id) + ", " + std::to_string(x_template) + ", " + obs
+    const std::string targs = rollout ? std::to_string(id) + ", " + std::to_string(x_template) + ", " + obs + ", " + kModes[rollout_mode]
                                       : std::to_string(id) + ", " + std::to_string(x_template) + ", " + (rnd ? "true" : "false") +
                                             ", " + obs;
     const std::string kname = rollout ? "rollout_kernel" : "step_kernel";

@@ -108,7 +108,27 @@ struct StepParams {
     // through once per step (actions, objectives in; observations, reward, done out): evict_normal while the
     // whole state fits its budget, evict_first beyond (mt_create; measured both ways in round 2).
     unsigned long long pol_state, pol_stream, pol_store;   // pol_store: the streamed OUTPUTS (observations, reward, done)
+    float *drawn;              // rollout_kernel<.., RolloutMode::kDrawTrajectory>: [n_steps][N][J] drawn actions, or nullptr
 };
+
+// Trajectory buffers (mt_rollout) are arrays of slices: slice s holds step s's rows 0 .. N-1, packed, so row `row` of
+// slice s starts at base + (s N + row) row_bytes.  Computed in 64 bits: s N row_bytes passes 2^32 at sizes users run
+// (2^20 envs x 36 steps x 120 B of observations).
+__host__ __device__ __forceinline__ unsigned long long slice_row_addr(unsigned long long base, unsigned long long s,
+                                                                      unsigned long long n, unsigned long long row,
+                                                                      unsigned long long row_bytes) {
+    return base + (s * n + row) * row_bytes;
+}
+// May a bulk copy (cp.async.bulk: store of an observation tile, L2 prefetch of an action tile) start at row `row` of
+// slice s?  It needs a 16-byte aligned global address; a misaligned one kills the context.  With a 16-byte aligned
+// base and `row` a multiple of the 32-env tile that is s N row_bytes % 16 == 0, which fails on some slices unless
+// N 3X % 4 == 0 (fp32 observations), N 3X % 8 == 0 (binary16) or N J % 4 == 0 (actions).  Decided per tile from the
+// address itself; a tile that may not goes the per-lane way.
+__host__ __device__ __forceinline__ bool bulk_aligned(unsigned long long addr) { return (addr & 15ull) == 0ull; }
+__host__ __device__ __forceinline__ bool slice_bulk_ok(unsigned long long base, unsigned long long s, unsigned long long n,
+                                                       unsigned long long row, unsigned long long row_bytes) {
+    return bulk_aligned(slice_row_addr(base, s, n, row, row_bytes));
+}
 
 __host__ __device__ __forceinline__ uint32_t alive_mask_of(const StepParams &P, uint32_t word) {
     return P.ep_shift ? (word & ((1u << P.ep_shift) - 1u)) : word;
@@ -754,6 +774,41 @@ __device__ __forceinline__ void load_scalars(const StepParams &P, int env32, Til
     s.cnt = ep_shift_of<X>(P) ? 0u : ld_hint(P.counters + env, keep);
 }
 
+// One env's row of J actions in a trajectory slice (rollout_kernel's trajectory modes), with the vector widths of
+// load_scalars: float4 at J = 4, float2 pairs for even J (rows of J floats are 16- / 8-byte aligned in every slice).
+// row = nullptr (an env past the shard's end): zeros, as load_scalars gives it.
+template <int J>
+__device__ __forceinline__ void load_action_row(const float *row, float *a, uint64_t pol) {
+    if (!row) {
+#pragma unroll
+        for (int i = 0; i < J; ++i) a[i] = 0.f;
+    } else if (J == 4) {
+        const float4 t = ld_hint(reinterpret_cast<const float4 *>(row), pol);
+        a[0] = t.x; a[1] = t.y; a[2] = t.z; a[3] = t.w;
+    } else if (J % 2 == 0) {
+#pragma unroll
+        for (int i = 0; i < J; i += 2) {
+            const float2 t = ld_hint(reinterpret_cast<const float2 *>(row + i), pol);
+            a[i] = t.x; a[i + 1] = t.y;
+        }
+    } else {
+#pragma unroll
+        for (int i = 0; i < J; ++i) a[i] = ld_hint(row + i, pol);
+    }
+}
+template <int J>
+__device__ __forceinline__ void store_action_row(float *row, const float *a, uint64_t pol) {
+    if (J == 4) {
+        st_hint(reinterpret_cast<float4 *>(row), make_float4(a[0], a[1], a[2], a[3]), pol);
+    } else if (J % 2 == 0) {
+#pragma unroll
+        for (int i = 0; i < J; i += 2) st_hint(reinterpret_cast<float2 *>(row + i), make_float2(a[i], a[i + 1]), pol);
+    } else {
+#pragma unroll
+        for (int i = 0; i < J; ++i) st_hint(row + i, a[i], pol);
+    }
+}
+
 // ---------------------------------------------------------------------------
 // What a step does to one env once its kinematics and objective walk are done (per lane, warp-converged):
 // reward / done (manytor.py:205-212, 258-259, 170-171), the block's statistics, and the auto-reset with
@@ -1165,11 +1220,27 @@ step_kernel(const __grid_constant__ StepParams P) {
 // read and write of the state (48 B), the read of the objectives (12 X B) and every launch boundary with its
 // staggered start and drain; results are bit-identical (same arithmetic, same action stream: step index of
 // the launch + s).  Algorithmic bytes per env-step: 12 X + 5 written, plus (48 + 12 X) / n_steps.
+//
+// MODE (RolloutMode) says where a step's actions come from and where its outputs go.  kDrawLast is
+// mt_rollout_random: every step overwrites the same outputs.  The trajectory modes (mt_rollout) write step s's
+// observations, reward and done into slice s of [n_steps][N] arrays (slice_row_addr); kDrawTrajectory also stores
+// the drawn actions when P.drawn is set, and kActionsTrajectory reads step s's actions from slice s of the caller's
+// [n_steps][N][J] array instead of drawing them, evaluating their sin / cos exactly as step_kernel<.., RAND = false, ..>
+// does (arbitrary floats: no ActionTrig table), with an L2 prefetch of the next step's action tile that costs no
+// register and no shared memory.
 // ---------------------------------------------------------------------------
-template <int ARM, int X, bool WOBS, bool F16>
+enum class RolloutMode : int {
+    kDrawLast = 0,             // in-kernel actions, outputs of the last step (mt_rollout_random)
+    kDrawTrajectory = 1,       // in-kernel actions, outputs of every step (mt_rollout, actions_dev = NULL)
+    kActionsTrajectory = 2,    // the caller's actions, outputs of every step (mt_rollout)
+};
+
+template <int ARM, int X, bool WOBS, bool F16, RolloutMode MODE>
 __global__ void __launch_bounds__(((ARM == 0) ? kMaxWarpsRefArm : kMaxWarpsGeneric) * kTile, 1)
 rollout_kernel(const __grid_constant__ StepParams P) {
     static_assert(WOBS || !F16, "F16 is an observation format");
+    constexpr bool TRAJ = MODE != RolloutMode::kDrawLast;
+    constexpr bool DRAW = MODE != RolloutMode::kActionsTrajectory;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ int queue_next;
     __shared__ unsigned int warps_done, warps_seen;
@@ -1230,10 +1301,23 @@ rollout_kernel(const __grid_constant__ StepParams P) {
             float rew = 0.f;
             uint8_t done = 0;
             for (int s = 0; s < P.n_steps; ++s) {
-                draw_actions(P, step0 + (unsigned long long)s, P.env_id_base + env32, J, sc.a);
+                const size_t srow = TRAJ ? (size_t)s * (size_t)n_envs : 0;      // first row of this step's slice
+                if constexpr (DRAW) {
+                    draw_actions(P, step0 + (unsigned long long)s, P.env_id_base + env32, J, sc.a);
+                    if (MODE == RolloutMode::kDrawTrajectory && P.drawn && valid)
+                        store_action_row<J>(P.drawn + (srow + env) * J, sc.a, pol_store);
+                } else {
+                    load_action_row<J>(valid ? P.actions + (srow + env) * J : nullptr, sc.a, pol_stream);
+                    // the next step's action tile towards the L2 while this step computes (a hint: aligned full tiles only)
+                    // (the address by pointer arithmetic, = slice_row_addr(actions, s + 1, N, env0, 4J): the 64-bit products
+                    // of slice_row_addr here cost rollout_kernel<0, 20, .., kActionsTrajectory> a spill)
+                    const float *next = P.actions + (srow + (size_t)n_envs + (size_t)env0) * J;
+                    if (full && lane == 0 && s + 1 < P.n_steps && bulk_aligned((uintptr_t)next))
+                        bulk_prefetch_l2(next, (uint32_t)(kTile * 4 * J));
+                }
                 Frames f;
-                if (ARM == 0) ref_arm<true>(sc.g, sc.a, P.substeps, P.inv_div, f, nullptr, trig);
-                else generic_arm<ARM, true>(P, sc.g, sc.a, f, nullptr, trig);
+                if (ARM == 0) ref_arm<DRAW>(sc.g, sc.a, P.substeps, P.inv_div, f, nullptr, trig);
+                else generic_arm<ARM, DRAW>(P, sc.g, sc.a, f, nullptr, trig);
                 const bool neg = f.zmin < 0.0f;
                 if (s == 0) mbar_wait_s(bar, k & 1u);
                 if (WOBS) {                                // the previous step's bulk store must have read the buffer
@@ -1249,20 +1333,24 @@ rollout_kernel(const __grid_constant__ StepParams P) {
 #pragma unroll
                 for (int i = 0; i < J; ++i) sc.g[i] = gn[i];
                 if (valid) {
-                    st_hint(P.reward + env, rew, pol_store);
-                    st_hint(P.done + env, done, pol_store);
+                    st_hint(P.reward + srow + env, rew, pol_store);
+                    st_hint(P.done + srow + env, done, pol_store);
                 }
                 if (WOBS) {
-                    if (full) {
+                    // a full tile whose slice address is misaligned takes the per-lane way (warp-uniform)
+                    const bool bulk = TRAJ ? full && slice_bulk_ok((uintptr_t)P.obs, (unsigned long long)s, (unsigned long long)n_envs,
+                                                                   (unsigned long long)env0, (unsigned long long)rowlen * (F16 ? 2 : 4))
+                                           : full;
+                    if (bulk) {
                         if (F16) pack_tile_f16<X>(obuf, rowlen, lane);
                         fence_async_smem();
                         __syncwarp();
                         if (lane == 0) {
-                            bulk_store_hint_s(obs_at<F16>(P.obs, (size_t)env0 * rowlen), obuf, F16 ? tile_bytes / 2 : tile_bytes, pol_store);
+                            bulk_store_hint_s(obs_at<F16>(P.obs, (srow + (size_t)env0) * rowlen), obuf, F16 ? tile_bytes / 2 : tile_bytes, pol_store);
                             bulk_commit();
                         }
                     } else if (valid) {
-                        void *dst = obs_at<F16>(P.obs, env * rowlen);
+                        void *dst = obs_at<F16>(P.obs, (srow + env) * rowlen);
                         for (int i = 0; i < rowlen; ++i) store_obs<F16>(dst, i, lds_f(orow + 4u * i));
                     }
                 }
