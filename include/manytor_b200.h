@@ -159,6 +159,24 @@ int mt_observe(mt_env *env, void *obs_dev, void *stream);
 int mt_step(mt_env *env, const float *actions_dev, void *obs_dev, float *reward_dev,
             uint8_t *done_dev, float *joints_dev, void *stream);
 
+/* mt_step plus what an episode that ends in this step leaves behind, which the in-kernel auto-reset
+ * otherwise wipes (Gymnasium's info["final_obs"] and the per-episode return / length of
+ * RecordEpisodeStatistics; V(final_obs) bootstraps a truncated episode):
+ *   final_obs_dev    [N][3X]  obs2 of the ending step (manytor.py:204), in the handle's obs format, bit for bit
+ *                             what mt_step returns for that env with obs_after_reset = 0
+ *   final_return_dev [N] fp32 total reward of the episode
+ *   final_length_dev [N] i32  its length: the episode-length counter, which saturates as
+ *                             mt_config.horizon documents
+ * Row n of each final array is written exactly when done[n] != 0; the other rows keep their contents.
+ * Everything else (obs, reward, done, joints, state, statistics, step index) is what mt_step computes.
+ * obs_dev and the three final pointers are required and 16-byte aligned; argument errors are reported
+ * before the handle is looked at.  A handle created without auto_reset returns MT_ERR_INVALID (without
+ * auto-reset nothing is lost: obs2 is the returned obs and mt_get_state holds the return and length);
+ * a call before the first mt_reset returns MT_ERR_STATE. */
+int mt_step_final(mt_env *env, const float *actions_dev, void *obs_dev, float *reward_dev, uint8_t *done_dev,
+                  float *joints_dev, void *final_obs_dev, float *final_return_dev, int32_t *final_length_dev,
+                  void *stream);
+
 /* Environment.action_sample / Multienv.action_sample -- manytor.py:215-217, 111-113:
  * integer degrees uniform on [action_low, action_high), Philox keyed by
  * (seed, global env id, step index). */

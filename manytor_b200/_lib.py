@@ -73,6 +73,7 @@ SIGNATURES = {
     "mt_reset": (C.c_int, [_P, _P, _P]),
     "mt_observe": (C.c_int, [_P, _P, _P]),
     "mt_step": (C.c_int, [_P, _P, _P, _P, _P, _P, _P]),
+    "mt_step_final": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "mt_sample_actions": (C.c_int, [_P, _P, _P]),
     "mt_rollout_random": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P]),
     "mt_rollout": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),

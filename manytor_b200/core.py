@@ -56,6 +56,11 @@ UR5_ARM = ArmSpec(
 # done (K, N) uint8, actions (K, N, J) float32 (the caller's, or the recorded draws) or None.
 Trajectory = namedtuple("Trajectory", "obs reward done actions")
 
+# What BatchedEnvs.step(final=True) appends: for each env that ended in the step (done != 0), the observation that
+# closed its episode (obs2, before the in-kernel reset; (N, 3X) of the handle's obs_dtype), the episode's return
+# ((N,) float32) and length ((N,) int32).  Rows of envs that did not end keep what an earlier step left there.
+FinalInfo = namedtuple("FinalInfo", "obs episode_return episode_length")
+
 
 # observation dtype -> mt_config.obs_dtype
 OBS_DTYPES = {torch.float32: _lib.MT_OBS_F32, torch.float16: _lib.MT_OBS_F16}
@@ -175,7 +180,7 @@ class BatchedEnvs:
                                terminate_on_ground, obs_after_reset, seed, fk_mode, substeps,
                                action_low, action_high, obs_dtype)
         _lib.check(self._lib.mt_create(C.byref(self.cfg), C.byref(self._h)))
-        self._obs = self._reward = self._done = self._joints = self._actions = None
+        self._obs = self._reward = self._done = self._joints = self._actions = self._final = None
         self._stream_keepalive = None
         self._pinned = {}
         self._pinned_ptr = {}                              # id(array) -> address, for the arrays in _pinned (kept alive there)
@@ -215,7 +220,7 @@ class BatchedEnvs:
             return None
         return self._as_dev(mask, torch.bool, (self.n,)).view(torch.uint8)
 
-    def _out_buffers(self, want_obs=True, want_joints=False):
+    def _out_buffers(self, want_obs=True, want_joints=False, want_final=False):
         if self._reward is None:
             self._reward = self._empty((self.n,), torch.float32)
             self._done = self._empty((self.n,), torch.uint8)
@@ -223,6 +228,9 @@ class BatchedEnvs:
             self._obs = self._empty((self.n, 3 * self.x), self.obs_dtype)
         if want_joints and self._joints is None:
             self._joints = self._empty((self.n, self.j, 3), torch.float32)
+        if want_final and self._final is None:
+            self._final = FinalInfo(self._empty((self.n, 3 * self.x), self.obs_dtype),
+                                    self._empty((self.n,), torch.float32), self._empty((self.n,), torch.int32))
 
     # -- reference operations --------------------------------------------------
     def reset(self, mask=None, returnable: bool = False):
@@ -245,25 +253,43 @@ class BatchedEnvs:
         _lib.check(self._lib.mt_observe(self._h, self._p(out), self._stream()))
         return out
 
-    def step(self, actions, joints: bool = False, write_obs: bool = True):
+    def step(self, actions, joints: bool = False, write_obs: bool = True, final: bool = False):
         """Environment.step / Multienv.step (manytor.py:255-260, 115-122).
 
         actions: (N, J) degrees.  Returns (obs (N,3X) obs_dtype, reward (N,) f32,
-        done (N,) u8 [, joints (N,J,3)]) -- views of buffers this object reuses
-        on the next step.
+        done (N,) u8 [, joints (N,J,3)] [, FinalInfo]) -- views of buffers this object
+        reuses on the next step.
+
+        final=True (mt_step_final; needs auto_reset and write_obs) appends a FinalInfo: the
+        last observation, return and length of every episode that ended in this step, in the
+        rows where done != 0, which the in-kernel reset would otherwise discard.
         """
+        if final:
+            if not write_obs:
+                raise ValueError("final=True needs write_obs=True: the final observation is the step's obs2")
+            if not self.cfg.auto_reset:
+                raise ValueError("final=True needs a handle created with auto_reset=True (without auto-reset the "
+                                 "returned obs is the final observation and get_state() holds the return and length)")
         if (isinstance(actions, torch.Tensor) and actions.is_cuda and actions.dtype == torch.float32
                 and actions.is_contiguous() and actions.numel() == self.n * self.j):
             a = actions                                    # fast path: already the device layout
         else:
             a = self._as_dev(actions, torch.float32, (self.n, self.j))
-        self._out_buffers(write_obs, joints)
-        _lib.check(self._lib.mt_step(self._h, self._p(a), self._p(self._obs if write_obs else None),
-                                     self._p(self._reward), self._p(self._done),
-                                     self._p(self._joints if joints else None), self._stream()))
+        self._out_buffers(write_obs, joints, final)
+        if final:
+            _lib.check(self._lib.mt_step_final(self._h, self._p(a), self._p(self._obs), self._p(self._reward),
+                                               self._p(self._done), self._p(self._joints if joints else None),
+                                               self._p(self._final.obs), self._p(self._final.episode_return),
+                                               self._p(self._final.episode_length), self._stream()))
+        else:
+            _lib.check(self._lib.mt_step(self._h, self._p(a), self._p(self._obs if write_obs else None),
+                                         self._p(self._reward), self._p(self._done),
+                                         self._p(self._joints if joints else None), self._stream()))
         self._actions = a  # keep alive until the stream has consumed it
         out = (self._obs if write_obs else None, self._reward, self._done)
-        return out + (self._joints,) if joints else out
+        if joints:
+            out += (self._joints,)
+        return out + (self._final,) if final else out
 
     def sample_actions(self, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Multienv.action_sample (manytor.py:111-113, 215-217): integer degrees, (N, J) f32."""

@@ -70,7 +70,7 @@ struct mt_env {
     bool jit = false;
     int jit_id = 0, jit_x = 0;
     std::string jit_preset;
-    cudaKernel_t jit_kernel[2][2] = {};      // [in-kernel actions][observations written] (in the handle's format)
+    cudaKernel_t jit_kernel[2][2][2] = {};   // [in-kernel actions][observations written] (in the handle's format)[final outputs]
     cudaKernel_t jit_rollout[3][2] = {};     // multi-step rollout kernel, [RolloutMode][observations written]
     bool jit_rollout_failed = false;
     float *goals = nullptr, *total_reward = nullptr, *points = nullptr;
@@ -392,10 +392,10 @@ extern "C" int mt_create(const mt_config *cfg, mt_env **out) {
             e->jit_id = runtime_table ? 1000 + nj : e->arm;
             e->jit_x = cfg->n_obj;                                    // compile-time X: unrolled objective walk
             e->jit_preset = runtime_table ? preset_source(e->jit_id, nj, e->base.arm) : std::string();
-            JitKernel k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, false, true, e->f16, err);
+            JitKernel k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, false, true, e->f16, false, err);
             if (k.kernel) {
                 e->jit = true;
-                e->jit_kernel[0][1] = k.kernel;
+                e->jit_kernel[0][1][0] = k.kernel;
             }
         }
         if (!e->jit && cfg->fk_mode == 3 && runtime_table) {
@@ -678,37 +678,43 @@ __global__ void r_theta_kernel(const float *v1, const float *v2, long long m, fl
 // ----------------------------------------------------------------------------
 typedef void (*StepFn)(const StepParams);
 
+// final: the FINAL = true kernels of mt_step_final, built only for the caller's actions with observations written
 template <int ARM, int X, bool RAND>
-static StepFn pick_obs(bool wobs, bool f16) {
-    if (!wobs) return step_kernel<ARM, X, RAND, false, false>;
-    return f16 ? step_kernel<ARM, X, RAND, true, true> : step_kernel<ARM, X, RAND, true, false>;
+static StepFn pick_obs(bool wobs, bool f16, bool final) {
+    if (final) {
+        if constexpr (RAND) return nullptr;
+        else if (!wobs) return nullptr;
+        else return f16 ? step_kernel<ARM, X, false, true, true, true> : step_kernel<ARM, X, false, true, false, true>;
+    }
+    if (!wobs) return step_kernel<ARM, X, RAND, false, false, false>;
+    return f16 ? step_kernel<ARM, X, RAND, true, true, false> : step_kernel<ARM, X, RAND, true, false, false>;
 }
 
 template <int ARM, int X>
-static StepFn pick_flags(bool rnd, bool wobs, bool f16) {
-    return rnd ? pick_obs<ARM, X, true>(wobs, f16) : pick_obs<ARM, X, false>(wobs, f16);
+static StepFn pick_flags(bool rnd, bool wobs, bool f16, bool final) {
+    return rnd ? pick_obs<ARM, X, true>(wobs, f16, final) : pick_obs<ARM, X, false>(wobs, f16, final);
 }
 
 template <int ARM>
-static StepFn pick_x(int x, bool rnd, bool wobs, bool f16) {
+static StepFn pick_x(int x, bool rnd, bool wobs, bool f16, bool final) {
     switch (x) {
-        case 10: return pick_flags<ARM, 10>(rnd, wobs, f16);
-        case 20: return pick_flags<ARM, 20>(rnd, wobs, f16);
-        default: return pick_flags<ARM, 0>(rnd, wobs, f16);
+        case 10: return pick_flags<ARM, 10>(rnd, wobs, f16, final);
+        case 20: return pick_flags<ARM, 20>(rnd, wobs, f16, final);
+        default: return pick_flags<ARM, 0>(rnd, wobs, f16, final);
     }
 }
 
-static StepFn pick_kernel(int arm, int x, bool rnd, bool wobs, bool f16) {
+static StepFn pick_kernel(int arm, int x, bool rnd, bool wobs, bool f16, bool final) {
     switch (arm) {
-        case 0: return pick_x<0>(x, rnd, wobs, f16);
-        case 2: return pick_flags<2, 0>(rnd, wobs, f16);
-        case 3: return pick_flags<3, 0>(rnd, wobs, f16);
-        case 4: return pick_flags<4, 0>(rnd, wobs, f16);
-        case 5: return pick_flags<5, 0>(rnd, wobs, f16);
-        case 6: return pick_x<6>(x, rnd, wobs, f16);
-        case 7: return pick_flags<7, 0>(rnd, wobs, f16);
-        case 8: return pick_flags<8, 0>(rnd, wobs, f16);
-#define MT_PICK(ID) case ID: return pick_x<ID>(x, rnd, wobs, f16);
+        case 0: return pick_x<0>(x, rnd, wobs, f16, final);
+        case 2: return pick_flags<2, 0>(rnd, wobs, f16, final);
+        case 3: return pick_flags<3, 0>(rnd, wobs, f16, final);
+        case 4: return pick_flags<4, 0>(rnd, wobs, f16, final);
+        case 5: return pick_flags<5, 0>(rnd, wobs, f16, final);
+        case 6: return pick_x<6>(x, rnd, wobs, f16, final);
+        case 7: return pick_flags<7, 0>(rnd, wobs, f16, final);
+        case 8: return pick_flags<8, 0>(rnd, wobs, f16, final);
+#define MT_PICK(ID) case ID: return pick_x<ID>(x, rnd, wobs, f16, final);
         MT_FOR_EACH_PRESET_ARM(MT_PICK)
 #undef MT_PICK
     }
@@ -801,9 +807,11 @@ static int launch_pdl(const void *fn, const LaunchShape &shape, const StepParams
     return MT_OK;
 }
 
-// launch the fused step kernel over tiles [t0, t1): a persistent grid sized to the SMs
+// launch the fused step kernel over tiles [t0, t1): a persistent grid sized to the SMs.  final_obs != nullptr selects
+// the FINAL = true kernel (mt_step_final), which also writes final_return / final_length.
 static int launch_step(mt_env *e, const float *actions, void *obs, float *reward, uint8_t *done, float *joints,
-                       bool rnd, long long t0, long long t1, cudaStream_t st, int ticket_slot = 0, bool advance = true) {
+                       bool rnd, long long t0, long long t1, cudaStream_t st, int ticket_slot = 0, bool advance = true,
+                       void *final_obs = nullptr, float *final_return = nullptr, int32_t *final_length = nullptr) {
     StepParams P = e->base;
     P.actions = actions;
     P.obs = obs;
@@ -819,18 +827,21 @@ static int launch_step(mt_env *e, const float *actions, void *obs, float *reward
     P.advance = advance ? 1 : 0;
     P.n_steps = 1;
     P.launch_envs = ((t1 * kTile < e->n) ? t1 * kTile : e->n) - t0 * kTile;
-    const bool wobs = obs != nullptr;
+    P.final_obs = final_obs;
+    P.final_return = final_return;
+    P.final_length = final_length;
+    const bool wobs = obs != nullptr, final = final_obs != nullptr;
     const void *fn = nullptr;
     if (e->jit) {
-        cudaKernel_t &k = e->jit_kernel[rnd ? 1 : 0][wobs ? 1 : 0];
+        cudaKernel_t &k = e->jit_kernel[rnd ? 1 : 0][wobs ? 1 : 0][final ? 1 : 0];
         if (!k) {                                             // other variants compile on first use
             std::string err;
-            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, rnd, wobs, e->f16, err).kernel;
+            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, rnd, wobs, e->f16, final, err).kernel;
             if (!k) return fail(MT_ERR_CUDA, "run-time specialisation failed: %s", err.c_str());
         }
         fn = (const void *)k;
     } else {
-        fn = (const void *)pick_kernel(e->arm, e->cfg.n_obj, rnd, wobs, e->f16);
+        fn = (const void *)pick_kernel(e->arm, e->cfg.n_obj, rnd, wobs, e->f16, final);
     }
     if (!fn) return fail(MT_ERR_INVALID, "no kernel for arm=%d", e->arm);
     const size_t nb = e->arm == 0 ? StepBuffers<0>::value : StepBuffers<1>::value;   // tile buffers per warp
@@ -892,7 +903,7 @@ static int launch_rollout(mt_env *e, RolloutMode mode, int n_steps, const float 
         cudaKernel_t &k = e->jit_rollout[(int)mode][obs ? 1 : 0];
         if (!k) {
             std::string err;
-            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, true, obs != nullptr, e->f16, err, (int)mode).kernel;
+            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, true, obs != nullptr, e->f16, false, err, (int)mode).kernel;
             if (!k) {
                 e->jit_rollout_failed = true;                 // keep working through the per-step launches
                 return MT_OK;
@@ -995,6 +1006,31 @@ extern "C" int mt_step(mt_env *e, const float *actions_dev, void *obs_dev, float
     cudaStream_t st = (cudaStream_t)stream;
     if ((rc = timing_begin(e, st))) return rc;
     if ((rc = launch_step(e, actions_dev, obs_dev, reward_dev, done_dev, joints_dev, false, 0, e->n_tiles, st))) return rc;
+    return timing_end(e, st);
+}
+
+extern "C" int mt_step_final(mt_env *e, const float *actions_dev, void *obs_dev, float *reward_dev, uint8_t *done_dev,
+                             float *joints_dev, void *final_obs_dev, float *final_return_dev, int32_t *final_length_dev,
+                             void *stream) {
+    // the arguments first: none of these checks needs the handle or a device
+    int rc;
+    if ((rc = check_ptr(actions_dev, "actions_dev", true))) return rc;
+    if ((rc = check_ptr(obs_dev, "obs_dev", true))) return rc;
+    if (!reward_dev || !done_dev) return fail(MT_ERR_INVALID, "reward_dev/done_dev is NULL");
+    if ((rc = check_ptr(final_obs_dev, "final_obs_dev", true))) return rc;
+    if ((rc = check_ptr(final_return_dev, "final_return_dev", true))) return rc;
+    if ((rc = check_ptr(final_length_dev, "final_length_dev", true))) return rc;
+    if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    if (!e->cfg.auto_reset)
+        return fail(MT_ERR_INVALID, "mt_step_final needs a handle created with auto_reset (without it obs2 is the returned "
+                                    "observation and mt_get_state holds the return and length)");
+    if (!e->was_reset) return fail(MT_ERR_STATE, "mt_step_final before mt_reset (the reference raises IndexError here, manytor.py:143)");
+    DeviceGuard guard(e->cfg.device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = timing_begin(e, st))) return rc;
+    if ((rc = launch_step(e, actions_dev, obs_dev, reward_dev, done_dev, joints_dev, false, 0, e->n_tiles, st, 0, true,
+                          final_obs_dev, final_return_dev, final_length_dev)))
+        return rc;
     return timing_end(e, st);
 }
 

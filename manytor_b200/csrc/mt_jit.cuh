@@ -2,7 +2,7 @@
 //
 // A preset arm (mt_step.cuh) gets its DH table folded at compile time; this file gives ANY table the
 // same treatment without rebuilding the library: at mt_create the table is printed into a
-// `Preset<ID>` specialisation, NVRTC compiles `step_kernel<ID, X, RAND, WOBS, F16>` for sm_100a from the
+// `Preset<ID>` specialisation, NVRTC compiles `step_kernel<ID, X, RAND, WOBS, F16, FINAL>` for sm_100a from the
 // very same headers the library was built from (embedded as strings by manytor_b200/build.py), and
 // the cubin is loaded through the runtime's library API.  ~0.8 s per variant, cached per process.
 // NVRTC is dlopen'ed: when it is absent the handle simply keeps the run-time-table kernels.
@@ -91,13 +91,13 @@ static std::string preset_source(int id, int J, const JointConst *rows) {
     return s;
 }
 
-// Compile (or fetch from the per-process cache) step_kernel<id, x_template, rnd, wobs, f16> for the table
+// Compile (or fetch from the per-process cache) step_kernel<id, x_template, rnd, wobs, f16, final> for the table
 // described by `preset`.  Returns an empty JitKernel and fills `err` on failure.
 // `rollout_mode` >= 0 selects the multi-step rollout_kernel<id, x_template, wobs, f16, RolloutMode(rollout_mode)>
-// (`rnd` is ignored).  The cache key holds the template arguments, so handles with the same table and different
-// observation formats or rollout modes get different kernels.
+// (`rnd` and `final` are ignored).  The cache key holds the template arguments, so handles with the same table and
+// different observation formats, final outputs or rollout modes get different kernels.
 static JitKernel jit_step_kernel(const std::string &preset, int id, int x_template, bool rnd, bool wobs, bool f16,
-                                 std::string &err, int rollout_mode = -1) {
+                                 bool final, std::string &err, int rollout_mode = -1) {
     static std::mutex mu;
     static std::map<std::string, JitKernel> cache;
     static const char *const kModes[] = {"mt::RolloutMode::kDrawLast", "mt::RolloutMode::kDrawTrajectory",
@@ -106,7 +106,7 @@ static JitKernel jit_step_kernel(const std::string &preset, int id, int x_templa
     const char *obs = wobs ? (f16 ? "true, true" : "true, false") : "false, false";
     const std::string targs = rollout ? std::to_string(id) + ", " + std::to_string(x_template) + ", " + obs + ", " + kModes[rollout_mode]
                                       : std::to_string(id) + ", " + std::to_string(x_template) + ", " + (rnd ? "true" : "false") +
-                                            ", " + obs;
+                                            ", " + obs + (final ? ", true" : ", false");
     const std::string kname = rollout ? "rollout_kernel" : "step_kernel";
     const std::string inst = "mt::" + kname + "<" + targs + ">";
     const std::string key = preset + inst;

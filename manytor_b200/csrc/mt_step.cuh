@@ -109,6 +109,11 @@ struct StepParams {
     // whole state fits its budget, evict_first beyond (mt_create; measured both ways in round 2).
     unsigned long long pol_state, pol_stream, pol_store;   // pol_store: the streamed OUTPUTS (observations, reward, done)
     float *drawn;              // rollout_kernel<.., RolloutMode::kDrawTrajectory>: [n_steps][N][J] drawn actions, or nullptr
+    // step_kernel<.., FINAL = true> (mt_step_final): what an ending env's episode leaves behind, written for the rows
+    // of the envs that end in this step only (settle_step)
+    void *final_obs;           // [N][3X] obs2 of the ending step, in the handle's obs format
+    float *final_return;       // [N] total reward of the episode
+    int32_t *final_length;     // [N] episode length (the saturating counter)
 };
 
 // Trajectory buffers (mt_rollout) are arrays of slices: slice s holds step s's rows 0 .. N-1, packed, so row `row` of
@@ -821,13 +826,19 @@ __device__ __forceinline__ void store_action_row(float *row, const float *a, uin
 // Resets are rare (one env-step in ~550 for random actions), so the warp handles its ending envs one at a
 // time and COOPERATIVELY: lane p draws objective p (x <= 32 lanes busy) instead of the one ending lane
 // drawing all x while 31 lanes idle.
+// FINAL (mt_step_final, needs WOBS): before the reset wipes them, an ending env's return and length go to
+// P.final_return / P.final_length, and its obs2 row -- still fp32 at obs_buf, in the public order -- to
+// P.final_obs (binary16 when F16, rounded as pack_tile_f16 rounds), lane p copying objective p's three words
+// ahead of the first observation of the new episode that replaces them.  Rows of envs that go on are not
+// touched.
 // ---------------------------------------------------------------------------
-template <int J, bool WOBS>
+template <int J, bool WOBS, bool FINAL = false, bool F16 = false>
 __device__ __forceinline__ void settle_step(const StepParams &P, int lane, int env0, bool valid, int x, int rowlen, bool neg,
                                             uint32_t alive0, uint32_t caught, const float *a, float *gn, float &total,
                                             uint32_t &alive1, uint32_t &eplen, float &rew, uint8_t &done,
                                             uint32_t &ground_steps, unsigned long long *blk_stat, uint32_t obs_buf,
                                             uint32_t pts_buf) {
+    static_assert(WOBS || !FINAL, "the final observation is the tile's obs2");
     alive1 = alive0 & ~caught;                                             // manytor.py:168
     rew = (alive1 != alive0) ? 1.0f : 0.0f;
     rew = neg ? -1.0f : rew;
@@ -855,6 +866,11 @@ __device__ __forceinline__ void settle_step(const StepParams &P, int lane, int e
             atomicAdd(&blk_stat[3], (unsigned long long)l_sum);
             atomicAdd(&blk_stat[4], (unsigned long long)c_sum);
         }
+        if (FINAL && ending) {
+            const size_t env = (size_t)(env0 + lane);
+            P.final_return[env] = total;
+            P.final_length[env] = (int32_t)eplen;
+        }
     }
     if (ending) {
 #pragma unroll
@@ -871,6 +887,13 @@ __device__ __forceinline__ void settle_step(const StepParams &P, int lane, int e
         __syncwarp();
         if (lane == src) P.episode[renv] = ep + 1u;
         if (lane < x) {
+            if (FINAL) {
+                const uint32_t orow = obs_buf + (uint32_t)(src * rowlen + lane * 3) * 4u;
+                const size_t i = renv * (size_t)rowlen + (size_t)(lane * 3);
+                store_obs<F16>(P.final_obs, i, lds_f(orow));
+                store_obs<F16>(P.final_obs, i + 1, lds_f(orow + 4));
+                store_obs<F16>(P.final_obs, i + 2, lds_f(orow + 8));
+            }
             float px, py, pz;
             if (P.obj_stream) {
                 const float *srcp = P.obj_stream + (((size_t)(ep % (uint32_t)P.obj_sets) * (size_t)P.n + renv) * x + lane) * 3;
@@ -964,6 +987,7 @@ __device__ __forceinline__ void block_epilogue(const StepParams &P, int lane, in
 //   X    objectives per env, 0 = run-time P.n_obj
 //   RAND draw actions in-kernel (mt_rollout_random)   WOBS write observations
 //   F16  observations leave as binary16 (pack_tile_f16); only instantiated with WOBS
+//   FINAL an ending env's obs2, return and length to P.final_* (mt_step_final, settle_step); only with WOBS
 //
 // Persistent blocks: one per SM (as many warps as the SM holds; several smaller
 // blocks for launches with few tiles), each owning every G-th tile and handing
@@ -985,7 +1009,7 @@ __device__ __forceinline__ unsigned long long trace_now() {
 }
 #endif
 
-template <int ARM, int X, bool RAND, bool WOBS, bool F16>
+template <int ARM, int X, bool RAND, bool WOBS, bool F16, bool FINAL>
 __global__ void __launch_bounds__(((ARM == 0) ? kMaxWarpsRefArm : kMaxWarpsGeneric) * kTile, 1)
 step_kernel(const __grid_constant__ StepParams P) {
     static_assert(WOBS || !F16, "F16 is an observation format");
@@ -1136,8 +1160,8 @@ step_kernel(const __grid_constant__ StepParams P) {
             uint32_t alive1;
             uint8_t done;
             if (ep_shift) eplen = word >> ep_shift;
-            settle_step<J, WOBS>(P, lane, env0, valid, x, rowlen, neg, alive0, caught, sc.a, gn, total, alive1, eplen, rew, done,
-                                 ground_steps, blk_stat, buf_cur, 0u);
+            settle_step<J, WOBS, FINAL, F16>(P, lane, env0, valid, x, rowlen, neg, alive0, caught, sc.a, gn, total, alive1, eplen,
+                                             rew, done, ground_steps, blk_stat, buf_cur, 0u);
 
             // 7. write back: state (coalesced), then the observation tile by one bulk store
             if (J == 4) {

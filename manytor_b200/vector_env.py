@@ -13,8 +13,18 @@ same GPU consumes it directly; `torch.utils.dlpack.to_dlpack(obs)` / `obs.__dlpa
 same memory to JAX/CuPy without a copy.  Auto-reset is "same-step": an env that terminates
 (all objectives collected, manytor.py:170-171) or is truncated (horizon reached, the `max_steps` of
 the reference's driver scripts) is reset inside the step kernel and the observation returned for it
-is the FIRST observation of its next episode.  No gymnasium import is needed; the space attributes
-are plain shape/bound tuples.
+is the FIRST observation of its next episode.
+
+With `final_info=True` the observation that closed the episode (obs2 of the ending step, which a
+truncated episode needs to bootstrap its return from V(final_obs)) and the episode's return and length
+come back in `info`, written by the same kernel (mt_step_final), as device tensors:
+
+    {"final_obs": (N, 3X), "_final_obs": terminated | truncated,
+     "episode": {"r": (N,) float32, "l": (N,) int32}, "_episode": terminated | truncated}
+
+Rows outside the masks are unspecified.  With the default `final_info=False` that observation, return
+and length are gone after the step and `info` is empty.  No gymnasium import is needed; the space
+attributes are plain shape/bound tuples.
 """
 from __future__ import annotations
 
@@ -30,8 +40,9 @@ class ManyTorVectorEnv:
 
     def __init__(self, num_envs: int, obj_number: int = 10, arm: ArmSpec = REFERENCE_ARM, max_episode_steps: int = 200,
                  device=None, seed: int = 0, terminate_on_ground: bool = False, env_id_base: int = 0,
-                 obs_dtype=torch.float32):
+                 obs_dtype=torch.float32, final_info: bool = False):
         self.num_envs = int(num_envs)
+        self.final_info = bool(final_info)
         self.envs = BatchedEnvs(num_envs, obj_number, arm=arm, device=device, env_id_base=env_id_base,
                                 horizon=max_episode_steps, auto_reset=True, obs_after_reset=True,
                                 terminate_on_ground=terminate_on_ground, seed=seed, obs_dtype=obs_dtype)
@@ -49,10 +60,18 @@ class ManyTorVectorEnv:
         return obs, {}
 
     def step(self, actions):
-        obs, reward, done = self.envs.step(actions)
+        if self.final_info:
+            obs, reward, done, final = self.envs.step(actions, final=True)
+        else:
+            obs, reward, done = self.envs.step(actions)
         terminated = (done & 1).bool()
         truncated = (done & 2).bool()
-        return obs, reward, terminated, truncated, {}
+        if not self.final_info:
+            return obs, reward, terminated, truncated, {}
+        ended = terminated | truncated
+        info = {"final_obs": final.obs, "_final_obs": ended,
+                "episode": {"r": final.episode_return, "l": final.episode_length}, "_episode": ended}
+        return obs, reward, terminated, truncated, info
 
     def sample_actions(self) -> torch.Tensor:
         """Uniform integer-degree actions like `action_sample()` (manytor.py:215-217), on device."""
