@@ -216,6 +216,27 @@ int mt_rollout_random(mt_env *env, int32_t n_steps, void *obs_dev, float *reward
 int mt_rollout(mt_env *env, int32_t n_steps, const float *actions_dev, float *drawn_dev, void *obs_dev,
                float *reward_dev, uint8_t *done_dev, void *stream);
 
+/* mt_rollout plus, for every step, what mt_step_final adds to mt_step: the final observation, return and
+ * length of each episode that ends inside the trajectory, which the in-kernel auto-reset otherwise wipes.
+ *   actions_dev, drawn_dev, reward_dev, done_dev  exactly as in mt_rollout
+ *   obs_dev            [n_steps][N][3X] required (the final observation is the step's obs2)
+ *   final_obs_dev      [n_steps][N][3X] in the handle's obs format
+ *   final_return_dev   [n_steps][N] fp32
+ *   final_length_dev   [n_steps][N] i32
+ * Slice s of every output, the final arrays included, is bit for bit what the s-th of n_steps consecutive
+ * mt_step_final calls writes (with the caller's actions, or the draws mt_rollout makes).  Row n of final
+ * slice s is written exactly when done[s][n] != 0; every other row keeps its contents.  Every pointer
+ * but drawn_dev is required, and all are 16-byte aligned.  Argument errors are reported before the
+ * handle is looked at, in mt_rollout's order and then mt_step_final's.  A handle without auto_reset
+ * returns MT_ERR_INVALID, a call before the first mt_reset MT_ERR_STATE; n_steps < 0 is MT_ERR_INVALID,
+ * n_steps = 0 does nothing.  One launch of the multi-step rollout kernel per 4096 steps, as mt_rollout;
+ * where mt_rollout takes one step-kernel launch per step, in-kernel draws here take two (the draw, as
+ * mt_sample_actions makes it, then the step with those actions).  The final rows cost 12X + 8 bytes per
+ * ending episode and nothing for the envs that go on. */
+int mt_rollout_final(mt_env *env, int32_t n_steps, const float *actions_dev, float *drawn_dev, void *obs_dev,
+                     float *reward_dev, uint8_t *done_dev, void *final_obs_dev, float *final_return_dev,
+                     int32_t *final_length_dev, void *stream);
+
 /* Host-buffer step: actions_host/obs_host/reward_host/done_host must be pinned
  * (mt_host_alloc).  Copies actions H2D, steps, copies results D2H, chunked over
  * internal streams so copies overlap the kernels; synchronous on return.  Ordered after

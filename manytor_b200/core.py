@@ -59,6 +59,7 @@ Trajectory = namedtuple("Trajectory", "obs reward done actions")
 # What BatchedEnvs.step(final=True) appends: for each env that ended in the step (done != 0), the observation that
 # closed its episode (obs2, before the in-kernel reset; (N, 3X) of the handle's obs_dtype), the episode's return
 # ((N,) float32) and length ((N,) int32).  Rows of envs that did not end keep what an earlier step left there.
+# BatchedEnvs.rollout(final=True) returns one slice per step: (K, N, 3X), (K, N) and (K, N).
 FinalInfo = namedtuple("FinalInfo", "obs episode_return episode_length")
 
 
@@ -265,11 +266,7 @@ class BatchedEnvs:
         rows where done != 0, which the in-kernel reset would otherwise discard.
         """
         if final:
-            if not write_obs:
-                raise ValueError("final=True needs write_obs=True: the final observation is the step's obs2")
-            if not self.cfg.auto_reset:
-                raise ValueError("final=True needs a handle created with auto_reset=True (without auto-reset the "
-                                 "returned obs is the final observation and get_state() holds the return and length)")
+            self._check_final(write_obs)
         if (isinstance(actions, torch.Tensor) and actions.is_cuda and actions.dtype == torch.float32
                 and actions.is_contiguous() and actions.numel() == self.n * self.j):
             a = actions                                    # fast path: already the device layout
@@ -304,8 +301,34 @@ class BatchedEnvs:
                                                self._p(self._reward), self._p(self._done), self._stream()))
         return (self._obs if write_obs else None, self._reward, self._done)
 
+    def _check_final(self, write_obs: bool):
+        if not write_obs:
+            raise ValueError("final=True needs write_obs=True: the final observation is the step's obs2")
+        if not self.cfg.auto_reset:
+            raise ValueError("final=True needs a handle created with auto_reset=True (without auto-reset the "
+                             "returned obs is the final observation and get_state() holds the return and length)")
+
+    def _check_out(self, out, kind, arg, want, flags):
+        """Validate a preallocated `out` / `final_out` namedtuple against want = {field: (shape, dtype) or None}."""
+        if not isinstance(out, kind):
+            raise ValueError(f"{arg} must be a {kind.__name__}")
+        for name, spec in want.items():
+            t = getattr(out, name)
+            if spec is None:
+                if t is not None:
+                    raise ValueError(f"{arg}.{name} must be None here ({flags})")
+                continue
+            if not isinstance(t, torch.Tensor):
+                raise ValueError(f"{arg}.{name} must be a tensor of shape {spec[0]} and dtype {spec[1]}")
+            if tuple(t.shape) != spec[0] or t.dtype != spec[1]:
+                raise ValueError(f"{arg}.{name} must have shape {spec[0]} and dtype {spec[1]}, "
+                                 f"not {tuple(t.shape)} {t.dtype}")
+            if not t.is_contiguous() or t.device != self.device:
+                raise ValueError(f"{arg}.{name} must be a contiguous tensor on {self.device}")
+
     def rollout(self, actions=None, n_steps: Optional[int] = None, write_obs: bool = True,
-                record_actions: bool = False, out: Optional[Trajectory] = None) -> Trajectory:
+                record_actions: bool = False, out: Optional[Trajectory] = None, final: bool = False,
+                final_out: Optional[FinalInfo] = None):
         """K steps in one call, keeping every step: slice s of the returned Trajectory is what the s-th of K
         consecutive `step` calls would have returned, bit for bit (mt_rollout).
 
@@ -314,7 +337,16 @@ class BatchedEnvs:
         `record_actions=True` returns the drawn actions as well.  `out`: a Trajectory of preallocated buffers
         (obs of this handle's obs_dtype, or None when write_obs is False; actions only with record_actions),
         e.g. fixed storage for a CUDA graph that captures this call.  Shape and dtype errors raise ValueError
-        before the library is called."""
+        before the library is called.
+
+        final=True (mt_rollout_final; needs auto_reset and write_obs) returns (Trajectory, FinalInfo): slice s of
+        the FinalInfo holds, in the rows where done[s] != 0, what `step(final=True)` would have returned at step s
+        -- the last observation ((K, N, 3X)), return and length ((K, N)) of every episode that ended there.  Other
+        rows keep their contents.  `final_out`: a FinalInfo of preallocated buffers, checked like `out`."""
+        if final:
+            self._check_final(write_obs)
+        elif final_out is not None:
+            raise ValueError("final_out needs final=True")
         if actions is not None:
             if record_actions:
                 raise ValueError("record_actions records in-kernel draws: it cannot be combined with actions")
@@ -334,25 +366,19 @@ class BatchedEnvs:
                 "reward": ((k, self.n), torch.float32), "done": ((k, self.n), torch.uint8),
                 "actions": ((k, self.n, self.j), torch.float32) if record_actions else None}
         if out is not None:
-            if not isinstance(out, Trajectory):
-                raise ValueError("out must be a Trajectory")
-            for name, spec in want.items():
-                t = getattr(out, name)
-                if spec is None:
-                    if t is not None:
-                        raise ValueError(f"out.{name} must be None here (write_obs={write_obs}, "
-                                         f"record_actions={record_actions})")
-                    continue
-                if not isinstance(t, torch.Tensor):
-                    raise ValueError(f"out.{name} must be a tensor of shape {spec[0]} and dtype {spec[1]}")
-                if tuple(t.shape) != spec[0] or t.dtype != spec[1]:
-                    raise ValueError(f"out.{name} must have shape {spec[0]} and dtype {spec[1]}, "
-                                     f"not {tuple(t.shape)} {t.dtype}")
-                if not t.is_contiguous() or t.device != self.device:
-                    raise ValueError(f"out.{name} must be a contiguous tensor on {self.device}")
+            self._check_out(out, Trajectory, "out", want, f"write_obs={write_obs}, record_actions={record_actions}")
             bufs = out
         else:
             bufs = Trajectory(*(self._empty(*spec) if spec is not None else None for spec in want.values()))
+        fin = None
+        if final:
+            want_fin = {"obs": ((k, self.n, 3 * self.x), self.obs_dtype), "episode_return": ((k, self.n), torch.float32),
+                        "episode_length": ((k, self.n), torch.int32)}
+            if final_out is not None:
+                self._check_out(final_out, FinalInfo, "final_out", want_fin, "")
+                fin = final_out
+            else:
+                fin = FinalInfo(*(self._empty(*spec) for spec in want_fin.values()))
         if actions is not None:
             if (isinstance(actions, torch.Tensor) and actions.is_cuda and actions.device == self.device
                     and actions.dtype == torch.float32 and actions.is_contiguous()):
@@ -361,12 +387,17 @@ class BatchedEnvs:
                 a = self._as_dev(actions, torch.float32, (k, self.n, self.j))
             bufs = bufs._replace(actions=a)
         if k == 0:                                         # nothing to do (and empty tensors have no address)
-            return bufs
-        _lib.check(self._lib.mt_rollout(self._h, k, self._p(a if actions is not None else None),
-                                        self._p(bufs.actions if actions is None else None), self._p(bufs.obs),
-                                        self._p(bufs.reward), self._p(bufs.done), self._stream()))
-        self._rollout_io = bufs                            # keep alive until the stream has consumed them
-        return bufs
+            return (bufs, fin) if final else bufs
+        a_p, d_p = self._p(a if actions is not None else None), self._p(bufs.actions if actions is None else None)
+        if final:
+            _lib.check(self._lib.mt_rollout_final(self._h, k, a_p, d_p, self._p(bufs.obs), self._p(bufs.reward),
+                                                  self._p(bufs.done), self._p(fin.obs), self._p(fin.episode_return),
+                                                  self._p(fin.episode_length), self._stream()))
+        else:
+            _lib.check(self._lib.mt_rollout(self._h, k, a_p, d_p, self._p(bufs.obs), self._p(bufs.reward),
+                                            self._p(bufs.done), self._stream()))
+        self._rollout_io = (bufs, fin)                     # keep alive until the stream has consumed them
+        return (bufs, fin) if final else bufs
 
     # -- host-buffer (end-to-end) step ------------------------------------------
     def pinned(self, name: str, shape, dtype) -> np.ndarray:

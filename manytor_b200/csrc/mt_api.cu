@@ -71,7 +71,7 @@ struct mt_env {
     int jit_id = 0, jit_x = 0;
     std::string jit_preset;
     cudaKernel_t jit_kernel[2][2][2] = {};   // [in-kernel actions][observations written] (in the handle's format)[final outputs]
-    cudaKernel_t jit_rollout[3][2] = {};     // multi-step rollout kernel, [RolloutMode][observations written]
+    cudaKernel_t jit_rollout[3][2][2] = {};  // multi-step rollout kernel, [RolloutMode][observations written][final outputs]
     bool jit_rollout_failed = false;
     float *goals = nullptr, *total_reward = nullptr, *points = nullptr;
     uint32_t *alive = nullptr, *counters = nullptr, *episode = nullptr;
@@ -91,6 +91,7 @@ struct mt_env {
     float *scratch_reward = nullptr;       // mt_rollout_random with reward_dev / done_dev = NULL
     uint8_t *scratch_done = nullptr;
     void *scratch_obs = nullptr;           // mt_rollout's per-step path: one step's observations for a misaligned slice
+    float *scratch_actions = nullptr;      // mt_rollout_final's per-step path: one step's draws when drawn_dev is NULL
     float *fetch_dev = nullptr, *fetch_host = nullptr;
     int64_t *stats_dev = nullptr, *stats_pin = nullptr;
     StepParams base;
@@ -415,7 +416,7 @@ extern "C" int mt_destroy(mt_env *e) {
     cudaFree(e->goals); cudaFree(e->alive); cudaFree(e->total_reward); cudaFree(e->counters);
     cudaFree(e->episode); cudaFree(e->points); cudaFree(e->stats); cudaFree(e->ctrl);
     cudaFree(e->fetch_dev); cudaFree(e->stats_dev); cudaFree(e->scratch_reward); cudaFree(e->scratch_done);
-    cudaFree(e->scratch_obs);
+    cudaFree(e->scratch_obs); cudaFree(e->scratch_actions);
     if (e->fetch_host) cudaFreeHost(e->fetch_host);
     if (e->stats_pin) cudaFreeHost(e->stats_pin);
     cudaFree(e->h_actions); cudaFree(e->h_obs); cudaFree(e->h_reward); cudaFree(e->h_done);
@@ -855,55 +856,64 @@ static int launch_step(mt_env *e, const float *actions, void *obs, float *reward
 
 // Multi-step rollout in ONE launch (rollout_kernel, mt_step.cuh): built-in arms and handles whose kernels come
 // from NVRTC; run-time DH tables take the per-step launches instead (`launched` stays false).
+// final: the FINAL = true kernels of mt_rollout_final, built only for the trajectory modes with observations written
 template <int ARM, int X, RolloutMode MODE>
-static StepFn pick_rollout_obs(bool wobs, bool f16) {
-    if (!wobs) return rollout_kernel<ARM, X, false, false, MODE>;
-    return f16 ? rollout_kernel<ARM, X, true, true, MODE> : rollout_kernel<ARM, X, true, false, MODE>;
+static StepFn pick_rollout_obs(bool wobs, bool f16, bool final) {
+    if (final) {
+        if constexpr (MODE == RolloutMode::kDrawLast) return nullptr;
+        else if (!wobs) return nullptr;
+        else return f16 ? rollout_kernel<ARM, X, true, true, MODE, true> : rollout_kernel<ARM, X, true, false, MODE, true>;
+    }
+    if (!wobs) return rollout_kernel<ARM, X, false, false, MODE, false>;
+    return f16 ? rollout_kernel<ARM, X, true, true, MODE, false> : rollout_kernel<ARM, X, true, false, MODE, false>;
 }
 
 template <int ARM, int X>
-static StepFn pick_rollout_mode(RolloutMode mode, bool wobs, bool f16) {
+static StepFn pick_rollout_mode(RolloutMode mode, bool wobs, bool f16, bool final) {
     switch (mode) {
-        case RolloutMode::kDrawLast: return pick_rollout_obs<ARM, X, RolloutMode::kDrawLast>(wobs, f16);
-        case RolloutMode::kDrawTrajectory: return pick_rollout_obs<ARM, X, RolloutMode::kDrawTrajectory>(wobs, f16);
-        case RolloutMode::kActionsTrajectory: return pick_rollout_obs<ARM, X, RolloutMode::kActionsTrajectory>(wobs, f16);
+        case RolloutMode::kDrawLast: return pick_rollout_obs<ARM, X, RolloutMode::kDrawLast>(wobs, f16, final);
+        case RolloutMode::kDrawTrajectory: return pick_rollout_obs<ARM, X, RolloutMode::kDrawTrajectory>(wobs, f16, final);
+        case RolloutMode::kActionsTrajectory: return pick_rollout_obs<ARM, X, RolloutMode::kActionsTrajectory>(wobs, f16, final);
     }
     return nullptr;
 }
 
 template <int ARM>
-static StepFn pick_rollout_x(int x, RolloutMode mode, bool wobs, bool f16) {
+static StepFn pick_rollout_x(int x, RolloutMode mode, bool wobs, bool f16, bool final) {
     switch (x) {
-        case 10: return pick_rollout_mode<ARM, 10>(mode, wobs, f16);
-        case 20: return pick_rollout_mode<ARM, 20>(mode, wobs, f16);
-        default: return pick_rollout_mode<ARM, 0>(mode, wobs, f16);
+        case 10: return pick_rollout_mode<ARM, 10>(mode, wobs, f16, final);
+        case 20: return pick_rollout_mode<ARM, 20>(mode, wobs, f16, final);
+        default: return pick_rollout_mode<ARM, 0>(mode, wobs, f16, final);
     }
 }
 
-static StepFn pick_rollout(int arm, int x, RolloutMode mode, bool wobs, bool f16) {
+static StepFn pick_rollout(int arm, int x, RolloutMode mode, bool wobs, bool f16, bool final) {
     switch (arm) {
-        case 0: return pick_rollout_x<0>(x, mode, wobs, f16);
-#define MT_PICK(ID) case ID: return pick_rollout_x<ID>(x, mode, wobs, f16);
+        case 0: return pick_rollout_x<0>(x, mode, wobs, f16, final);
+#define MT_PICK(ID) case ID: return pick_rollout_x<ID>(x, mode, wobs, f16, final);
         MT_FOR_EACH_PRESET_ARM(MT_PICK)
 #undef MT_PICK
     }
     return nullptr;
 }
 
-// n_steps (<= 4096) steps of `mode` in one launch.  The trajectory modes take the bases of slice 0 (mt_rollout).
+// n_steps (<= 4096) steps of `mode` in one launch.  The trajectory modes take the bases of slice 0 (mt_rollout);
+// final_obs != nullptr selects the FINAL = true kernel (mt_rollout_final), which also writes the final slices.
 static int launch_rollout(mt_env *e, RolloutMode mode, int n_steps, const float *actions, float *drawn, void *obs,
-                          float *reward, uint8_t *done, cudaStream_t st, bool &launched) {
+                          float *reward, uint8_t *done, cudaStream_t st, bool &launched, void *final_obs = nullptr,
+                          float *final_return = nullptr, int32_t *final_length = nullptr) {
     launched = false;
     if (n_steps < 2) return MT_OK;
     if (const char *v = std::getenv("MT_ROLLOUT_PERSISTENT"))
         if (v[0] == '0') return MT_OK;
+    const bool final = final_obs != nullptr;
     const void *fn = nullptr;
     if (e->jit) {                                             // this handle's own table: compiled on first use
         if (e->jit_rollout_failed) return MT_OK;
-        cudaKernel_t &k = e->jit_rollout[(int)mode][obs ? 1 : 0];
+        cudaKernel_t &k = e->jit_rollout[(int)mode][obs ? 1 : 0][final ? 1 : 0];
         if (!k) {
             std::string err;
-            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, true, obs != nullptr, e->f16, false, err, (int)mode).kernel;
+            k = jit_step_kernel(e->jit_preset, e->jit_id, e->jit_x, true, obs != nullptr, e->f16, final, err, (int)mode).kernel;
             if (!k) {
                 e->jit_rollout_failed = true;                 // keep working through the per-step launches
                 return MT_OK;
@@ -911,7 +921,7 @@ static int launch_rollout(mt_env *e, RolloutMode mode, int n_steps, const float 
         }
         fn = (const void *)k;
     } else {
-        fn = (const void *)pick_rollout(e->arm, e->cfg.n_obj, mode, obs != nullptr, e->f16);
+        fn = (const void *)pick_rollout(e->arm, e->cfg.n_obj, mode, obs != nullptr, e->f16, final);
     }
     if (!fn) return MT_OK;
     StepParams P = e->base;
@@ -929,6 +939,9 @@ static int launch_rollout(mt_env *e, RolloutMode mode, int n_steps, const float 
     P.advance = n_steps;
     P.n_steps = n_steps;
     P.launch_envs = e->n * (long long)n_steps;
+    P.final_obs = final_obs;
+    P.final_return = final_return;
+    P.final_length = final_length;
     const size_t nb = obs ? 2 : 1;                            // objectives (+ observations) per warp, one barrier
     P.trig_span = mode == RolloutMode::kActionsTrajectory ? 0 : trig_table_entries(e);   // the caller's actions: any float
     LaunchShape shape;
@@ -1080,13 +1093,22 @@ extern "C" int mt_rollout_random(mt_env *e, int32_t n_steps, void *obs_dev, floa
 
 // One step of mt_rollout through the step kernel, into the slice pointers of that step.  step_kernel bulk-stores
 // every full observation tile, so a slice whose base may not take a bulk copy (obs_bulk_ok false) gets the step's
-// observations through the handle's own buffer and one device-to-device copy.
+// observations through the handle's own buffer and one device-to-device copy.  The final observations
+// (mt_rollout_final) are stored lane by lane and go to their slice directly.  step_kernel<.., FINAL = true> exists
+// for the caller's actions only, so in-kernel draws are drawn first, as mt_sample_actions draws them at this step
+// index, and stepped as the caller's actions: bit for bit the same step, as the ActionTrig table is bit for bit the
+// kernel's own sin / cos evaluation (fill_action_trig).
 static int rollout_one_step(mt_env *e, const float *actions, float *drawn, void *obs, bool obs_bulk_ok, float *reward,
-                            uint8_t *done, cudaStream_t st) {
+                            uint8_t *done, cudaStream_t st, void *final_obs, float *final_return, int32_t *final_length) {
+    if (!actions && final_obs && !drawn) {
+        if (!e->scratch_actions) CU(cudaMalloc((void **)&e->scratch_actions, (size_t)e->n * e->cfg.n_joints * 4));
+        drawn = e->scratch_actions;
+    }
     if (!actions && drawn) {                          // what mt_sample_actions returns at this step index
         sample_actions_kernel<<<blocks_for(e->n), 256, 0, st>>>(e->base, drawn);
         CU(cudaGetLastError());
         e->launches++;
+        if (final_obs) actions = drawn;
     }
     const size_t obs_bytes = (size_t)e->n * 3 * e->cfg.n_obj * (e->f16 ? 2 : 4);
     void *dst = obs;
@@ -1094,9 +1116,43 @@ static int rollout_one_step(mt_env *e, const float *actions, float *drawn, void 
         if (!e->scratch_obs) CU(cudaMalloc(&e->scratch_obs, obs_bytes));
         dst = e->scratch_obs;
     }
-    if (int rc = launch_step(e, actions, dst, reward, done, nullptr, actions == nullptr, 0, e->n_tiles, st)) return rc;
+    if (int rc = launch_step(e, actions, dst, reward, done, nullptr, actions == nullptr, 0, e->n_tiles, st, 0, true,
+                             final_obs, final_return, final_length))
+        return rc;
     if (dst != obs) CU(cudaMemcpyAsync(obs, dst, obs_bytes, cudaMemcpyDeviceToDevice, st));
     return MT_OK;
+}
+
+// The chunk loop of mt_rollout and mt_rollout_final (that of mt_rollout_random, with slices): every pointer below is
+// the base of slice s (64-bit offsets).  final_obs = nullptr: mt_rollout.
+static int rollout_trajectory(mt_env *e, int32_t n_steps, const float *actions_dev, float *drawn_dev, void *obs_dev,
+                              float *reward_dev, uint8_t *done_dev, void *final_obs_dev, float *final_return_dev,
+                              int32_t *final_length_dev, cudaStream_t st) {
+    const RolloutMode mode = actions_dev ? RolloutMode::kActionsTrajectory : RolloutMode::kDrawTrajectory;
+    const size_t n = (size_t)e->n, J = (size_t)e->cfg.n_joints, obs_row = (size_t)3 * e->cfg.n_obj * (e->f16 ? 2 : 4);
+    int rc;
+    if ((rc = timing_begin(e, st))) return rc;
+    for (int s = 0; s < n_steps;) {
+        const int chunk = n_steps - s < 4096 ? n_steps - s : 4096;
+        const size_t rows = (size_t)s * n;
+        const float *a = actions_dev ? actions_dev + rows * J : nullptr;
+        float *d = drawn_dev ? drawn_dev + rows * J : nullptr;
+        void *o = obs_dev ? (void *)((char *)obs_dev + rows * obs_row) : nullptr;
+        void *fo = final_obs_dev ? (void *)((char *)final_obs_dev + rows * obs_row) : nullptr;
+        float *fr = final_obs_dev ? final_return_dev + rows : nullptr;
+        int32_t *fl = final_obs_dev ? final_length_dev + rows : nullptr;
+        bool launched = false;
+        if ((rc = launch_rollout(e, mode, chunk, a, d, o, reward_dev + rows, done_dev + rows, st, launched, fo, fr, fl)))
+            return rc;
+        if (launched) {
+            s += chunk;
+        } else {
+            const bool bulk_ok = slice_bulk_ok((uintptr_t)obs_dev, (unsigned long long)s, n, 0, obs_row);
+            if ((rc = rollout_one_step(e, a, d, o, bulk_ok, reward_dev + rows, done_dev + rows, st, fo, fr, fl))) return rc;
+            ++s;
+        }
+    }
+    return timing_end(e, st);
 }
 
 extern "C" int mt_rollout(mt_env *e, int32_t n_steps, const float *actions_dev, float *drawn_dev, void *obs_dev,
@@ -1114,28 +1170,34 @@ extern "C" int mt_rollout(mt_env *e, int32_t n_steps, const float *actions_dev, 
     if (!e->was_reset) return fail(MT_ERR_STATE, "mt_rollout before mt_reset");
     if (n_steps == 0) return MT_OK;
     DeviceGuard guard(e->cfg.device);
-    cudaStream_t st = (cudaStream_t)stream;
-    const RolloutMode mode = actions_dev ? RolloutMode::kActionsTrajectory : RolloutMode::kDrawTrajectory;
-    const size_t n = (size_t)e->n, J = (size_t)e->cfg.n_joints, obs_row = (size_t)3 * e->cfg.n_obj * (e->f16 ? 2 : 4);
-    if ((rc = timing_begin(e, st))) return rc;
-    // the chunk loop of mt_rollout_random; every pointer below is the base of slice s (64-bit offsets)
-    for (int s = 0; s < n_steps;) {
-        const int chunk = n_steps - s < 4096 ? n_steps - s : 4096;
-        const size_t rows = (size_t)s * n;
-        const float *a = actions_dev ? actions_dev + rows * J : nullptr;
-        float *d = drawn_dev ? drawn_dev + rows * J : nullptr;
-        void *o = obs_dev ? (void *)((char *)obs_dev + rows * obs_row) : nullptr;
-        bool launched = false;
-        if ((rc = launch_rollout(e, mode, chunk, a, d, o, reward_dev + rows, done_dev + rows, st, launched))) return rc;
-        if (launched) {
-            s += chunk;
-        } else {
-            const bool bulk_ok = slice_bulk_ok((uintptr_t)obs_dev, (unsigned long long)s, n, 0, obs_row);
-            if ((rc = rollout_one_step(e, a, d, o, bulk_ok, reward_dev + rows, done_dev + rows, st))) return rc;
-            ++s;
-        }
-    }
-    return timing_end(e, st);
+    return rollout_trajectory(e, n_steps, actions_dev, drawn_dev, obs_dev, reward_dev, done_dev, nullptr, nullptr, nullptr,
+                              (cudaStream_t)stream);
+}
+
+extern "C" int mt_rollout_final(mt_env *e, int32_t n_steps, const float *actions_dev, float *drawn_dev, void *obs_dev,
+                                float *reward_dev, uint8_t *done_dev, void *final_obs_dev, float *final_return_dev,
+                                int32_t *final_length_dev, void *stream) {
+    // the arguments first, in mt_rollout's order and then mt_step_final's: none of these checks needs the handle
+    if (n_steps < 0) return fail(MT_ERR_INVALID, "n_steps < 0");
+    int rc;
+    if ((rc = check_ptr(actions_dev, "actions_dev", false))) return rc;
+    if ((rc = check_ptr(drawn_dev, "drawn_dev", false))) return rc;
+    if (actions_dev && drawn_dev) return fail(MT_ERR_INVALID, "drawn_dev must be NULL when actions_dev is given");
+    if ((rc = check_ptr(obs_dev, "obs_dev", true))) return rc;
+    if ((rc = check_ptr(reward_dev, "reward_dev", true))) return rc;
+    if ((rc = check_ptr(done_dev, "done_dev", true))) return rc;
+    if ((rc = check_ptr(final_obs_dev, "final_obs_dev", true))) return rc;
+    if ((rc = check_ptr(final_return_dev, "final_return_dev", true))) return rc;
+    if ((rc = check_ptr(final_length_dev, "final_length_dev", true))) return rc;
+    if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    if (!e->cfg.auto_reset)
+        return fail(MT_ERR_INVALID, "mt_rollout_final needs a handle created with auto_reset (without it obs2 is the "
+                                    "returned observation and mt_get_state holds the return and length)");
+    if (!e->was_reset) return fail(MT_ERR_STATE, "mt_rollout_final before mt_reset");
+    if (n_steps == 0) return MT_OK;
+    DeviceGuard guard(e->cfg.device);
+    return rollout_trajectory(e, n_steps, actions_dev, drawn_dev, obs_dev, reward_dev, done_dev, final_obs_dev,
+                              final_return_dev, final_length_dev, (cudaStream_t)stream);
 }
 
 extern "C" int mt_host_alloc(void **out, uint64_t bytes) {

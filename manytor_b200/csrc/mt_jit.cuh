@@ -93,9 +93,9 @@ static std::string preset_source(int id, int J, const JointConst *rows) {
 
 // Compile (or fetch from the per-process cache) step_kernel<id, x_template, rnd, wobs, f16, final> for the table
 // described by `preset`.  Returns an empty JitKernel and fills `err` on failure.
-// `rollout_mode` >= 0 selects the multi-step rollout_kernel<id, x_template, wobs, f16, RolloutMode(rollout_mode)>
-// (`rnd` and `final` are ignored).  The cache key holds the template arguments, so handles with the same table and
-// different observation formats, final outputs or rollout modes get different kernels.
+// `rollout_mode` >= 0 selects the multi-step rollout_kernel<id, x_template, wobs, f16, RolloutMode(rollout_mode), final>
+// (`rnd` is ignored).  The cache key holds the template arguments, so handles with the same table and different
+// observation formats, final outputs or rollout modes get different kernels.
 static JitKernel jit_step_kernel(const std::string &preset, int id, int x_template, bool rnd, bool wobs, bool f16,
                                  bool final, std::string &err, int rollout_mode = -1) {
     static std::mutex mu;
@@ -104,9 +104,9 @@ static JitKernel jit_step_kernel(const std::string &preset, int id, int x_templa
                                          "mt::RolloutMode::kActionsTrajectory"};
     const bool rollout = rollout_mode >= 0;
     const char *obs = wobs ? (f16 ? "true, true" : "true, false") : "false, false";
-    const std::string targs = rollout ? std::to_string(id) + ", " + std::to_string(x_template) + ", " + obs + ", " + kModes[rollout_mode]
-                                      : std::to_string(id) + ", " + std::to_string(x_template) + ", " + (rnd ? "true" : "false") +
-                                            ", " + obs + (final ? ", true" : ", false");
+    const std::string targs = (rollout ? std::to_string(id) + ", " + std::to_string(x_template) + ", " + obs + ", " + kModes[rollout_mode]
+                                       : std::to_string(id) + ", " + std::to_string(x_template) + ", " + (rnd ? "true" : "false") +
+                                             ", " + obs) + (final ? ", true" : ", false");
     const std::string kname = rollout ? "rollout_kernel" : "step_kernel";
     const std::string inst = "mt::" + kname + "<" + targs + ">";
     const std::string key = preset + inst;

@@ -109,8 +109,9 @@ struct StepParams {
     // whole state fits its budget, evict_first beyond (mt_create; measured both ways in round 2).
     unsigned long long pol_state, pol_stream, pol_store;   // pol_store: the streamed OUTPUTS (observations, reward, done)
     float *drawn;              // rollout_kernel<.., RolloutMode::kDrawTrajectory>: [n_steps][N][J] drawn actions, or nullptr
-    // step_kernel<.., FINAL = true> (mt_step_final): what an ending env's episode leaves behind, written for the rows
-    // of the envs that end in this step only (settle_step)
+    // step_kernel<.., FINAL = true> (mt_step_final) and rollout_kernel<.., FINAL = true> (mt_rollout_final): what an
+    // ending env's episode leaves behind, written for the rows of the envs that end in this step only (settle_step);
+    // the rollout kernel writes step s into slice s of [n_steps][N] arrays, as it does its other outputs
     void *final_obs;           // [N][3X] obs2 of the ending step, in the handle's obs format
     float *final_return;       // [N] total reward of the episode
     int32_t *final_length;     // [N] episode length (the saturating counter)
@@ -826,18 +827,19 @@ __device__ __forceinline__ void store_action_row(float *row, const float *a, uin
 // Resets are rare (one env-step in ~550 for random actions), so the warp handles its ending envs one at a
 // time and COOPERATIVELY: lane p draws objective p (x <= 32 lanes busy) instead of the one ending lane
 // drawing all x while 31 lanes idle.
-// FINAL (mt_step_final, needs WOBS): before the reset wipes them, an ending env's return and length go to
-// P.final_return / P.final_length, and its obs2 row -- still fp32 at obs_buf, in the public order -- to
+// FINAL (mt_step_final, mt_rollout_final; needs WOBS): before the reset wipes them, an ending env's return and
+// length go to P.final_return / P.final_length, and its obs2 row -- still fp32 at obs_buf, in the public order -- to
 // P.final_obs (binary16 when F16, rounded as pack_tile_f16 rounds), lane p copying objective p's three words
 // ahead of the first observation of the new episode that replaces them.  Rows of envs that go on are not
-// touched.
+// touched.  srow: the first row of the final arrays' slice (0 for step_kernel, s N for step s of a trajectory),
+// so env `env` of the slice is row srow + env; the offsets are 64-bit (a slice passes 4 GiB at sizes users run).
 // ---------------------------------------------------------------------------
 template <int J, bool WOBS, bool FINAL = false, bool F16 = false>
 __device__ __forceinline__ void settle_step(const StepParams &P, int lane, int env0, bool valid, int x, int rowlen, bool neg,
                                             uint32_t alive0, uint32_t caught, const float *a, float *gn, float &total,
                                             uint32_t &alive1, uint32_t &eplen, float &rew, uint8_t &done,
                                             uint32_t &ground_steps, unsigned long long *blk_stat, uint32_t obs_buf,
-                                            uint32_t pts_buf) {
+                                            uint32_t pts_buf, size_t srow) {
     static_assert(WOBS || !FINAL, "the final observation is the tile's obs2");
     alive1 = alive0 & ~caught;                                             // manytor.py:168
     rew = (alive1 != alive0) ? 1.0f : 0.0f;
@@ -867,7 +869,7 @@ __device__ __forceinline__ void settle_step(const StepParams &P, int lane, int e
             atomicAdd(&blk_stat[4], (unsigned long long)c_sum);
         }
         if (FINAL && ending) {
-            const size_t env = (size_t)(env0 + lane);
+            const size_t env = srow + (size_t)(env0 + lane);
             P.final_return[env] = total;
             P.final_length[env] = (int32_t)eplen;
         }
@@ -889,7 +891,7 @@ __device__ __forceinline__ void settle_step(const StepParams &P, int lane, int e
         if (lane < x) {
             if (FINAL) {
                 const uint32_t orow = obs_buf + (uint32_t)(src * rowlen + lane * 3) * 4u;
-                const size_t i = renv * (size_t)rowlen + (size_t)(lane * 3);
+                const size_t i = (srow + renv) * (size_t)rowlen + (size_t)(lane * 3);
                 store_obs<F16>(P.final_obs, i, lds_f(orow));
                 store_obs<F16>(P.final_obs, i + 1, lds_f(orow + 4));
                 store_obs<F16>(P.final_obs, i + 2, lds_f(orow + 8));
@@ -1161,7 +1163,7 @@ step_kernel(const __grid_constant__ StepParams P) {
             uint8_t done;
             if (ep_shift) eplen = word >> ep_shift;
             settle_step<J, WOBS, FINAL, F16>(P, lane, env0, valid, x, rowlen, neg, alive0, caught, sc.a, gn, total, alive1, eplen,
-                                             rew, done, ground_steps, blk_stat, buf_cur, 0u);
+                                             rew, done, ground_steps, blk_stat, buf_cur, 0u, 0);
 
             // 7. write back: state (coalesced), then the observation tile by one bulk store
             if (J == 4) {
@@ -1252,6 +1254,8 @@ step_kernel(const __grid_constant__ StepParams P) {
 // [n_steps][N][J] array instead of drawing them, evaluating their sin / cos exactly as step_kernel<.., RAND = false, ..>
 // does (arbitrary floats: no ActionTrig table), with an L2 prefetch of the next step's action tile that costs no
 // register and no shared memory.
+// FINAL (mt_rollout_final, trajectory modes with WOBS only): settle_step also writes each ending env's obs2, return
+// and length into slice s of P.final_* -- what mt_step_final writes at the s-th step.
 // ---------------------------------------------------------------------------
 enum class RolloutMode : int {
     kDrawLast = 0,             // in-kernel actions, outputs of the last step (mt_rollout_random)
@@ -1259,11 +1263,12 @@ enum class RolloutMode : int {
     kActionsTrajectory = 2,    // the caller's actions, outputs of every step (mt_rollout)
 };
 
-template <int ARM, int X, bool WOBS, bool F16, RolloutMode MODE>
+template <int ARM, int X, bool WOBS, bool F16, RolloutMode MODE, bool FINAL = false>
 __global__ void __launch_bounds__(((ARM == 0) ? kMaxWarpsRefArm : kMaxWarpsGeneric) * kTile, 1)
 rollout_kernel(const __grid_constant__ StepParams P) {
     static_assert(WOBS || !F16, "F16 is an observation format");
     constexpr bool TRAJ = MODE != RolloutMode::kDrawLast;
+    static_assert(!FINAL || TRAJ, "final outputs come in slices: trajectory modes only");
     constexpr bool DRAW = MODE != RolloutMode::kActionsTrajectory;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ int queue_next;
@@ -1351,8 +1356,11 @@ rollout_kernel(const __grid_constant__ StepParams P) {
                 const uint32_t caught = walk_row<X, WOBS>(row, orow, x, f, P.catch_tol, alive);
                 float gn[J];
                 uint32_t alive1;
-                settle_step<J, WOBS>(P, lane, env0, valid, x, rowlen, neg, alive, caught, sc.a, gn, total, alive1, eplen, rew, done,
-                                     ground_steps, blk_stat, obuf, pts);
+                // FINAL: obuf holds this step's obs2 here -- the wait above ordered the previous step's bulk store (which
+                // may have packed the buffer to binary16) before walk_row refilled it -- so the final observation is copied
+                // out before a reset writes the new episode's first observation over it, as in step_kernel
+                settle_step<J, WOBS, FINAL, F16>(P, lane, env0, valid, x, rowlen, neg, alive, caught, sc.a, gn, total, alive1, eplen,
+                                                 rew, done, ground_steps, blk_stat, obuf, pts, srow);
                 alive = alive1;
 #pragma unroll
                 for (int i = 0; i < J; ++i) sc.g[i] = gn[i];
