@@ -133,7 +133,9 @@ int mt_set_seed(mt_env *env, uint64_t seed);
  * mt_step_host and of each step of mt_rollout_random), as are mt_stats.env_steps and the other
  * statistics.  Consequence for CUDA graphs: a captured mt_step / mt_rollout_random can be replayed
  * any number of times -- every replay counts its env-steps and draws fresh actions, exactly like the
- * same calls issued eagerly.  Get/set are synchronous 8-byte copies (checkpoint / resume).
+ * same calls issued eagerly.  Get/set are synchronous 8-byte copies on the legacy default stream
+ * (checkpoint / resume), ordered after everything submitted earlier to it / blocking streams (work on
+ * cudaStreamNonBlocking streams must be synchronised by the caller); the set has landed on return.
  * The index lies in [0, MT_STEP_INDEX_MAX]; mt_set_step_index returns MT_ERR_INVALID above it and leaves
  * the index as it was.  The bound exists because the kernels' launch bookkeeping needs bit 63 of the index
  * to be clear: each warp orders its launch ticket after its read of the index through that bit.  At most
@@ -268,12 +270,16 @@ int mt_set_objective_stream(mt_env *env, const float *points_dev, int32_t n_sets
 
 /* One-env copy-back for the render shim and per-env attribute reads (manytor.py:131-139,
  * 196-201).  Synchronous, on the legacy default stream: one small kernel + one copy through
- * scratch buffers the handle owns (no allocation, no device-wide synchronisation). */
+ * scratch buffers the handle owns (no allocation, no device-wide synchronisation).  Ordered after
+ * everything submitted earlier to the legacy default stream / blocking streams (work on
+ * cudaStreamNonBlocking streams must be synchronised by the caller). */
 int mt_fetch_env(mt_env *env, int64_t index, float *goals_host, float *joints_host,
                  float *points_host, uint32_t *alive_host, float *total_reward_host);
 
 /* Episode statistics.  mt_stats_device writes MT_STATS_WORDS int64 to a device
- * buffer (for an NCCL all-reduce); mt_stats_host is the synchronous host read. */
+ * buffer (for an NCCL all-reduce); mt_stats_host is the synchronous host read, on the legacy default
+ * stream: ordered after everything submitted earlier to it / blocking streams (work on
+ * cudaStreamNonBlocking streams must be synchronised by the caller). */
 int mt_stats_device(mt_env *env, int64_t *stats_dev, void *stream);
 int mt_stats_host(mt_env *env, mt_stats *out);
 int mt_stats_clear(mt_env *env, void *stream);

@@ -164,6 +164,8 @@ class BatchedEnvs:
     observations are the float32 ones rounded to nearest even, written by the kernels themselves
     (half the bytes to HBM and across PCIe)."""
 
+    _side = None                                           # non-default stream of the last enqueued call (_stream)
+
     def __init__(self, n_envs: int, obj_number: int = 10, arm: ArmSpec = REFERENCE_ARM, device=None,
                  env_id_base: int = 0, horizon: int = 0, auto_reset: bool = False,
                  terminate_on_ground: bool = False, obs_after_reset: bool = False, seed: int = 0,
@@ -200,7 +202,23 @@ class BatchedEnvs:
             pass
 
     def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        """The current stream, for an asynchronous call.  A non-default stream is remembered (not while a CUDA
+        graph is being captured: a capture enqueues nothing) so that the synchronous calls can wait for it."""
+        s = torch.cuda.current_stream(self.device)
+        if not s.cuda_stream:
+            self._side = None
+        elif not torch.cuda.is_current_stream_capturing():
+            self._side = s
+        return C.c_void_p(s.cuda_stream)
+
+    def _after_side_stream(self):
+        """Before a call that runs on the legacy default stream or on the handle's own streams (stats, step_index,
+        fetch_env, step_host): wait for this handle's work on a non-default stream.  The legacy stream does not
+        wait for PyTorch's streams (they are non-blocking), so without this such a call could run before the work
+        it is meant to see.  Work on the default stream is already ordered: nothing to do there."""
+        if self._side is not None and not torch.cuda.is_current_stream_capturing():
+            self._side.synchronize()
+            self._side = None
 
     def _empty(self, shape, dtype):
         return torch.empty(shape, dtype=dtype, device=self.device)
@@ -428,6 +446,7 @@ class BatchedEnvs:
         if own is None:
             np.copyto(act, np.asarray(actions_host, dtype=np.float32).reshape(self.n, self.j))
             own = act_ptr
+        self._after_side_stream()
         _lib.check(self._lib.mt_step_host(self._h, own, obs_ptr, rew_ptr, done_ptr))
         return obs, rew, done
 
@@ -506,6 +525,7 @@ class BatchedEnvs:
         points = np.zeros((self.x, 3), dtype=np.float32)
         alive = C.c_uint32()
         total = C.c_float()
+        self._after_side_stream()
         _lib.check(self._lib.mt_fetch_env(self._h, int(index), goals.ctypes.data, joints.ctypes.data,
                                           points.ctypes.data, C.byref(alive), C.byref(total)))
         alives = np.array([(alive.value >> p) & 1 for p in range(self.x)], dtype=bool)
@@ -524,6 +544,7 @@ class BatchedEnvs:
         """Steps executed so far; keys the action stream.  Lives on the device (advanced by the step
         kernel, so CUDA-graph replays count); reading it synchronises."""
         v = C.c_uint64()
+        self._after_side_stream()
         _lib.check(self._lib.mt_get_step_index(self._h, C.byref(v)))
         return int(v.value)
 
@@ -533,6 +554,7 @@ class BatchedEnvs:
         value = int(value)
         if not 0 <= value <= _lib.MT_STEP_INDEX_MAX:
             raise ValueError(f"step_index must be in [0, 2**62], not {value}")
+        self._after_side_stream()
         _lib.check(self._lib.mt_set_step_index(self._h, value))
 
     # -- statistics ---------------------------------------------------------------
@@ -544,6 +566,7 @@ class BatchedEnvs:
 
     def stats(self) -> dict:
         s = MtStats()
+        self._after_side_stream()
         _lib.check(self._lib.mt_stats_host(self._h, C.byref(s)))
         return {k: int(getattr(s, k)) for k in STATS_FIELDS}
 

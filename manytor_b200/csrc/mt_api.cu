@@ -445,7 +445,9 @@ extern "C" int mt_set_seed(mt_env *e, uint64_t seed) {
 }
 
 // The step index that keys the action stream (mt_sample_actions / mt_rollout_random): part of a
-// checkpoint next to mt_get_state.  Synchronous (one 8-byte copy on the legacy default stream).
+// checkpoint next to mt_get_state.  Synchronous (one 8-byte copy on the legacy default stream; the set waits for
+// its copy to land, which a copy from pageable memory does not promise on return, so that a launch on any stream
+// issued after it reads the new index).
 extern "C" int mt_get_step_index(mt_env *e, uint64_t *out) {
     if (!e || !out) return fail(MT_ERR_INVALID, "NULL argument");
     DeviceGuard guard(e->cfg.device);
@@ -462,6 +464,7 @@ extern "C" int mt_set_step_index(mt_env *e, uint64_t value) {
     DeviceGuard guard(e->cfg.device);
     const unsigned long long v = value;
     CU(cudaMemcpy(e->ctrl + kCtrlStep, &v, 8, cudaMemcpyHostToDevice));
+    CU(cudaStreamSynchronize(nullptr));
     return MT_OK;
 }
 
