@@ -123,9 +123,9 @@ int mt_create(const mt_config *cfg, mt_env **out);
 int mt_destroy(mt_env *env);
 int mt_get_config(const mt_env *env, mt_config *out);
 /* Re-seed the on-device Philox streams (actions, objective refresh): new key AND the counters that
- * index the streams (per-env episode count, step index) back to zero, so reset(seed=s) reproduces the
- * same objectives and actions every time it is called with the same s (Gymnasium's reset(seed=...)
- * contract).  Synchronous (waits for the device). */
+ * index the streams (per-env reset count of mt_get_reset_counts, step index) back to zero, so
+ * reset(seed=s) reproduces the same objectives and actions every time it is called with the same s
+ * (Gymnasium's reset(seed=...) contract).  Synchronous (waits for the device). */
 int mt_set_seed(mt_env *env, uint64_t seed);
 
 /* The step index that keys the action stream of mt_sample_actions / mt_rollout_random.  It lives in
@@ -134,8 +134,9 @@ int mt_set_seed(mt_env *env, uint64_t seed);
  * statistics.  Consequence for CUDA graphs: a captured mt_step / mt_rollout_random can be replayed
  * any number of times -- every replay counts its env-steps and draws fresh actions, exactly like the
  * same calls issued eagerly.  Get/set are synchronous 8-byte copies on the legacy default stream
- * (checkpoint / resume), ordered after everything submitted earlier to it / blocking streams (work on
- * cudaStreamNonBlocking streams must be synchronised by the caller); the set has landed on return.
+ * (checkpoint / resume, with the state listed at mt_set_points), ordered after everything submitted
+ * earlier to it / blocking streams (work on cudaStreamNonBlocking streams must be synchronised by the
+ * caller); the set has landed on return.
  * The index lies in [0, MT_STEP_INDEX_MAX]; mt_set_step_index returns MT_ERR_INVALID above it and leaves
  * the index as it was.  The bound exists because the kernels' launch bookkeeping needs bit 63 of the index
  * to be clear: each warp orders its launch ticket after its read of the index through that bit.  At most
@@ -255,7 +256,13 @@ int mt_host_alloc(void **out, uint64_t bytes);
 int mt_host_free(void *p);
 
 /* State exchange (parity upload of reference objectives, checkpoint, render copy-back).
- * Any pointer may be NULL to skip that array; mask_dev as in mt_reset. */
+ * Any pointer may be NULL to skip that array; mask_dev as in mt_reset.
+ * A checkpoint from which a new handle continues bit for bit holds: the config (mt_get_config: the seed may
+ * have been changed by mt_set_seed), goals / alive / total_reward / ep_len (mt_get_state), the reset counts
+ * (mt_get_reset_counts), the raw objectives (mt_get_points with zero_dead = 0) and the step index
+ * (mt_get_step_index).  To restore, create a handle with that config, mt_reset it, then set all of them
+ * (and the same objective stream, if one was set).  Statistics restart at zero in the new handle: a caller
+ * who wants running totals adds the checkpoint's statistics. */
 int mt_set_points(mt_env *env, const float *points_dev, const uint8_t *mask_dev, void *stream);
 int mt_get_points(mt_env *env, float *points_dev, int32_t zero_dead, void *stream);
 int mt_set_state(mt_env *env, const float *goals_dev, const uint32_t *alive_dev,
@@ -263,6 +270,14 @@ int mt_set_state(mt_env *env, const float *goals_dev, const uint32_t *alive_dev,
                  const uint8_t *mask_dev, void *stream);
 int mt_get_state(mt_env *env, float *goals_dev, uint32_t *alive_dev, float *total_reward_dev,
                  int32_t *ep_len_dev, void *stream);
+/* counts_dev [N] uint32: the resets each env has had so far (mt_reset and the in-kernel auto-reset each add
+ * one).  The count keys the on-device objective sampler -- the e-th reset of an env draws with Philox counter
+ * e*32 + objective, mod 2^32, so the sampler repeats after 2^27 episodes of one env -- and selects the set
+ * e mod n_sets of an objective stream.  Counts wrap mod 2^32.  mt_set_seed zeroes them.  mask_dev as in
+ * mt_reset; counts_dev is required.  A restore sets them AFTER the new handle's first mt_reset, because
+ * mt_reset advances the counts of the envs it resets. */
+int mt_get_reset_counts(mt_env *env, uint32_t *counts_dev, void *stream);
+int mt_set_reset_counts(mt_env *env, const uint32_t *counts_dev, const uint8_t *mask_dev, void *stream);
 
 /* Objective refresh stream for parity runs: points_dev [n_sets][N][X][3], borrowed.
  * The e-th reset of env n takes set (e mod n_sets).  NULL/0 restores the sampler. */

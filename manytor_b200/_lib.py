@@ -86,6 +86,8 @@ SIGNATURES = {
     "mt_get_points": (C.c_int, [_P, _P, C.c_int32, _P]),
     "mt_set_state": (C.c_int, [_P, _P, _P, _P, _P, _P, _P]),
     "mt_get_state": (C.c_int, [_P, _P, _P, _P, _P, _P]),
+    "mt_get_reset_counts": (C.c_int, [_P, _P, _P]),
+    "mt_set_reset_counts": (C.c_int, [_P, _P, _P, _P]),
     "mt_set_objective_stream": (C.c_int, [_P, _P, C.c_int32]),
     "mt_fetch_env": (C.c_int, [_P, C.c_int64, _P, _P, _P, _P, _P]),
     "mt_stats_device": (C.c_int, [_P, _P, _P]),

@@ -466,13 +466,21 @@ class BatchedEnvs:
         _lib.check(self._lib.mt_get_points(self._h, self._p(out), int(zero_dead), self._stream()))
         return out
 
-    def set_state(self, goals=None, alive=None, total_reward=None, ep_len=None, mask=None):
+    def set_state(self, goals=None, alive=None, total_reward=None, ep_len=None, mask=None, resets=None):
+        """Overwrite parts of the state (None = keep).  `resets`: (N,) per-env reset counts, integers whose low 32 bits
+        are the uint32 count (the int32 `get_state()["resets"]` as it is).  Restoring a checkpoint: see get_state."""
+        if resets is not None and tuple(np.shape(resets)) != (self.n,):
+            raise ValueError(f"resets must have shape ({self.n},), not {tuple(np.shape(resets))}")
         g = self._as_dev(goals, torch.float32, (self.n, self.j)) if goals is not None else None
         al = self._alive_words(alive) if alive is not None else None
         tr = self._as_dev(total_reward, torch.float32, (self.n,)) if total_reward is not None else None
         el = self._as_dev(ep_len, torch.int32, (self.n,)) if ep_len is not None else None
+        m = self._mask(mask)
         _lib.check(self._lib.mt_set_state(self._h, self._p(g), self._p(al), self._p(tr), self._p(el),
-                                          self._p(self._mask(mask)), self._stream()))
+                                          self._p(m), self._stream()))
+        if resets is not None:
+            rc = self._u32_words(resets)
+            _lib.check(self._lib.mt_set_reset_counts(self._h, self._p(rc), self._p(m), self._stream()))
         torch.cuda.current_stream(self.device).synchronize()
 
     def _alive_words(self, alive) -> torch.Tensor:
@@ -481,17 +489,28 @@ class BatchedEnvs:
         if al.dim() == 2:
             w = (1 << torch.arange(self.x, dtype=torch.int64))
             al = (al.to(torch.int64) * w).sum(dim=1)
-        al = al.to(torch.int64) & 0xFFFFFFFF
-        al = torch.where(al >= 2 ** 31, al - 2 ** 32, al).to(torch.int32)
-        return al.to(self.device).contiguous().reshape(self.n)
+        return self._u32_words(al)
+
+    def _u32_words(self, words) -> torch.Tensor:
+        """(N,) integers -> (N,) int32 on the device holding their low 32 bits (the uint32 bit pattern)."""
+        w = torch.as_tensor(words).to(torch.int64) & 0xFFFFFFFF
+        w = torch.where(w >= 2 ** 31, w - 2 ** 32, w).to(torch.int32)
+        return w.to(self.device).contiguous().reshape(self.n)
 
     def get_state(self) -> dict:
+        """goals (N, J) f32, alive (N,) int32 holding the uint32 bitmask, total_reward (N,) f32, ep_len (N,) int32 and
+        resets (N,) int32 holding each env's uint32 reset count (it keys the objective sampler and picks the objective
+        stream's set).  With raw points (get_points(zero_dead=False)) and step_index this is what a handle created with
+        the same config (and objective stream) needs to continue bit for bit: reset() it, then set_state(**state),
+        set_points and step_index.  Statistics are not part of it: the new handle counts from zero."""
         g = self._empty((self.n, self.j), torch.float32)
         al = self._empty((self.n,), torch.int32)
         tr = self._empty((self.n,), torch.float32)
         el = self._empty((self.n,), torch.int32)
+        rc = self._empty((self.n,), torch.int32)
         _lib.check(self._lib.mt_get_state(self._h, self._p(g), self._p(al), self._p(tr), self._p(el), self._stream()))
-        return dict(goals=g, alive=al, total_reward=tr, ep_len=el)
+        _lib.check(self._lib.mt_get_reset_counts(self._h, self._p(rc), self._stream()))
+        return dict(goals=g, alive=al, total_reward=tr, ep_len=el, resets=rc)
 
     def alive_matrix(self) -> torch.Tensor:
         """(N, X) bool view of the alive bitmask (the reference's `alives`, manytor.py:134)."""

@@ -598,6 +598,20 @@ __global__ void get_state_kernel(const __grid_constant__ StepParams P, float *go
     if (eplen) eplen[env] = (int32_t)(P.ep_shift ? (w >> P.ep_shift) : P.counters[env]);
 }
 
+__global__ void set_reset_counts_kernel(const __grid_constant__ StepParams P, const uint32_t *counts,
+                                        const uint8_t *mask) {
+    const long long env = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (env >= P.n) return;
+    if (mask && !mask[env]) return;
+    P.episode[env] = counts[env];
+}
+
+__global__ void get_reset_counts_kernel(const __grid_constant__ StepParams P, uint32_t *counts) {
+    const long long env = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (env >= P.n) return;
+    counts[env] = P.episode[env];
+}
+
 __global__ void sample_actions_kernel(const __grid_constant__ StepParams P, float *actions) {
     const long long env = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (env >= P.n) return;
@@ -1347,6 +1361,28 @@ extern "C" int mt_get_state(mt_env *e, float *goals_dev, uint32_t *alive_dev, fl
     DeviceGuard guard(e->cfg.device);
     get_state_kernel<<<blocks_for(e->n), 256, 0, (cudaStream_t)stream>>>(e->base, goals_dev, alive_dev, total_reward_dev,
                                                                           ep_len_dev);
+    CU(cudaGetLastError());
+    e->launches++;
+    return MT_OK;
+}
+
+// The per-env reset counts (StepParams::episode): they key sample_point and pick the objective-stream set, so a
+// checkpoint needs them next to mt_get_state.
+extern "C" int mt_get_reset_counts(mt_env *e, uint32_t *counts_dev, void *stream) {
+    if (!counts_dev) return fail(MT_ERR_INVALID, "counts_dev is NULL");
+    if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    DeviceGuard guard(e->cfg.device);
+    get_reset_counts_kernel<<<blocks_for(e->n), 256, 0, (cudaStream_t)stream>>>(e->base, counts_dev);
+    CU(cudaGetLastError());
+    e->launches++;
+    return MT_OK;
+}
+
+extern "C" int mt_set_reset_counts(mt_env *e, const uint32_t *counts_dev, const uint8_t *mask_dev, void *stream) {
+    if (!counts_dev) return fail(MT_ERR_INVALID, "counts_dev is NULL");
+    if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    DeviceGuard guard(e->cfg.device);
+    set_reset_counts_kernel<<<blocks_for(e->n), 256, 0, (cudaStream_t)stream>>>(e->base, counts_dev, mask_dev);
     CU(cudaGetLastError());
     e->launches++;
     return MT_OK;
