@@ -240,6 +240,39 @@ int mt_rollout_final(mt_env *env, int32_t n_steps, const float *actions_dev, flo
                      float *reward_dev, uint8_t *done_dev, void *final_obs_dev, float *final_return_dev,
                      int32_t *final_length_dev, void *stream);
 
+/* Score action sequences from copies of chosen envs in one launch, leaving the handle untouched -- what an
+ * open-loop planner (random shooting, CEM, MPPI, MPC with a terminal value) asks many times per decision.
+ *   src_dev     [M] int64: branch m starts from the current state of env src[m]: its goals, alive word, episode
+ *                          length and raw objectives (dead ones included).  Sources may repeat, in any order; M may
+ *                          be smaller or larger than N.
+ *   actions_dev [n_steps][M][J] fp32 degrees: step s of branch m reads actions_dev + (s*M + m)*J (mt_rollout's layout)
+ * Every step is computed as mt_step computes it for an env in that state with those actions (reward, catches,
+ * ground test, terminate_on_ground, truncation at the handle's horizon counted from the source's episode length).
+ * A branch ends at the first step whose done byte is non-zero, that step included; nothing resets inside a branch.
+ * Outputs, one row per branch:
+ *   return_dev  [M] fp32: the discounted return up to and including the ending step, in this fp32 order:
+ *               d_0 = 1, d_{s+1} = fl(d_s * gamma), G_{s+1} = fl(G_s + d_s * r_s) (d_s * r_s is exact: r_s is -1, 0, +1)
+ *   length_dev  [M] i32: the steps the branch executed, T in [1, n_steps] when it ended at step T-1, else n_steps
+ *   done_dev    [M] u8: the done byte of the ending step (bit0 terminated, bit1 truncated), 0 if it ran all steps
+ *   obs_dev     [M][3X] in the handle's obs format, or NULL (not written): the observation mt_step returns at the
+ *               branch's last executed step with obs_after_reset = 0 (obs2; where the branch ended, what
+ *               mt_step_final writes as the final observation)
+ * A branch whose source is outside [0, N) reads nothing of any env: it gets return NaN, length -1, done 0, and its
+ * obs row is not written.  The handle is not changed: goals, alive words, episode lengths, total rewards, objectives,
+ * reset counts, step index and statistics stay as they were; auto_reset and the objective stream play no part.
+ * Only mt_launch_count moves.  Every pointer but obs_dev is required, and all are 16-byte aligned.  Argument errors
+ * are reported before the handle is looked at: n_steps outside [0, 4096], n_branches outside [0, 2e9] and gamma
+ * not in [0, 1] (NaN included) are MT_ERR_INVALID.  A call before the first mt_reset is MT_ERR_STATE; n_steps = 0
+ * or n_branches = 0 then does nothing.  ONE launch: a branch's state stays in registers and its objectives in shared
+ * memory for all the steps, so a branch-step moves its 4J bytes of actions plus (state + 12X + outputs) / n_steps.
+ * Every arm runs it: the built-in ones at X = 10, 20 and any X, and any other DH table through the run-time-table
+ * kernel.  For a handle whose steps NVRTC specialises to its table, branches are therefore bit for bit the step of the
+ * same table with fk_mode = 1; the specialised kernel folds the table's zeros and orders two multiply-adds differently,
+ * so positions, and with them observations, can differ in the last bits from that handle's own mt_step. */
+int mt_rollout_branches(mt_env *env, int32_t n_steps, int64_t n_branches, const int64_t *src_dev,
+                        const float *actions_dev, float gamma, float *return_dev, int32_t *length_dev,
+                        uint8_t *done_dev, void *obs_dev, void *stream);
+
 /* Host-buffer step: actions_host/obs_host/reward_host/done_host must be pinned
  * (mt_host_alloc).  Copies actions H2D, steps, copies results D2H, chunked over
  * internal streams so copies overlap the kernels; synchronous on return.  Ordered after

@@ -62,6 +62,11 @@ Trajectory = namedtuple("Trajectory", "obs reward done actions")
 # BatchedEnvs.rollout(final=True) returns one slice per step: (K, N, 3X), (K, N) and (K, N).
 FinalInfo = namedtuple("FinalInfo", "obs episode_return episode_length")
 
+# What BatchedEnvs.rollout_branches returns, one row per branch: the discounted return ((M,) float32), the steps executed
+# ((M,) int32), the done byte of the ending step ((M,) uint8, 0 if the branch ran every step) and obs2 of the last
+# executed step ((M, 3X) of the handle's obs_dtype, or None without write_obs).
+Branches = namedtuple("Branches", "ret length done obs")
+
 
 # observation dtype -> mt_config.obs_dtype
 OBS_DTYPES = {torch.float32: _lib.MT_OBS_F32, torch.float16: _lib.MT_OBS_F16}
@@ -416,6 +421,66 @@ class BatchedEnvs:
                                             self._p(bufs.done), self._stream()))
         self._rollout_io = (bufs, fin)                     # keep alive until the stream has consumed them
         return (bufs, fin) if final else bufs
+
+    def rollout_branches(self, actions, src=None, gamma: float = 1.0, write_obs: bool = False,
+                         out: Optional[Branches] = None) -> Branches:
+        """Score K-step action sequences from copies of chosen envs in one launch, leaving this handle untouched
+        (mt_rollout_branches): branch m starts from the current state of env src[m] and steps with actions[:, m] as
+        `step` would, until its first done step (included) or the K-th step.  No env is reset inside a branch, and the
+        state, objectives, reset counts, statistics and step index of the handle stay as they were.
+
+        actions: (K, M, J) degrees, converted like `rollout`'s input.  src: (M,) integers, the source env of each branch
+        (repeats and any order allowed); a tensor on this device is used as it is, without a host synchronisation.
+        None means arange(N), which needs M == N.  A source outside [0, N) gives that branch ret NaN, length -1, done 0
+        and leaves its obs row alone.  gamma in [0, 1]: ret is sum of gamma**s * r_s in fp32, d_0 = 1, d_{s+1} = d_s *
+        gamma, G += d_s * r_s.  write_obs: also return obs2 of each branch's last executed step.  `out`: a Branches of
+        preallocated buffers (obs None unless write_obs), e.g. fixed storage for a CUDA graph that captures this call.
+        Shape and dtype errors raise ValueError before the library is called."""
+        shape = tuple(actions.shape) if hasattr(actions, "shape") else tuple(np.shape(actions))
+        if len(shape) != 3 or shape[2] != self.j:
+            raise ValueError(f"actions must have shape (K, M, {self.j}), not {shape}")
+        k, m = shape[0], shape[1]
+        if k > 4096:
+            raise ValueError(f"rollout_branches takes at most 4096 steps, not {k}")
+        g = float(gamma)
+        if not 0.0 <= g <= 1.0:
+            raise ValueError(f"gamma must be finite and in [0, 1], not {gamma}")
+        if src is None:
+            if m != self.n:
+                raise ValueError(f"src=None branches every env once: actions need M = {self.n} branches, not {m}")
+        else:
+            src_shape = tuple(src.shape) if hasattr(src, "shape") else tuple(np.shape(src))
+            if src_shape != (m,):
+                raise ValueError(f"src must have shape ({m},) (one source per branch), not {src_shape}")
+            src_dtype = src.dtype if isinstance(src, torch.Tensor) else torch.as_tensor(np.asarray(src)).dtype
+            if src_dtype.is_floating_point or src_dtype.is_complex or src_dtype == torch.bool:
+                raise ValueError(f"src must hold integers, not {src_dtype}")
+        want = {"ret": ((m,), torch.float32), "length": ((m,), torch.int32), "done": ((m,), torch.uint8),
+                "obs": ((m, 3 * self.x), self.obs_dtype) if write_obs else None}
+        if out is not None:
+            self._check_out(out, Branches, "out", want, f"write_obs={write_obs}")
+            bufs = out
+        else:
+            bufs = Branches(*(self._empty(*spec) if spec is not None else None for spec in want.values()))
+        if k == 0 or m == 0:                               # nothing to do (and empty tensors have no address)
+            return bufs
+        if (isinstance(actions, torch.Tensor) and actions.is_cuda and actions.device == self.device
+                and actions.dtype == torch.float32 and actions.is_contiguous()):
+            a = actions                                    # fast path: already the device layout
+        else:
+            a = self._as_dev(actions, torch.float32, (k, m, self.j))
+        if src is None:
+            s = torch.arange(self.n, dtype=torch.int64, device=self.device)
+        elif (isinstance(src, torch.Tensor) and src.is_cuda and src.device == self.device and src.dtype == torch.int64
+                and src.is_contiguous()):
+            s = src
+        else:
+            s = self._as_dev(src, torch.int64, (m,))
+        _lib.check(self._lib.mt_rollout_branches(self._h, k, m, self._p(s), self._p(a), g, self._p(bufs.ret),
+                                                 self._p(bufs.length), self._p(bufs.done), self._p(bufs.obs),
+                                                 self._stream()))
+        self._branch_io = (a, s, bufs)                     # keep alive until the stream has consumed them
+        return bufs
 
     # -- host-buffer (end-to-end) step ------------------------------------------
     def pinned(self, name: str, shape, dtype) -> np.ndarray:

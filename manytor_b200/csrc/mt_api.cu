@@ -695,6 +695,7 @@ __global__ void r_theta_kernel(const float *v1, const float *v2, long long m, fl
 // step dispatch
 // ----------------------------------------------------------------------------
 typedef void (*StepFn)(const StepParams);
+typedef void (*BranchFn)(const StepParams, const BranchParams);
 
 // final: the FINAL = true kernels of mt_step_final, built only for the caller's actions with observations written
 template <int ARM, int X, bool RAND>
@@ -808,8 +809,9 @@ static int plan_launch(mt_env *e, const void *fn, size_t per_warp, size_t extra,
     return MT_OK;
 }
 
-// programmatic dependent launch: see griddep_wait() in mt_ptx.cuh
-static int launch_pdl(const void *fn, const LaunchShape &shape, const StepParams &P, cudaStream_t st) {
+// programmatic dependent launch: see griddep_wait() in mt_ptx.cuh.  B: branch_kernel's second parameter
+static int launch_pdl(const void *fn, const LaunchShape &shape, const StepParams &P, cudaStream_t st,
+                      const BranchParams *B = nullptr) {
     cudaLaunchConfig_t lc = {};
     lc.gridDim = dim3(shape.grid);
     lc.blockDim = dim3(shape.wpb * kTile);
@@ -820,7 +822,7 @@ static int launch_pdl(const void *fn, const LaunchShape &shape, const StepParams
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     lc.attrs = attr;
     lc.numAttrs = 1;
-    void *args[] = {(void *)&P};
+    void *args[] = {(void *)&P, (void *)B};
     CU(cudaLaunchKernelExC(&lc, fn, args));
     return MT_OK;
 }
@@ -1215,6 +1217,81 @@ extern "C" int mt_rollout_final(mt_env *e, int32_t n_steps, const float *actions
     DeviceGuard guard(e->cfg.device);
     return rollout_trajectory(e, n_steps, actions_dev, drawn_dev, obs_dev, reward_dev, done_dev, final_obs_dev,
                               final_return_dev, final_length_dev, (cudaStream_t)stream);
+}
+
+// Branch kernels (branch_kernel, mt_step.cuh): the built-in arms at X = 10, 20 and run time, as pick_rollout; every other
+// DH table -- run-time tables and the tables of NVRTC handles alike (`arm` is J for both, StepParams::arm holds the
+// table) -- through the run-time-table instantiation ARM = J, X = 0.
+template <int ARM, int X>
+static BranchFn pick_branch_obs(bool wobs, bool f16) {
+    if (!wobs) return branch_kernel<ARM, X, false, false>;
+    return f16 ? branch_kernel<ARM, X, true, true> : branch_kernel<ARM, X, true, false>;
+}
+
+template <int ARM>
+static BranchFn pick_branch_x(int x, bool wobs, bool f16) {
+    switch (x) {
+        case 10: return pick_branch_obs<ARM, 10>(wobs, f16);
+        case 20: return pick_branch_obs<ARM, 20>(wobs, f16);
+        default: return pick_branch_obs<ARM, 0>(wobs, f16);
+    }
+}
+
+static BranchFn pick_branch(int arm, int x, bool wobs, bool f16) {
+    switch (arm) {
+        case 0: return pick_branch_x<0>(x, wobs, f16);
+        case 2: return pick_branch_obs<2, 0>(wobs, f16);
+        case 3: return pick_branch_obs<3, 0>(wobs, f16);
+        case 4: return pick_branch_obs<4, 0>(wobs, f16);
+        case 5: return pick_branch_obs<5, 0>(wobs, f16);
+        case 6: return pick_branch_obs<6, 0>(wobs, f16);
+        case 7: return pick_branch_obs<7, 0>(wobs, f16);
+        case 8: return pick_branch_obs<8, 0>(wobs, f16);
+#define MT_PICK(ID) case ID: return pick_branch_x<ID>(x, wobs, f16);
+        MT_FOR_EACH_PRESET_ARM(MT_PICK)
+#undef MT_PICK
+    }
+    return nullptr;
+}
+
+constexpr long long kMaxBranches = 2000000000ll;   // the 32-bit env index of mt_create
+
+extern "C" int mt_rollout_branches(mt_env *e, int32_t n_steps, int64_t n_branches, const int64_t *src_dev,
+                                   const float *actions_dev, float gamma, float *return_dev, int32_t *length_dev,
+                                   uint8_t *done_dev, void *obs_dev, void *stream) {
+    // the arguments first: none of these checks needs the handle or a device
+    if (n_steps < 0 || n_steps > 4096) return fail(MT_ERR_INVALID, "n_steps must be in [0, 4096]");
+    if (n_branches < 0 || n_branches > kMaxBranches) return fail(MT_ERR_INVALID, "n_branches must be in [0, 2000000000]");
+    if (!(gamma >= 0.0f && gamma <= 1.0f)) return fail(MT_ERR_INVALID, "gamma must be finite and in [0, 1]");
+    int rc;
+    if ((rc = check_ptr(src_dev, "src_dev", true))) return rc;
+    if ((rc = check_ptr(actions_dev, "actions_dev", true))) return rc;
+    if ((rc = check_ptr(return_dev, "return_dev", true))) return rc;
+    if ((rc = check_ptr(length_dev, "length_dev", true))) return rc;
+    if ((rc = check_ptr(done_dev, "done_dev", true))) return rc;
+    if ((rc = check_ptr(obs_dev, "obs_dev", false))) return rc;
+    if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    if (!e->was_reset) return fail(MT_ERR_STATE, "mt_rollout_branches before mt_reset");
+    if (n_steps == 0 || n_branches == 0) return MT_OK;
+    DeviceGuard guard(e->cfg.device);
+    const bool wobs = obs_dev != nullptr;
+    const void *fn = (const void *)pick_branch(e->arm, e->cfg.n_obj, wobs, e->f16);
+    if (!fn) return fail(MT_ERR_INVALID, "no branch kernel for arm=%d", e->arm);
+    StepParams P = e->base;
+    P.flags &= ~kAutoReset;                       // settle_step then resets nothing and writes nothing
+    P.actions = actions_dev;
+    P.obs = obs_dev;
+    P.done = done_dev;
+    P.n_steps = n_steps;
+    P.tile_begin = 0;
+    P.tile_end = (n_branches + kTile - 1) / kTile;
+    const BranchParams B{src_dev, return_dev, length_dev, (long long)n_branches, gamma};
+    const size_t nb = wobs ? 2 : 1;               // objectives (+ observations) per warp
+    LaunchShape shape;
+    if ((rc = plan_launch(e, fn, nb * P.tile_bytes, 0, P.tile_end, shape))) return rc;
+    if ((rc = launch_pdl(fn, shape, P, (cudaStream_t)stream, &B))) return rc;
+    e->launches++;
+    return MT_OK;
 }
 
 extern "C" int mt_host_alloc(void **out, uint64_t bytes) {

@@ -117,6 +117,17 @@ struct StepParams {
     int32_t *final_length;     // [N] episode length (the saturating counter)
 };
 
+// branch_kernel's own parameters (mt_rollout_branches), beside a StepParams whose actions ([n_steps][M][J]), done ([M]) and
+// obs ([M][3X] or nullptr) are per branch.  A second parameter rather than more StepParams fields: every other kernel
+// keeps its parameter layout, and with it its code.
+struct BranchParams {
+    const int64_t *src;        // [M] source env of each branch
+    float *ret;                // [M] discounted return
+    int32_t *length;           // [M] steps executed
+    long long n;               // M
+    float gamma;
+};
+
 // Trajectory buffers (mt_rollout) are arrays of slices: slice s holds step s's rows 0 .. N-1, packed, so row `row` of
 // slice s starts at base + (s N + row) row_bytes.  Computed in 64 bits: s N row_bytes passes 2^32 at sizes users run
 // (2^20 envs x 36 steps x 120 B of observations).
@@ -1406,6 +1417,134 @@ rollout_kernel(const __grid_constant__ StepParams P) {
         if (WOBS && lane == 0) bulk_wait_read0();
     }
     block_epilogue(P, lane, wpb, ground_steps, blk_stat, &warps_done);
+}
+
+// ---------------------------------------------------------------------------
+// Branches: K steps of the caller's actions from copies of chosen envs, leaving the handle untouched (mt_rollout_branches).
+//
+// Branch m starts from the current state of env B.src[m] -- goals, alive word, episode length and raw objectives --
+// and takes the actions of slice s of P.actions ([K][M][J], the layout of mt_rollout) at step s.  A step is the step of
+// every other kernel (the arm code, walk_row, settle_step) with kAutoReset cleared in P.flags by the host, so settle_step
+// writes nothing and no branch is reset.  A branch ends at the first step whose done byte is non-zero; from then on its
+// outputs are frozen: the discounted return (d_0 = 1, d_{s+1} = fl(d_s gamma), G_{s+1} = fl(G_s + d_s r_s), exact
+// products as r_s is -1, 0 or +1), the steps executed, the done byte of the ending step (0 after all K) and, when WOBS,
+// obs2 of the last executed step.  Nothing of the handle is written: no state, no statistics, no launch ticket.
+//
+// One lane per branch, a persistent grid over ceil(M / 32) tiles taken from the block's queue, as in rollout_kernel.
+// Each lane gathers its source's scalars and copies its source's objective row into its row of the warp's buffer, once
+// per call; a gathered row is 12X bytes at an arbitrary row, generally not 16-byte aligned, so this is a per-lane copy and
+// not a bulk copy.  The source index is bounds-checked before any load that uses it: a branch whose source is outside
+// [0, N) computes as if from row 0 and writes NaN / -1 / 0 and no observation.  A lane past M has the zero goals and
+// actions of a padding row.  An ended branch keeps stepping, with its own actions, exactly as an env of a handle without
+// auto-reset does: ref_arm picks its sub-pose recurrence for the whole warp (__all_sync), so a lane that froze its pose or
+// skipped its actions could change the path, and with it the last bits, of the branches that go on.  The warp leaves
+// the step loop once all its branches have ended.
+// With WOBS, a step on which some lane of the warp ends (about one env-step in 550 under random actions), and the last
+// step, walks the objectives a second time into the warp's second buffer, with the same frames and entry alive mask; each
+// lane that ends there, or is still running at the last step, stores its row.  Other steps cost what a rollout without
+// observations costs.
+// ---------------------------------------------------------------------------
+template <int ARM, int X, bool WOBS, bool F16>
+__global__ void __launch_bounds__(((ARM == 0) ? kMaxWarpsRefArm : kMaxWarpsGeneric) * kTile, 1)
+branch_kernel(const __grid_constant__ StepParams P, const __grid_constant__ BranchParams B) {
+    static_assert(WOBS || !F16, "F16 is an observation format");
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ int queue_next;
+    constexpr int J = ArmJoints<ARM>::value;
+    constexpr int NB = WOBS ? 2 : 1;                      // objectives (+ observations) of the warp's branches
+    const int lane = threadIdx.x & 31;
+    const int warp = __reduce_max_sync(0xffffffffu, (int)(threadIdx.x >> 5));
+    const int x = X ? X : P.n_obj;
+    const int rowlen = 3 * x;
+    const uint32_t pts = smem_addr(smem) + (uint32_t)(NB * warp) * P.tile_bytes, obuf = pts + P.tile_bytes;
+    const uint32_t row = pts + (uint32_t)(lane * rowlen) * 4u, orow = obuf + (uint32_t)(lane * rowlen) * 4u;
+    const uint32_t queue = smem_addr(&queue_next);
+    const uint64_t pol_stream = P.pol_stream, pol_keep = P.pol_state;
+    const int tile_end = (int)P.tile_end, n_branches = (int)B.n, n_src = (int)P.n;
+    auto tile_of = [&](int li) -> int {
+        const int t = li * (int)gridDim.x + (int)blockIdx.x;
+        return t < tile_end ? t : -1;
+    };
+    if (threadIdx.x == 0) queue_next = blockDim.x >> 5;
+    __syncthreads();
+    int cur = tile_of(warp);
+    griddep_launch_dependents();
+    griddep_wait();                                       // nothing is read before the previous grid is complete
+    const int ep_shift = ep_shift_of<X>(P);
+    const uint32_t amask = ep_shift ? ((1u << ep_shift) - 1u) : 0xffffffffu;
+    while (cur >= 0) {
+        const int m0 = cur * kTile, m = m0 + lane;
+        const bool in = m < n_branches, full = m0 + kTile <= n_branches;
+        const long long src64 = in ? (long long)B.src[m] : 0ll;
+        const bool ok = in && src64 >= 0 && src64 < (long long)n_src;
+        const int src = ok ? (int)src64 : 0;              // every gathered load below reads row `src`, inside [0, N)
+        TileScalars<J> sc;
+        load_scalars<J, X, true>(P, src, sc, pol_keep, pol_stream);
+        if (!in) {
+#pragma unroll
+            for (int i = 0; i < J; ++i) sc.g[i] = 0.f;
+        }
+        uint32_t alive = sc.word & amask, eplen = ep_shift ? sc.word >> ep_shift : sc.cnt;
+        float total = sc.total;
+        const float *prow = P.points + (size_t)src * (size_t)rowlen;
+        if ((rowlen & 1) == 0) {                          // even X: rows are 8-byte aligned
+            for (int i = 0; i < rowlen; i += 2) sts_f2(row + 4u * i, ld_hint(reinterpret_cast<const float2 *>(prow + i), pol_keep));
+        } else {
+            for (int i = 0; i < rowlen; ++i) sts_f(row + 4u * i, ld_hint(prow + i, pol_keep));
+        }
+        bool live = ok;
+        float ret = 0.f, disc = 1.f;
+        int len = 0;
+        uint8_t end_done = 0;
+        uint32_t ground_steps = 0;                        // settle_step counts them; nothing reads them here
+        for (int s = 0; s < P.n_steps && __any_sync(0xffffffffu, live); ++s) {
+            const size_t srow = (size_t)s * (size_t)n_branches;
+            load_action_row<J>(in ? P.actions + (srow + (size_t)m) * J : nullptr, sc.a, pol_stream);
+            // the next step's action tile towards the L2 while this step computes (a hint: aligned full tiles only)
+            const float *next = P.actions + (srow + (size_t)n_branches + (size_t)m0) * J;
+            if (full && lane == 0 && s + 1 < P.n_steps && bulk_aligned((uintptr_t)next))
+                bulk_prefetch_l2(next, (uint32_t)(kTile * 4 * J));
+            Frames f;
+            if (ARM == 0) ref_arm<false>(sc.g, sc.a, P.substeps, P.inv_div, f, nullptr);
+            else generic_arm<ARM, false>(P, sc.g, sc.a, f, nullptr);
+            const bool neg = f.zmin < 0.0f;
+            const uint32_t caught = walk_row<X, false>(row, row, x, f, P.catch_tol, alive);
+            float gn[J], rew;
+            uint32_t alive1;
+            uint8_t done;
+            settle_step<J, false>(P, lane, m0, in, x, rowlen, neg, alive, caught, sc.a, gn, total, alive1, eplen, rew, done,
+                                  ground_steps, nullptr, 0u, 0u, 0);
+            if (WOBS) {
+                const bool last = live && (done != 0 || s + 1 == P.n_steps);
+                if (__any_sync(0xffffffffu, last)) {      // warp-uniform, rare
+                    walk_row<X, true>(row, orow, x, f, P.catch_tol, alive);
+                    if (last) {
+                        void *dst = obs_at<F16>(P.obs, (size_t)m * rowlen);
+                        for (int i = 0; i < rowlen; ++i) store_obs<F16>(dst, i, lds_f(orow + 4u * i));
+                    }
+                }
+            }
+            if (live) {
+                ret = ret + disc * rew;
+                disc = disc * B.gamma;
+                len = s + 1;
+                end_done = done;
+                live = done == 0;
+            }
+            alive = alive1;
+#pragma unroll
+            for (int i = 0; i < J; ++i) sc.g[i] = gn[i];
+        }
+        if (in) {
+            B.ret[m] = ok ? ret : __int_as_float(0x7fc00000);
+            B.length[m] = ok ? len : -1;
+            P.done[m] = ok ? end_done : (uint8_t)0;
+        }
+        int li = 0;
+        if (lane == 0) li = atom_add_s(queue, 1);
+        cur = tile_of(__reduce_max_sync(0xffffffffu, li));
+        __syncwarp();                                     // every lane is done with its rows before the next tile's copy
+    }
 }
 
 }  // namespace mt
