@@ -273,6 +273,40 @@ int mt_rollout_branches(mt_env *env, int32_t n_steps, int64_t n_branches, const 
                         const float *actions_dev, float gamma, float *return_dev, int32_t *length_dev,
                         uint8_t *done_dev, void *obs_dev, void *stream);
 
+/* mt_rollout_branches with the actions of steps n_prefix .. n_steps-1 drawn in the kernel from the environment's own
+ * random policy (mt_sample_actions: integer degrees uniform on [action_low, action_high)) -- random shooting,
+ * Monte-Carlo state values, rollout-based Q estimates -- in O(M) memory instead of O(n_steps M).
+ *   prefix_dev   [n_prefix][M][J] fp32 degrees, mt_rollout_branches' layout: the actions of steps s < n_prefix.  Required
+ *                when n_prefix > 0, and NULL when n_prefix = 0; 0 <= n_prefix <= n_steps <= 4096.
+ *   draw_key_dev one uint64 on the device, read by the kernel (so a CUDA graph that captures this call and an increment
+ *                of the key draws fresh actions at every replay); required, 8-byte aligned.
+ * Draw contract: step s >= n_prefix of branch m (s counted from the start of the branch) takes exactly what
+ * mt_sample_actions draws for GLOBAL ENV ID m at STEP INDEX key + s (mod 2^64), with the handle's current seed (after
+ * any mt_set_seed), action range and J.  So a branch's draws depend on (seed, m, key) only: not on src, on M, on
+ * env_id_base or on the handle's step index.  Two calls whose [key, key + n_steps) ranges overlap reuse draws for the
+ * same m: advance the key by n_steps per call.  Two handles with the same seed and key draw the same actions for the
+ * same m: sharded callers give each rank its own key range.
+ * Everything else is mt_rollout_branches': sources, steps, endings, the fp32 return order, the outputs, sources outside
+ * [0, N) (NaN / -1 / 0, obs row untouched), the handle left untouched, the argument errors and their order (n_prefix
+ * outside [0, n_steps] and a prefix_dev that disagrees with n_prefix are MT_ERR_INVALID too) and MT_ERR_STATE before
+ * mt_reset.  The result is bit for bit mt_rollout_branches fed concat(prefix, mt_branch_actions(key, n_prefix,
+ * n_steps - n_prefix, rows 0 .. M-1)).  A branch-step reads no action bytes past the prefix. */
+int mt_rollout_branches_random(mt_env *env, int32_t n_steps, int32_t n_prefix, int64_t n_branches,
+                               const int64_t *src_dev, const float *prefix_dev, const uint64_t *draw_key_dev,
+                               float gamma, float *return_dev, int32_t *length_dev, uint8_t *done_dev,
+                               void *obs_dev, void *stream);
+
+/* The draws of chosen branches of mt_rollout_branches_random: out_dev [n_steps][n_rows][J] fp32, slice s, row r =
+ * the actions of branch id branch_dev[r] at branch step first_step + s under the key *draw_key_dev, i.e. what
+ * mt_sample_actions draws for global env id branch_dev[r] at step index key + first_step + s (mod 2^64).  Any int64
+ * id is valid (its 64-bit pattern is the global id).  A planner that picked branch b of a call gets the action it
+ * executes with first_step = 0, n_steps = 1.  Reads only the seed, the action range and J of the handle: it needs no
+ * mt_reset, and writes nothing of the handle.  Asynchronous on `stream`.  Argument errors come before the handle is
+ * looked at: draw_key_dev NULL or not 8-byte aligned, first_step < 0, n_steps < 0, n_rows outside [0, 2e9], and
+ * branch_dev / out_dev NULL or not 16-byte aligned are MT_ERR_INVALID; n_steps = 0 or n_rows = 0 does nothing. */
+int mt_branch_actions(mt_env *env, const uint64_t *draw_key_dev, int32_t first_step, int32_t n_steps,
+                      int64_t n_rows, const int64_t *branch_dev, float *out_dev, void *stream);
+
 /* Host-buffer step: actions_host/obs_host/reward_host/done_host must be pinned
  * (mt_host_alloc).  Copies actions H2D, steps, copies results D2H, chunked over
  * internal streams so copies overlap the kernels; synchronous on return.  Ordered after

@@ -79,6 +79,9 @@ SIGNATURES = {
     "mt_rollout": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "mt_rollout_final": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "mt_rollout_branches": (C.c_int, [_P, C.c_int32, C.c_int64, _P, _P, C.c_float, _P, _P, _P, _P, _P]),
+    "mt_rollout_branches_random": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int64, _P, _P, _P, C.c_float, _P, _P, _P,
+                                             _P, _P]),
+    "mt_branch_actions": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int64, _P, _P, _P]),
     "mt_step_host": (C.c_int, [_P, _P, _P, _P, _P]),
     "mt_host_step_mode": (C.c_int, [_P]),
     "mt_host_alloc": (C.c_int, [C.POINTER(_P), C.c_uint64]),

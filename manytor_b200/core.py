@@ -423,7 +423,7 @@ class BatchedEnvs:
         return (bufs, fin) if final else bufs
 
     def rollout_branches(self, actions, src=None, gamma: float = 1.0, write_obs: bool = False,
-                         out: Optional[Branches] = None) -> Branches:
+                         out: Optional[Branches] = None, *, n_steps: Optional[int] = None, draw_key=None) -> Branches:
         """Score K-step action sequences from copies of chosen envs in one launch, leaving this handle untouched
         (mt_rollout_branches): branch m starts from the current state of env src[m] and steps with actions[:, m] as
         `step` would, until its first done step (included) or the K-th step.  No env is reset inside a branch, and the
@@ -435,7 +435,18 @@ class BatchedEnvs:
         and leaves its obs row alone.  gamma in [0, 1]: ret is sum of gamma**s * r_s in fp32, d_0 = 1, d_{s+1} = d_s *
         gamma, G += d_s * r_s.  write_obs: also return obs2 of each branch's last executed step.  `out`: a Branches of
         preallocated buffers (obs None unless write_obs), e.g. fixed storage for a CUDA graph that captures this call.
-        Shape and dtype errors raise ValueError before the library is called."""
+        Shape and dtype errors raise ValueError before the library is called.
+
+        In-kernel draws (mt_rollout_branches_random), with `n_steps` and / or `draw_key`: the branches run n_steps = K
+        steps (default: the prefix's length; required without a prefix); `actions` is None (every step drawn) or a
+        (P, M, J) prefix of the first P <= K steps, and the other steps take the environment's own random policy,
+        integer degrees uniform on [action_low, action_high).  Step s of branch m draws what `sample_actions` draws for global env id m at step
+        index draw_key + s (mod 2^64): the draws depend on (seed, m, draw_key) only, and `branch_actions` returns them
+        again.  Calls whose [draw_key, draw_key + K) overlap reuse draws, so advance the key by K per call.  draw_key:
+        an int, or a (1,) int64 tensor on this device holding the key's bits, read by the kernel (a CUDA graph that
+        captures this call and a `key += K` draws fresh actions at every replay).  M is len(src), or N with src=None."""
+        if n_steps is not None or draw_key is not None:
+            return self._rollout_branches_random(actions, src, gamma, write_obs, out, n_steps, draw_key)
         shape = tuple(actions.shape) if hasattr(actions, "shape") else tuple(np.shape(actions))
         if len(shape) != 3 or shape[2] != self.j:
             raise ValueError(f"actions must have shape (K, M, {self.j}), not {shape}")
@@ -481,6 +492,118 @@ class BatchedEnvs:
                                                  self._stream()))
         self._branch_io = (a, s, bufs)                     # keep alive until the stream has consumed them
         return bufs
+
+    def _draw_key(self, draw_key, check_only: bool = False):
+        """The device word of a draw key: a (1,) int64 tensor on this device as it is, or an int (mod 2^64) in a fresh
+        one-element tensor of its own, so that no later call, on whatever stream, can overwrite it before it is read."""
+        if isinstance(draw_key, torch.Tensor):
+            if tuple(draw_key.shape) != (1,) or draw_key.dtype != torch.int64 or draw_key.device != self.device:
+                raise ValueError(f"draw_key must be an int or a (1,) int64 tensor on {self.device}, not a "
+                                 f"{tuple(draw_key.shape)} {draw_key.dtype} tensor on {draw_key.device}")
+            return draw_key
+        if isinstance(draw_key, (bool, np.bool_)) or not isinstance(draw_key, (int, np.integer)):
+            raise ValueError(f"draw_key must be an int or a (1,) int64 tensor on {self.device}, not {draw_key!r}")
+        if check_only:
+            return None
+        k = int(draw_key) % (1 << 64)
+        return torch.full((1,), k - (1 << 64) if k >= 1 << 63 else k, dtype=torch.int64, device=self.device)
+
+    def _aligned_dev(self, a, dtype, shape) -> torch.Tensor:
+        """`a` as a contiguous device tensor of `dtype` and `shape` whose address is 16-byte aligned, as the library
+        requires: such a tensor on this device as it is, anything else converted, and a view that starts off the
+        alignment (e.g. best[1:]) copied into storage of its own."""
+        if (isinstance(a, torch.Tensor) and a.is_cuda and a.device == self.device and a.dtype == dtype
+                and a.is_contiguous() and a.data_ptr() % 16 == 0):
+            return a.reshape(shape)
+        t = self._as_dev(a, dtype, shape)
+        return t if t.data_ptr() % 16 == 0 else t.clone()
+
+    def _dev_ids(self, ids, m: int) -> torch.Tensor:
+        """(m,) integers as an int64 device tensor (_aligned_dev)."""
+        return self._aligned_dev(ids, torch.int64, (m,))
+
+    @staticmethod
+    def _int_vector(v, name: str, m: Optional[int] = None) -> int:
+        """Check that v is a 1-D array of integers (of m entries when m is given); return its length."""
+        shape = tuple(v.shape) if hasattr(v, "shape") else tuple(np.shape(v))
+        if len(shape) != 1 or (m is not None and shape[0] != m):
+            raise ValueError(f"{name} must have shape ({'M' if m is None else m},), not {shape}")
+        dtype = v.dtype if isinstance(v, torch.Tensor) else torch.as_tensor(np.asarray(v)).dtype
+        if dtype.is_floating_point or dtype.is_complex or dtype == torch.bool:
+            raise ValueError(f"{name} must hold integers, not {dtype}")
+        return shape[0]
+
+    def _rollout_branches_random(self, actions, src, gamma, write_obs, out, n_steps, draw_key) -> Branches:
+        if draw_key is None:
+            raise ValueError("in-kernel draws need an explicit draw_key: the same key regenerates them (branch_actions)")
+        self._draw_key(draw_key, check_only=True)
+        m = self.n if src is None else self._int_vector(src, "src")
+        p = 0
+        if actions is not None:
+            shape = tuple(actions.shape) if hasattr(actions, "shape") else tuple(np.shape(actions))
+            if len(shape) != 3 or shape[1:] != (m, self.j):
+                raise ValueError(f"a prefix of actions must have shape (P, {m}, {self.j}) (M = "
+                                 f"{'N' if src is None else 'len(src)'}), not {shape}")
+            p = shape[0]
+        if n_steps is None and actions is None:
+            raise ValueError("n_steps is required when actions is None (every step drawn): it is the branches' length")
+        k = p if n_steps is None else int(n_steps)
+        if not 0 <= k <= 4096:
+            raise ValueError(f"n_steps must be in [0, 4096], not {k}")
+        if p > k:
+            raise ValueError(f"the prefix has {p} steps, more than n_steps = {k}")
+        g = float(gamma)
+        if not 0.0 <= g <= 1.0:
+            raise ValueError(f"gamma must be finite and in [0, 1], not {gamma}")
+        want = {"ret": ((m,), torch.float32), "length": ((m,), torch.int32), "done": ((m,), torch.uint8),
+                "obs": ((m, 3 * self.x), self.obs_dtype) if write_obs else None}
+        if out is not None:
+            self._check_out(out, Branches, "out", want, f"write_obs={write_obs}")
+            bufs = out
+        else:
+            bufs = Branches(*(self._empty(*spec) if spec is not None else None for spec in want.values()))
+        if k == 0 or m == 0:                               # nothing to do (and empty tensors have no address)
+            return bufs
+        a = self._aligned_dev(actions, torch.float32, (p, m, self.j)) if p > 0 else None
+        s = torch.arange(self.n, dtype=torch.int64, device=self.device) if src is None else self._dev_ids(src, m)
+        key = self._draw_key(draw_key)
+        _lib.check(self._lib.mt_rollout_branches_random(self._h, k, p, m, self._p(s), self._p(a), self._p(key), g,
+                                                        self._p(bufs.ret), self._p(bufs.length), self._p(bufs.done),
+                                                        self._p(bufs.obs), self._stream()))
+        self._branch_io = (a, s, key, bufs)                # keep alive until the stream has consumed them
+        return bufs
+
+    def branch_actions(self, branches, draw_key, n_steps: int, first_step: int = 0,
+                       out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The actions in-kernel draws give chosen branches (mt_branch_actions): out[s, r] = the actions of branch id
+        branches[r] at branch step first_step + s under `draw_key`, as `rollout_branches(draw_key=...)` drew them --
+        `sample_actions` for global env id branches[r] at step index draw_key + first_step + s (mod 2^64).  Returns
+        (n_steps, R, J) float32.  The action a planner executes after picking branch b: branch_actions([b], key, 1).
+        branches: (R,) integers, any int64 value.  draw_key: as in rollout_branches.  Needs no reset and changes nothing
+        of the handle.  Shape and range errors raise ValueError before the library is called."""
+        r = self._int_vector(branches, "branches")
+        self._draw_key(draw_key, check_only=True)
+        k, first = int(n_steps), int(first_step)
+        if not 0 <= k < 1 << 31:
+            raise ValueError(f"n_steps must be in [0, 2^31), not {n_steps}")
+        if not 0 <= first < 1 << 31:
+            raise ValueError(f"first_step must be in [0, 2^31), not {first_step}")
+        if r > 2000000000:
+            raise ValueError(f"at most 2000000000 branches, not {r}")
+        shape = (k, r, self.j)
+        if out is None:
+            out = self._empty(shape, torch.float32)
+        elif not isinstance(out, torch.Tensor) or tuple(out.shape) != shape or out.dtype != torch.float32:
+            raise ValueError(f"out must be a tensor of shape {shape} and dtype torch.float32")
+        elif not out.is_contiguous() or out.device != self.device or out.data_ptr() % 16 != 0:
+            raise ValueError(f"out must be a contiguous, 16-byte aligned tensor on {self.device}")
+        if k == 0 or r == 0:                               # nothing to do (and empty tensors have no address)
+            return out
+        ids, key = self._dev_ids(branches, r), self._draw_key(draw_key)
+        _lib.check(self._lib.mt_branch_actions(self._h, self._p(key), first, k, r, self._p(ids), self._p(out),
+                                               self._stream()))
+        self._branch_actions_io = (ids, key, out)          # keep alive until the stream has consumed them
+        return out
 
     # -- host-buffer (end-to-end) step ------------------------------------------
     def pinned(self, name: str, shape, dtype) -> np.ndarray:

@@ -620,6 +620,24 @@ __global__ void sample_actions_kernel(const __grid_constant__ StepParams P, floa
     for (int i = 0; i < P.n_joints; ++i) actions[env * P.n_joints + i] = a[i];
 }
 
+// mt_branch_actions: out[s][r] = the draws of branch id ids[r] at branch step first + s, i.e. what mt_sample_actions
+// draws for global env id ids[r] at step index *key + first + s (mod 2^64) -- what branch_kernel<.., DRAW = true>
+// draws.  One thread per (s, r), grid-stride.
+__global__ void branch_actions_kernel(const __grid_constant__ StepParams P, const unsigned long long *key, int first,
+                                      int n_steps, long long rows, const int64_t *ids, float *out) {
+    const long long total = (long long)n_steps * rows;
+    const unsigned long long k0 = *key + (unsigned long long)first;
+    const int J = P.n_joints;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const long long s = i / rows, r = i - s * rows;
+        float a[MT_MAX_JOINTS];
+        draw_actions(P, k0 + (unsigned long long)s, (long long)ids[r], J, a);
+#pragma unroll
+        for (int j = 0; j < MT_MAX_JOINTS; ++j)       // constant indices: `a` stays in registers
+            if (j < J) out[i * J + j] = a[j];
+    }
+}
+
 // stats: the device-side counters (env-steps, finished-episode sums, ground-contact steps) + a
 // block/warp-shuffle reduction of the in-progress total_reward, written as MT_STATS_WORDS int64.
 __global__ void stats_kernel(const __grid_constant__ StepParams P, long long *out) {
@@ -1222,32 +1240,34 @@ extern "C" int mt_rollout_final(mt_env *e, int32_t n_steps, const float *actions
 // Branch kernels (branch_kernel, mt_step.cuh): the built-in arms at X = 10, 20 and run time, as pick_rollout; every other
 // DH table -- run-time tables and the tables of NVRTC handles alike (`arm` is J for both, StepParams::arm holds the
 // table) -- through the run-time-table instantiation ARM = J, X = 0.
-template <int ARM, int X>
+// DRAW: the kernels of mt_rollout_branches_random (in-kernel draws after the caller's prefix).
+template <int ARM, int X, bool DRAW>
 static BranchFn pick_branch_obs(bool wobs, bool f16) {
-    if (!wobs) return branch_kernel<ARM, X, false, false>;
-    return f16 ? branch_kernel<ARM, X, true, true> : branch_kernel<ARM, X, true, false>;
+    if (!wobs) return branch_kernel<ARM, X, false, false, DRAW>;
+    return f16 ? branch_kernel<ARM, X, true, true, DRAW> : branch_kernel<ARM, X, true, false, DRAW>;
 }
 
-template <int ARM>
+template <int ARM, bool DRAW>
 static BranchFn pick_branch_x(int x, bool wobs, bool f16) {
     switch (x) {
-        case 10: return pick_branch_obs<ARM, 10>(wobs, f16);
-        case 20: return pick_branch_obs<ARM, 20>(wobs, f16);
-        default: return pick_branch_obs<ARM, 0>(wobs, f16);
+        case 10: return pick_branch_obs<ARM, 10, DRAW>(wobs, f16);
+        case 20: return pick_branch_obs<ARM, 20, DRAW>(wobs, f16);
+        default: return pick_branch_obs<ARM, 0, DRAW>(wobs, f16);
     }
 }
 
+template <bool DRAW>
 static BranchFn pick_branch(int arm, int x, bool wobs, bool f16) {
     switch (arm) {
-        case 0: return pick_branch_x<0>(x, wobs, f16);
-        case 2: return pick_branch_obs<2, 0>(wobs, f16);
-        case 3: return pick_branch_obs<3, 0>(wobs, f16);
-        case 4: return pick_branch_obs<4, 0>(wobs, f16);
-        case 5: return pick_branch_obs<5, 0>(wobs, f16);
-        case 6: return pick_branch_obs<6, 0>(wobs, f16);
-        case 7: return pick_branch_obs<7, 0>(wobs, f16);
-        case 8: return pick_branch_obs<8, 0>(wobs, f16);
-#define MT_PICK(ID) case ID: return pick_branch_x<ID>(x, wobs, f16);
+        case 0: return pick_branch_x<0, DRAW>(x, wobs, f16);
+        case 2: return pick_branch_obs<2, 0, DRAW>(wobs, f16);
+        case 3: return pick_branch_obs<3, 0, DRAW>(wobs, f16);
+        case 4: return pick_branch_obs<4, 0, DRAW>(wobs, f16);
+        case 5: return pick_branch_obs<5, 0, DRAW>(wobs, f16);
+        case 6: return pick_branch_obs<6, 0, DRAW>(wobs, f16);
+        case 7: return pick_branch_obs<7, 0, DRAW>(wobs, f16);
+        case 8: return pick_branch_obs<8, 0, DRAW>(wobs, f16);
+#define MT_PICK(ID) case ID: return pick_branch_x<ID, DRAW>(x, wobs, f16);
         MT_FOR_EACH_PRESET_ARM(MT_PICK)
 #undef MT_PICK
     }
@@ -1275,7 +1295,7 @@ extern "C" int mt_rollout_branches(mt_env *e, int32_t n_steps, int64_t n_branche
     if (n_steps == 0 || n_branches == 0) return MT_OK;
     DeviceGuard guard(e->cfg.device);
     const bool wobs = obs_dev != nullptr;
-    const void *fn = (const void *)pick_branch(e->arm, e->cfg.n_obj, wobs, e->f16);
+    const void *fn = (const void *)pick_branch<false>(e->arm, e->cfg.n_obj, wobs, e->f16);
     if (!fn) return fail(MT_ERR_INVALID, "no branch kernel for arm=%d", e->arm);
     StepParams P = e->base;
     P.flags &= ~kAutoReset;                       // settle_step then resets nothing and writes nothing
@@ -1290,6 +1310,79 @@ extern "C" int mt_rollout_branches(mt_env *e, int32_t n_steps, int64_t n_branche
     LaunchShape shape;
     if ((rc = plan_launch(e, fn, nb * P.tile_bytes, 0, P.tile_end, shape))) return rc;
     if ((rc = launch_pdl(fn, shape, P, (cudaStream_t)stream, &B))) return rc;
+    e->launches++;
+    return MT_OK;
+}
+
+// The draw key is one uint64 word on the device, read by the kernels: 8-byte alignment is all it needs.
+static int check_key(const uint64_t *key) {
+    if (!key) return fail(MT_ERR_INVALID, "draw_key_dev is NULL");
+    if (((uintptr_t)key & 7u) != 0) return fail(MT_ERR_INVALID, "draw_key_dev must be 8-byte aligned");
+    return MT_OK;
+}
+
+extern "C" int mt_rollout_branches_random(mt_env *e, int32_t n_steps, int32_t n_prefix, int64_t n_branches,
+                                          const int64_t *src_dev, const float *prefix_dev, const uint64_t *draw_key_dev,
+                                          float gamma, float *return_dev, int32_t *length_dev, uint8_t *done_dev,
+                                          void *obs_dev, void *stream) {
+    // the arguments first, in mt_rollout_branches' order: none of these checks needs the handle or a device
+    if (n_steps < 0 || n_steps > 4096) return fail(MT_ERR_INVALID, "n_steps must be in [0, 4096]");
+    if (n_prefix < 0 || n_prefix > n_steps) return fail(MT_ERR_INVALID, "n_prefix must be in [0, n_steps]");
+    if (n_branches < 0 || n_branches > kMaxBranches) return fail(MT_ERR_INVALID, "n_branches must be in [0, 2000000000]");
+    if (!(gamma >= 0.0f && gamma <= 1.0f)) return fail(MT_ERR_INVALID, "gamma must be finite and in [0, 1]");
+    int rc;
+    if ((rc = check_ptr(src_dev, "src_dev", true))) return rc;
+    if ((rc = check_ptr(prefix_dev, "prefix_dev", n_prefix > 0))) return rc;
+    if (n_prefix == 0 && prefix_dev) return fail(MT_ERR_INVALID, "prefix_dev must be NULL when n_prefix is 0");
+    if ((rc = check_key(draw_key_dev))) return rc;
+    if ((rc = check_ptr(return_dev, "return_dev", true))) return rc;
+    if ((rc = check_ptr(length_dev, "length_dev", true))) return rc;
+    if ((rc = check_ptr(done_dev, "done_dev", true))) return rc;
+    if ((rc = check_ptr(obs_dev, "obs_dev", false))) return rc;
+    if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    if (!e->was_reset) return fail(MT_ERR_STATE, "mt_rollout_branches_random before mt_reset");
+    if (n_steps == 0 || n_branches == 0) return MT_OK;
+    DeviceGuard guard(e->cfg.device);
+    const bool wobs = obs_dev != nullptr;
+    const void *fn = (const void *)pick_branch<true>(e->arm, e->cfg.n_obj, wobs, e->f16);
+    if (!fn) return fail(MT_ERR_INVALID, "no branch kernel for arm=%d", e->arm);
+    StepParams P = e->base;
+    P.flags &= ~kAutoReset;                       // settle_step then resets nothing and writes nothing
+    P.actions = prefix_dev;
+    P.obs = obs_dev;
+    P.done = done_dev;
+    P.n_steps = n_steps;
+    P.tile_begin = 0;
+    P.tile_end = (n_branches + kTile - 1) / kTile;
+    P.trig_span = trig_table_entries(e);          // the drawn steps' sin / cos table, after the per-warp buffers
+    const BranchParams B{src_dev, return_dev, length_dev, (long long)n_branches, gamma, n_prefix,
+                         reinterpret_cast<const unsigned long long *>(draw_key_dev)};
+    const size_t nb = wobs ? 2 : 1;               // objectives (+ observations) per warp
+    LaunchShape shape;
+    if ((rc = plan_launch(e, fn, nb * P.tile_bytes, (size_t)P.trig_span * 8, P.tile_end, shape))) return rc;
+    if ((rc = launch_pdl(fn, shape, P, (cudaStream_t)stream, &B))) return rc;
+    e->launches++;
+    return MT_OK;
+}
+
+extern "C" int mt_branch_actions(mt_env *e, const uint64_t *draw_key_dev, int32_t first_step, int32_t n_steps,
+                                 int64_t n_rows, const int64_t *branch_dev, float *out_dev, void *stream) {
+    // the arguments first: none of these checks needs the handle or a device
+    int rc;
+    if ((rc = check_key(draw_key_dev))) return rc;
+    if (first_step < 0) return fail(MT_ERR_INVALID, "first_step must be >= 0");
+    if (n_steps < 0) return fail(MT_ERR_INVALID, "n_steps must be >= 0");
+    if (n_rows < 0 || n_rows > kMaxBranches) return fail(MT_ERR_INVALID, "n_rows must be in [0, 2000000000]");
+    if ((rc = check_ptr(branch_dev, "branch_dev", true))) return rc;
+    if ((rc = check_ptr(out_dev, "out_dev", true))) return rc;
+    if (!e) return fail(MT_ERR_INVALID, "env is NULL");
+    if (n_steps == 0 || n_rows == 0) return MT_OK;
+    DeviceGuard guard(e->cfg.device);
+    const long long total = (long long)n_steps * n_rows;
+    const long long blocks = (total + 255) / 256, cap = (long long)e->num_sms * 64;
+    branch_actions_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, (cudaStream_t)stream>>>(
+        e->base, reinterpret_cast<const unsigned long long *>(draw_key_dev), first_step, n_steps, n_rows, branch_dev, out_dev);
+    CU(cudaGetLastError());
     e->launches++;
     return MT_OK;
 }

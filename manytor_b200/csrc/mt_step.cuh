@@ -126,6 +126,9 @@ struct BranchParams {
     int32_t *length;           // [M] steps executed
     long long n;               // M
     float gamma;
+    // branch_kernel<.., DRAW = true> only (mt_rollout_branches_random); after the fields above, whose offsets stay put
+    int32_t n_prefix;          // steps 0 .. n_prefix-1 read P.actions ([n_prefix][M][J]); the others are drawn
+    const unsigned long long *draw_key;   // step s >= n_prefix of branch m draws as mt_sample_actions at env m, index key + s
 };
 
 // Trajectory buffers (mt_rollout) are arrays of slices: slice s holds step s's rows 0 .. N-1, packed, so row `row` of
@@ -1443,8 +1446,16 @@ rollout_kernel(const __grid_constant__ StepParams P) {
 // step, walks the objectives a second time into the warp's second buffer, with the same frames and entry alive mask; each
 // lane that ends there, or is still running at the last step, stores its row.  Other steps cost what a rollout without
 // observations costs.
+// DRAW (mt_rollout_branches_random): steps s < B.n_prefix read slice s of P.actions ([n_prefix][M][J]) as above; every
+// later step draws its actions in the kernel, as mt_sample_actions draws them for global env id m at step index
+// *B.draw_key + s (mod 2^64): draw_actions with gid = m, whatever the source, M or the handle's step index.  The key is
+// read once per lane, after griddep_wait.  A lane past M takes zeros on drawn steps too, so the warp computes what
+// branch_kernel<.., DRAW = false> computes when fed the drawn actions, bit for bit.  Drawn steps take sin / cos from the
+// block's ActionTrig table (after the per-warp buffers, as in rollout_kernel) when P.trig_span > 0; prefix steps, and
+// the zeros of a lane past M (0 is outside a range such as [10, 100), so its entry is not in the table), pass no table
+// and evaluate, as DRAW = false does.  No L2 prefetch past the prefix.
 // ---------------------------------------------------------------------------
-template <int ARM, int X, bool WOBS, bool F16>
+template <int ARM, int X, bool WOBS, bool F16, bool DRAW = false>
 __global__ void __launch_bounds__(((ARM == 0) ? kMaxWarpsRefArm : kMaxWarpsGeneric) * kTile, 1)
 branch_kernel(const __grid_constant__ StepParams P, const __grid_constant__ BranchParams B) {
     static_assert(WOBS || !F16, "F16 is an observation format");
@@ -1458,6 +1469,8 @@ branch_kernel(const __grid_constant__ StepParams P, const __grid_constant__ Bran
     const int rowlen = 3 * x;
     const uint32_t pts = smem_addr(smem) + (uint32_t)(NB * warp) * P.tile_bytes, obuf = pts + P.tile_bytes;
     const uint32_t row = pts + (uint32_t)(lane * rowlen) * 4u, orow = obuf + (uint32_t)(lane * rowlen) * 4u;
+    const ActionTrig trig{DRAW && P.trig_span > 0 ? smem_addr(smem) + (uint32_t)(NB * (int)(blockDim.x >> 5)) * P.tile_bytes : 0u,
+                          P.action_low};
     const uint32_t queue = smem_addr(&queue_next);
     const uint64_t pol_stream = P.pol_stream, pol_keep = P.pol_state;
     const int tile_end = (int)P.tile_end, n_branches = (int)B.n, n_src = (int)P.n;
@@ -1466,10 +1479,12 @@ branch_kernel(const __grid_constant__ StepParams P, const __grid_constant__ Bran
         return t < tile_end ? t : -1;
     };
     if (threadIdx.x == 0) queue_next = blockDim.x >> 5;
+    if (DRAW && trig.table) fill_action_trig<ARM>(P, trig.table);
     __syncthreads();
     int cur = tile_of(warp);
     griddep_launch_dependents();
     griddep_wait();                                       // nothing is read before the previous grid is complete
+    const unsigned long long key = DRAW ? *B.draw_key : 0ull;
     const int ep_shift = ep_shift_of<X>(P);
     const uint32_t amask = ep_shift ? ((1u << ep_shift) - 1u) : 0xffffffffu;
     while (cur >= 0) {
@@ -1499,14 +1514,23 @@ branch_kernel(const __grid_constant__ StepParams P, const __grid_constant__ Bran
         uint32_t ground_steps = 0;                        // settle_step counts them; nothing reads them here
         for (int s = 0; s < P.n_steps && __any_sync(0xffffffffu, live); ++s) {
             const size_t srow = (size_t)s * (size_t)n_branches;
-            load_action_row<J>(in ? P.actions + (srow + (size_t)m) * J : nullptr, sc.a, pol_stream);
-            // the next step's action tile towards the L2 while this step computes (a hint: aligned full tiles only)
-            const float *next = P.actions + (srow + (size_t)n_branches + (size_t)m0) * J;
-            if (full && lane == 0 && s + 1 < P.n_steps && bulk_aligned((uintptr_t)next))
-                bulk_prefetch_l2(next, (uint32_t)(kTile * 4 * J));
+            const bool drawn = DRAW && s >= B.n_prefix;
+            if (drawn) {
+                draw_actions(P, key + (unsigned long long)s, (long long)m, J, sc.a);
+#pragma unroll
+                for (int i = 0; i < J; ++i) sc.a[i] = in ? sc.a[i] : 0.f;
+            } else {
+                load_action_row<J>(in ? P.actions + (srow + (size_t)m) * J : nullptr, sc.a, pol_stream);
+                // the next step's action tile towards the L2 while this step computes (a hint: aligned full tiles only)
+                const float *next = P.actions + (srow + (size_t)n_branches + (size_t)m0) * J;
+                if (full && lane == 0 && s + 1 < (DRAW ? B.n_prefix : P.n_steps) && bulk_aligned((uintptr_t)next))
+                    bulk_prefetch_l2(next, (uint32_t)(kTile * 4 * J));
+            }
             Frames f;
-            if (ARM == 0) ref_arm<false>(sc.g, sc.a, P.substeps, P.inv_div, f, nullptr);
-            else generic_arm<ARM, false>(P, sc.g, sc.a, f, nullptr);
+            // a lane past M holds zeros, which need not lie in [action_low, action_low + span): it evaluates, never looks up
+            const ActionTrig tab = drawn && in ? trig : ActionTrig{0u, 0};
+            if (ARM == 0) ref_arm<DRAW>(sc.g, sc.a, P.substeps, P.inv_div, f, nullptr, tab);
+            else generic_arm<ARM, DRAW>(P, sc.g, sc.a, f, nullptr, tab);
             const bool neg = f.zmin < 0.0f;
             const uint32_t caught = walk_row<X, false>(row, row, x, f, P.catch_tol, alive);
             float gn[J], rew;
